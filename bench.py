@@ -1,7 +1,7 @@
 #!/usr/bin/env python
 """bench.py — headline benchmark of the ISWM hot path on B200.
 
-  python bench.py [--gpus N] [--steps K] [--warmup W] [--impl ours|reference] [--workload train|predict|lossmetric]
+  python bench.py [--gpus N] [--steps K] [--warmup W] [--impl ours|reference] [--workload train|predict|lossmetric] [--dump-outputs DIR]
 
 Metric (BASELINE.json): train img/s of DeepLabV3+ ResNet-50 OS16, synthetic 512x512 tiles, batch 16
 per GPU (cfg2), one step = forward + adaptive weighted CE + backward + SGD step. For N > 1 launch
@@ -116,6 +116,28 @@ def synth_batch(B, H, W, seed, device=None, pinned=False):
     return x, y
 
 
+DUMP_SAMPLE = 1 << 22      # elements kept of a larger output: 16 MB of float32, so that no workload dumps more than 64 MB
+
+
+def dump_sample(t):
+    """`t` flattened; above DUMP_SAMPLE elements, a fixed seeded choice of DUMP_SAMPLE of them (in index order), the same
+    on every run and for every output of that size."""
+    flat = t.detach().reshape(-1)
+    if flat.numel() <= DUMP_SAMPLE:
+        return flat
+    idx = torch.randperm(flat.numel(), generator=torch.Generator().manual_seed(0))[:DUMP_SAMPLE].sort().values
+    return flat[idx.to(flat.device)]
+
+
+def dump_outputs(out_dir, arrays):
+    """--dump-outputs: every array as <out_dir>/<name>.npy, int64 counts as float64 (exact), everything else as float32."""
+    import numpy as np
+    os.makedirs(out_dir, exist_ok=True)
+    for name, t in arrays.items():
+        t = t.detach().cpu()
+        np.save(os.path.join(out_dir, name + ".npy"), (t.double() if t.dtype == torch.int64 else t.float()).numpy())
+
+
 # ----------------------------------------------------------------------------- CPU arms
 def cpu_train_step_rate(B, H, W, steps, warmup, threads=None, backbone="resnet50", output_stride=16):
     """The reference algorithm on the host: fp32 torch oracle (oracle/torch_model.py), zero_grad ->
@@ -158,7 +180,7 @@ def run_reference(args):
     if rank != 0:
         return
     H = W = args.size
-    steps, warmup = max(1, min(args.steps, 3)), 1
+    steps, warmup = args.steps, 1
     if args.workload == "predict":
         Hs = min(H, 1024)
         rate, per, n = cpu_predict_rate(1, Hs, Hs, steps, warmup)
@@ -331,9 +353,11 @@ def run_predict(args, dev, world, rank, local):
     if rank == 0:
         sampler.wait_first_sample(5.0)
     launches0 = _lib.launch_count()
-    ms, w0, w1, _ = _time_region(lambda: step(x_dev, y_dev), args.steps, barrier)
+    ms, w0, w1, (pred, conf) = _time_region(lambda: step(x_dev, y_dev), args.steps, barrier)
     launches = _lib.launch_count() - launches0
     clocks = sampler.stop(w0, w1) if rank == 0 else None
+    if args.dump_outputs and rank == 0:                 # this rank's counters: the metric's all-reduce needs every rank
+        dump_outputs(args.dump_outputs, {"pred": dump_sample(pred), "conf": dump_sample(conf), "confusion": metrics._cm()})
     metrics.reset()
 
     from iswm_b200.data import HostBatchPrefetcher
@@ -416,7 +440,7 @@ def run_lossmetric(args, dev, world, rank, local):
            "wce_fwd_bwd": lambda: ops.wce_fwd_bwd(logits, labels, w, hist),
            "argmax_confusion": lambda: ops.argmax_confusion(logits, labels, mode=1, threshold=0.5, out=cm)}
     flush = torch.empty(256 << 20, dtype=torch.uint8, device=dev)       # > 126 MB L2
-    res = {}
+    res, last = {}, {}
     sampler = ClockSampler(local)
     sampler.start()
     sampler.wait_first_sample(5.0)
@@ -430,7 +454,7 @@ def run_lossmetric(args, dev, world, rank, local):
             flush.zero_()
             e0, e1 = torch.cuda.Event(enable_timing=True), torch.cuda.Event(enable_timing=True)
             e0.record()
-            fn()
+            last[name] = fn()
             e1.record()
             torch.cuda.synchronize()
             ts.append(e0.elapsed_time(e1))
@@ -438,6 +462,10 @@ def run_lossmetric(args, dev, world, rank, local):
         res[name] = {"us": ts[len(ts) // 2] * 1e3, "algorithmic_bytes": algo[name]}
     launches = _lib.launch_count() - launches0
     clocks = sampler.stop(w0, time.time())
+    if args.dump_outputs and rank == 0:
+        loss, grad = last["wce_fwd_bwd"]
+        dump_outputs(args.dump_outputs, {"class_hist": last["class_hist"], "wce_loss": loss, "wce_grad": dump_sample(grad),
+                                         "confusion": last["argmax_confusion"][0]})
     pk = peaks()
     for name, r in res.items():
         r["GB/s"] = r["algorithmic_bytes"] / (r["us"] * 1e-6) / 1e9
@@ -448,9 +476,9 @@ def run_lossmetric(args, dev, world, rank, local):
     lh, yh = logits.cpu().pin_memory(), labels.cpu().pin_memory()
     torch.cuda.synchronize()
     t0 = time.perf_counter()
-    for _ in range(3):
+    for _ in range(args.steps):
         v = float(crit(lh.to(dev, non_blocking=True), yh.to(dev, non_blocking=True)))
-    e2e_s = (time.perf_counter() - t0) / 3
+    e2e_s = (time.perf_counter() - t0) / args.steps
     total_us = sum(r["us"] for r in res.values())
     k = "wce_fwd_bwd"
     cpu = None
@@ -780,6 +808,19 @@ def run_ours(args):
     # captured step's int64 label buffer
     y_host = y_host.to(torch.uint8).pin_memory()
 
+    def dump_step(loss):
+        # --dump-outputs: what the run's SECOND step returned (the loss) and left in the model: parameters after the update, their
+        # gradients, the BatchNorm buffers. It is a steady-state step (in graph mode a plain replay: operands packed by the previous
+        # step's optimiser kernel, momentum carried over) and still reproducible: weight gradients are summed with fp32 atomics in no
+        # fixed order, and from the third step on BatchNorm amplifies those last bits far beyond rounding, so the run's last
+        # step is not (DESIGN.md, "A multi-step RUN"; measured at cfg2 by tools/steps_divergence_probe.py).
+        if args.dump_outputs and rank == 0:
+            params = list(model.parameters())
+            dump_outputs(args.dump_outputs, {
+                "loss": loss, "params": dump_sample(torch.cat([p.detach().reshape(-1) for p in params])),
+                "grads": dump_sample(torch.cat([p.grad.reshape(-1) for p in params])),
+                "buffers": torch.cat([b.reshape(-1).float() for b in model.buffers()])})
+
     # the step is captured once and replayed as ONE CUDA graph launch (iswm_b200.graphs.GraphedTrainStep, the recommended
     # API; ISWM_BENCH_GRAPH=0 times the eager ~430-launch step instead). Data-parallel steps are captured too when the
     # peer-memory transport is up (every exchange is a plain kernel); on the torch.distributed transport they stay eager.
@@ -833,8 +874,12 @@ def run_ours(args):
     sampler = ClockSampler(local)
     if rank == 0:
         sampler.start()
-    for _ in range(args.warmup):
-        step(x_dev, y_dev)
+    done = 0 if stepper is None else 1      # the capture call above ran the first step (capture-time warm-up state restored)
+    for _ in range(args.warmup):            # at least 3
+        loss = step(x_dev, y_dev)
+        done += 1
+        if done == 2:
+            dump_step(loss)
     barrier()
     if rank == 0:
         sampler.wait_first_sample(5.0)
@@ -988,6 +1033,7 @@ def run_ours(args):
 
 
 def main():
+    sys.dont_write_bytecode = True      # the package is imported below this point: a run leaves no __pycache__ in the tree
     ap = argparse.ArgumentParser()
     ap.add_argument("--gpus", type=int, default=1)
     ap.add_argument("--steps", type=int, default=10)
@@ -1004,7 +1050,15 @@ def main():
     ap.add_argument("--no-extras", action="store_true", help="N=1 cfg2 only: skip the compact cfg5 / cfg4 side measurements (config.extra)")
     ap.add_argument("--no-dp-parity", action="store_true", help="N>1 only: skip the multi-rank parity step before the timed region (config.dp_parity)")
     ap.add_argument("--profile-detail", default="", help="write the per-launch table of the instrumented step here")
+    ap.add_argument("--dump-outputs", default="", metavar="DIR",
+                    help="write what the timed step function computed as DIR/<name>.npy (float32 / float64, a fixed seeded sample of any "
+                         "output over 4 Mi elements): train, its second step from the seeded weights; predict and lossmetric, the last "
+                         "timed step. Inputs are seeded, so two runs or two builds can be compared output for output")
     args = ap.parse_args()
+    if args.steps < 1:
+        ap.error("--steps must be at least 1")
+    if args.dump_outputs and args.impl != "ours":
+        ap.error("--dump-outputs dumps the CUDA path (--impl ours)")
     args.warmup = max(args.warmup, 3) if args.impl == "ours" else args.warmup
     args.batch = args.batch or {"train": 16, "predict": 8, "lossmetric": 16}[args.workload]
     args.size = args.size or {"train": 512, "predict": 2048, "lossmetric": 1024}[args.workload]
