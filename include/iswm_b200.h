@@ -135,8 +135,7 @@ enum {
   ISWM_EPI_RESIDUAL = 4,  /* y += residual (bf16, same geometry, own ld)      */
   ISWM_EPI_STATS    = 8,  /* accumulate per-channel fp32 sum / sum^2 of the STORED bf16 outputs (needs bf16 out, out_ld % 8 == 0) */
   ISWM_EPI_OUT_F32  = 16, /* write fp32 instead of bf16                       */
-  ISWM_EPI_RES_MASK = 32, /* the residual is gated by packed ReLU sign bits (iswm_conv_igemm_ex): y += res * bit  */
-  ISWM_EPI_BN_DZ    = 64  /* BatchNorm-backward pass 1 rides on this data gradient's epilogue (iswm_conv_igemm_bn) */
+  ISWM_EPI_RES_MASK = 32  /* the residual is gated by packed ReLU sign bits (iswm_conv_igemm_ex): y += res * bit  */
 };
 
 /* Geometry of one implicit-GEMM convolution over NHWC bf16 activations.
@@ -194,26 +193,6 @@ int iswm_conv_igemm(const iswm_conv_desc* desc, const void* d_in, const void* d_
 int iswm_conv_igemm_ex(const iswm_conv_desc* desc, const void* d_in, const void* d_wgt,
                        void* d_out, const float* d_scale, const float* d_shift,
                        const void* d_res, double* d_stats, const uint8_t* d_res_mask, void* stream);
-
-/* Data gradient + the FIRST pass of the BatchNorm backward of the unit whose activation gradient it produces
- * (conv -> BatchNorm -> ReLU, network/backbone/resnet.py:99-108, network/_deeplab.py:44-50: autograd's
- * threshold_backward + the two per-channel reductions of native_batch_norm_backward). The launch computes the data gradient
- * dout of a convolution whose INPUT was that unit's activation, and in its epilogue
- *   dz = dout where the unit's ReLU was active (mask recomputed from `raw`, the unit's pre-BN bf16 output, with the
- *        forward kernel's own fma), 0 elsewhere                                   -> written to d_out instead of dout,
- *   sums[c] += sum(dz), sums[Cout + c] += sum(dz * xhat)                          -> what iswm_bn_bwd_reduce would produce,
- * so that tensor is not re-read for the reduction: the unit's backward continues with iswm_bn_bwd_apply(relu_mode = 0) on dz.
- * Dense bf16 output with Cout %% 64 == 0; desc->flags must be 0 or ISWM_EPI_BN_DZ. */
-typedef struct {
-  const void*  raw;     /* bf16 [B*Ho*Wo][Cout]: pre-BatchNorm output of the unit (iswm_conv_igemm with ISWM_EPI_STATS) */
-  const float* mean;    /* float[Cout] saved batch mean   (iswm_bn_train_apply) */
-  const float* invstd;  /* float[Cout] saved 1/sqrt(var + eps)                  */
-  const float* gamma;   /* float[Cout] BatchNorm weight                         */
-  const float* beta;    /* float[Cout] BatchNorm bias                           */
-  double*      sums;    /* double[2*Cout], ACCUMULATED (zero it first)          */
-} iswm_bn_dz;
-int iswm_conv_igemm_bn(const iswm_conv_desc* desc, const void* d_in, const void* d_wgt, void* d_out,
-                       const iswm_bn_dz* bn, void* stream);
 
 /* ASPP backward, data-gradient half (network/_deeplab.py:143-172: the 1x1 branch and the three dilated 3x3 branches all
  * read the SAME 2048-channel feature map): ONE K-concatenated implicit GEMM
@@ -399,29 +378,12 @@ int iswm_bn_dual_bwd_apply(const void* d_dout, int dout_ld, const uint8_t* d_rel
                            float* d_dgamma, float* d_dbeta, float* d_dgamma_ds, float* d_dbeta_ds, void* stream);
 
 /* ---- stem tail: BatchNorm + ReLU + 3x3/s2/p1 max pooling in ONE pass (csrc/stem_pool.cu; network/backbone/resnet.py:145-147) ----
- * forward: d_raw bf16 [B,H,W,64] = the stem convolution's pre-BN output (with its statistics in bn->stats); writes the pooled
+ * d_raw bf16 [B,H,W,64] = the stem convolution's pre-BN output (with its statistics in bn->stats); writes the pooled
  * bf16 [B,Ho,Wo,64] tensor and, per pooled element, which of the 9 window positions won (uint8 [B,Ho,Wo,64], first maximum in
  * window order) - the normalised half-resolution activation is never written. bn: stats / gamma / beta read, running statistics
  * updated, save_mean / save_invstd written. */
 int iswm_stem_pool_fwd(const void* d_raw, const iswm_bn_side* bn, int B, int H, int W, int C, int Ho, int Wo,
                        float eps, float momentum, void* d_out, uint8_t* d_idx, void* stream);
-/* backward (two launches inside): d_dpool bf16 [B,Ho,Wo,64] gradient of the pooled tensor -> d_dy bf16 [B,H,W,64] gradient of the
- * pre-BN tensor; both BatchNorm-backward passes gather the activation gradient through the argmax codes and recompute the ReLU
- * mask from d_raw, so that gradient is never written either. d_sums double[128], zeroed by the caller; dgamma / dbeta ACCUMULATE. */
-int iswm_stem_pool_bwd(const void* d_dpool, const uint8_t* d_idx, const void* d_raw, const iswm_bn_side* bn,
-                       int B, int H, int W, int C, int Ho, int Wo, double* d_sums, void* d_dy,
-                       float* d_dgamma, float* d_dbeta, void* stream);
-
-/* Both passes in ONE launch (what the engine uses): pass 1, a grid-wide barrier, pass 2 over the same rows (served
- * from L2 for all but the largest tensors). d_sums: double[2*C + 1], zeroed by the caller; the extra cell is the
- * barrier's arrival counter. The grid is sized to be co-resident; the barrier wait is bounded
- * (iswm_debug_abort_code() reports 21 if it ever timed out). */
-int iswm_bn_bwd(const void* d_dout, int dout_ld, const void* d_x, int x_ld,
-                const void* d_out_act, int act_ld, int64_t M, int C,
-                const float* d_gamma, const float* d_beta, const float* d_save_mean,
-                const float* d_save_invstd, double* d_sums, int relu, float drop_p, uint64_t drop_seed, const int64_t* d_drop_step,
-                void* d_dx, int dx_ld, void* d_dz, int dz_ld,
-                float* d_dgamma, float* d_dbeta, void* stream);
 
 /* Stem 7x7 / stride 2 / pad 3 (network/backbone/resnet.py:144), ROW-TAP form - what the engine runs. The fp32 NCHW image is
  * unrolled along x only: d_out bf16 [2][B][Hh][Wo][kpitch], element [p][b][hh][wo][s*Cin + c] = img[b][c][2*hh + p][2*wo + s - 3]

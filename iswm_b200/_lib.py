@@ -17,7 +17,7 @@ LIB_PATH = os.environ.get("ISWM_B200_LIB") or os.path.join(_HERE, "libiswm_b200.
 MAX_TAPS = 32
 U8, I32, I64 = 0, 1, 2
 F32, BF16 = 0, 1
-EPI_AFFINE, EPI_RELU, EPI_RESIDUAL, EPI_STATS, EPI_OUT_F32, EPI_RES_MASK, EPI_BN_DZ = 1, 2, 4, 8, 16, 32, 64
+EPI_AFFINE, EPI_RELU, EPI_RESIDUAL, EPI_STATS, EPI_OUT_F32, EPI_RES_MASK = 1, 2, 4, 8, 16, 32
 
 
 class ConvDesc(C.Structure):
@@ -33,13 +33,6 @@ class ConvDesc(C.Structure):
         ("flags", C.c_int32), ("out_ws", C.c_int32), ("out_hs", C.c_int32), ("out_bs", C.c_int64),
         ("w_ntaps", C.c_int32), ("stats_replicas", C.c_int32), ("in_phase_view", C.c_int32), ("reserved2_", C.c_int32),
     ]
-
-
-class BnDz(C.Structure):
-    """Mirror of iswm_bn_dz."""
-
-    _fields_ = [("raw", C.c_void_p), ("mean", C.c_void_p), ("invstd", C.c_void_p), ("gamma", C.c_void_p),
-                ("beta", C.c_void_p), ("sums", C.c_void_p)]
 
 
 class BnSide(C.Structure):
@@ -116,7 +109,6 @@ SIGNATURES = {
     "iswm_focal_fwd_bwd": (_i, [_p, _i, _p, _i, _p, _i64, _i, _i64, _i, _f, _f, _i, _p, _p, _p, _p]),
     "iswm_conv_igemm": (_i, [C.POINTER(ConvDesc), _p, _p, _p, _p, _p, _p, _p, _p]),
     "iswm_conv_igemm_ex": (_i, [C.POINTER(ConvDesc), _p, _p, _p, _p, _p, _p, _p, _p, _p]),
-    "iswm_conv_igemm_bn": (_i, [C.POINTER(ConvDesc), _p, _p, _p, C.POINTER(BnDz), _p]),
     "iswm_aspp_bwd": (_i, [_p, _i, _p, _i, _i, _i, _i, _i, C.POINTER(C.c_int), _p, _i, _i, _p]),
     "iswm_peer_barrier": (_i, [C.POINTER(_p), _i, _i, _p, _p]),
     "iswm_peer_allreduce_f32": (_i, [C.POINTER(_p), _i, _i, _i64, _i64, _i, _p]),
@@ -140,8 +132,6 @@ SIGNATURES = {
     "iswm_bn_dual_bwd_apply": (_i, [_p, _i, _p, _p, _i, C.POINTER(BnSide), _p, _p, _i, C.POINTER(BnSide), _p, _i64, _i, _p, _i, _p, _i,
                                     _p, _p, _p, _p, _p]),
     "iswm_stem_pool_fwd": (_i, [_p, C.POINTER(BnSide), _i, _i, _i, _i, _i, _i, _f, _f, _p, _p, _p]),
-    "iswm_stem_pool_bwd": (_i, [_p, _p, _p, C.POINTER(BnSide), _i, _i, _i, _i, _i, _i, _p, _p, _p, _p, _p]),
-    "iswm_bn_bwd": (_i, [_p, _i, _p, _i, _p, _i, _i64, _i, _p, _p, _p, _p, _p, _i, _f, _u64, _p, _p, _i, _p, _i, _p, _p, _p]),
     "iswm_stem_rows": (_i, [_p, _i, _i, _i, _i, _i, _i, _i, _p, _p]),
     "iswm_unpack_wgrad_stem": (_i, [_p, _i, _i, _i, _i, _f, _p, _p]),
     "iswm_stem_im2col": (_i, [_p, _i, _i, _i, _i, _i, _i, _i, _p, _p]),

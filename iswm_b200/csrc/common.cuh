@@ -45,9 +45,6 @@ inline int check_launch(const char* what) {
 __device__ __forceinline__ void pdl_wait() { asm volatile("griddepcontrol.wait;" ::: "memory"); }
 __device__ __forceinline__ void pdl_launch() { asm volatile("griddepcontrol.launch_dependents;" ::: "memory"); }
 bool pdl_enabled();
-// Experiment switch (ISWM_CARVEOUT=1, default off): ask for the same L1 / shared-memory split (maximum shared memory) for every
-// kernel of the library, so that no conv <-> BatchNorm boundary changes the SM's carve-out. Measured slower (see lib.cu).
-void ensure_carveout(const void* kernel);
 
 template <typename... KArgs, typename... Args>
 inline void launch_k(void (*kernel)(KArgs...), dim3 grid, dim3 block, size_t smem, cudaStream_t st, Args&&... args) {
@@ -61,7 +58,6 @@ inline void launch_k(void (*kernel)(KArgs...), dim3 grid, dim3 block, size_t sme
   attr[0].val.programmaticStreamSerializationAllowed = 1;
   cfg.attrs = attr;
   cfg.numAttrs = pdl_enabled() ? 1 : 0;
-  ensure_carveout(reinterpret_cast<const void*>(kernel));
   cudaLaunchKernelEx(&cfg, kernel, static_cast<KArgs>(args)...);   // errors surface in check_launch()
 }
 

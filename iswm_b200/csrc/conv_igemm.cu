@@ -25,7 +25,6 @@
 // same kernel with transposed packed weights and negated tap offsets.
 #include "tc_common.cuh"
 #include <algorithm>
-#include <stdlib.h>
 
 namespace iswm {
 
@@ -62,11 +61,6 @@ struct ConvKParams {
   const uint8_t* mask;           // ISWM_EPI_RES_MASK: ReLU sign bits [pixels][Cout/8] gating the residual (dz = dout . mask)
   double* stats;                 // fp64 accumulators: cross-CTA summation order no longer shows up in fp32 results
   int stats_rep;                 // copies of the accumulator vector; this CTA adds into copy blockIdx.x % stats_rep
-  // ISWM_EPI_BN_DZ: BatchNorm-backward pass 1 of the unit whose activation gradient this launch produces (res = its pre-BN output)
-  const float* bn_mean;
-  const float* bn_invstd;
-  const float* bn_gamma;
-  const float* bn_beta;
   int* abort_flag;
 };
 
@@ -100,12 +94,13 @@ struct TileIter {
   }
 };
 
-// NWG = number of epilogue warpgroups: 2 (384 threads, up to 168 registers each) for long-K convolutions whose epilogue
-// hides under the MMA main loop, 3 (512 threads, 128 registers) for short-K ones that are bound by the epilogue.
-// BNDZ: the instantiation that carries the BatchNorm-backward epilogue (ISWM_EPI_BN_DZ); kept apart so that its extra
-// live registers (the operand row stays live until the per-channel products) do not cost the ordinary epilogues a spill.
-template <int NWG, bool BNDZ>
-__global__ void __launch_bounds__(128 * (NWG + 1), 1)
+// Epilogue warpgroups: two (384 threads, up to 168 registers each). A third one for short-K (epilogue-bound) convolutions
+// was measured and lost (cfg2 16.05 vs 15.64 ms/step, cfg4 27.1 vs 26.5): it costs a ring stage and 40 registers per
+// thread, and the epilogue is paced by TMEM-read and barrier latency rather than by warp count (DESIGN.md).
+constexpr int kEpiWG = 2;
+constexpr int kConvThreads = 128 * (kEpiWG + 1);
+
+__global__ void __launch_bounds__(kConvThreads, 1)
 conv_igemm_kernel(const __grid_constant__ CUtensorMap tmap_a,
                   const __grid_constant__ CUtensorMap tmap_b,
                   const __grid_constant__ CUtensorMap tmap_out, const ConvKParams p) {
@@ -120,12 +115,12 @@ conv_igemm_kernel(const __grid_constant__ CUtensorMap tmap_a,
   const uint32_t b_bytes = (uint32_t)p.BN * 128u;
   const uint32_t stage_bytes = kABytes + b_bytes;
   // [ring stages][out staging: one 16K tile per epilogue warpgroup, if TMA out][residual prefetch: same][barriers][scale, shift]
-  const bool tma_out = BNDZ || p.use_tma_out != 0;
+  const bool tma_out = p.use_tma_out != 0;
   uint32_t off = (uint32_t)p.stages * stage_bytes;
   const uint32_t obuf = ring + off;
-  if (tma_out) off += NWG * kStageBuf;
+  if (tma_out) off += kEpiWG * kStageBuf;
   const uint32_t rbuf = ring + off;                        // residual prefetch tile, one per epilogue warpgroup
-  if (p.res_prefetch) off += NWG * kStageBuf;
+  if (p.res_prefetch) off += kEpiWG * kStageBuf;
   uint8_t* tail = smem + off;
   uint64_t* bars = reinterpret_cast<uint64_t*>(tail);      // full[8] empty[8] tfull[2] tempty[2]
   uint32_t* tmem_slot = reinterpret_cast<uint32_t*>(bars + 2 * kMaxStages + 6);
@@ -151,7 +146,7 @@ conv_igemm_kernel(const __grid_constant__ CUtensorMap tmap_a,
     }
     for (int s = 0; s < 2; s++) {
       tc::mbar_init(bar_tfull + 8 * s, 1);
-      tc::mbar_init(bar_tempty + 8 * s, 4 * NWG);   // one arrival per epilogue warp
+      tc::mbar_init(bar_tempty + 8 * s, 4 * kEpiWG);   // one arrival per epilogue warp
     }
     tc::fence_barrier_init();
   }
@@ -288,26 +283,18 @@ conv_igemm_kernel(const __grid_constant__ CUtensorMap tmap_a,
   } else if (warp >= 4) {
     // ===================== epilogue: two warpgroups, 64-channel chunks alternate between them =====================
     const int nchunk64 = (p.BN + 63) >> 6;
-    const int wg = (warp - 4) >> 2;                     // warpgroup 0 .. NWG-1
-    constexpr int NSLOT = (NWG == 2) ? 2 : 4;           // statistics slots per thread (chunk positions it can own)
-    // which warpgroup owns 64-channel chunk c of this CTA's it-th tile: two warpgroups take alternate chunks
-    // (alternate tiles when a tile is a single chunk), three rotate over the running chunk count
-    auto owner_of = [&](int it_, int c_) -> int {
-      if (NWG == 2) return ((nchunk64 == 1) ? it_ : c_) & 1;
-      return (it_ * nchunk64 + c_) % 3;
-    };
+    const int wg = (warp - 4) >> 2;                     // warpgroup 0 or 1
+    constexpr int NSLOT = 2;                            // statistics slots per thread (chunk positions it can own)
+    // which warpgroup owns 64-channel chunk c of this CTA's it-th tile: the two warpgroups take alternate chunks
+    // (alternate tiles when a tile is a single chunk)
+    auto owner_of = [&](int it_, int c_) -> int { return ((nchunk64 == 1) ? it_ : c_) & 1; };
     const int q = warp & 3;                             // TMEM lane quadrant of this warp (warp % 4)
     const int row = q * 32 + lane;                      // accumulator row = thread index inside the warpgroup
     const int bb = row >> (p.lgBW + p.lgBH);
     const int hh = (row >> p.lgBW) & (BH - 1);
     const int ww = row & (BW - 1);
-    // (the BNDZ instantiation combines with no other epilogue option: they fold away at compile time)
-    const bool f_aff = !BNDZ && (p.flags & ISWM_EPI_AFFINE), f_relu = !BNDZ && (p.flags & ISWM_EPI_RELU),
-               f_res = !BNDZ && (p.flags & ISWM_EPI_RESIDUAL), f_stats = !BNDZ && (p.flags & ISWM_EPI_STATS),
-               f_mask = !BNDZ && (p.flags & ISWM_EPI_RES_MASK), f_f32 = !BNDZ && (p.flags & ISWM_EPI_OUT_F32);
-    constexpr bool f_bndz = BNDZ;
-    const bool f_sums = f_stats || f_bndz;              // per-channel column sums leave the CTA (forward statistics / BN-backward sums)
-    const bool f_row = f_res || f_bndz;                 // a [pixels][Cout] bf16 operand row is read per chunk (p.res)
+    const bool f_aff = p.flags & ISWM_EPI_AFFINE, f_relu = p.flags & ISWM_EPI_RELU, f_res = p.flags & ISWM_EPI_RESIDUAL,
+               f_stats = p.flags & ISWM_EPI_STATS, f_mask = p.flags & ISWM_EPI_RES_MASK, f_f32 = p.flags & ISWM_EPI_OUT_F32;
     // Each epilogue WARP is independent between channel-tile changes: it stages its own 32 rows (a 4 KiB, 1 KiB-aligned
     // slice of the warpgroup's staging tile), issues its own TMA store (a 32-pixel sub-box of the tile) and sums its own
     // rows for the statistics - __syncwarp() instead of three 128-thread named barriers per chunk, so the eight warps
@@ -344,7 +331,7 @@ conv_igemm_kernel(const __grid_constant__ CUtensorMap tmap_a,
       if (q == 0) {
 #pragma unroll
         for (int slot = 0; slot < NSLOT; slot++) {
-          const int c64 = (NWG == 2) ? ((nchunk64 == 1) ? 0 : 2 * slot + wg) : slot;
+          const int c64 = (nchunk64 == 1) ? 0 : 2 * slot + wg;
           if (c64 >= nchunk64) continue;
           float t[4];
 #pragma unroll
@@ -358,18 +345,6 @@ conv_igemm_kernel(const __grid_constant__ CUtensorMap tmap_a,
             }
           }
           const int col = n0f + c64 * 64 + 2 * lane;
-          if (f_bndz) {
-            // t[0..1] = sum(dz), t[2..3] = sum(dz * x): sum(dz * xhat) = invstd * (sum(dz*x) - mean * sum(dz)), formed in fp64
-            // per CTA exactly as bn_bwd_reduce_kernel forms it per block
-#pragma unroll
-            for (int e = 0; e < 2; e++)
-              if (col + e < p.Cout) {
-                atomicAdd(stats_mine + col + e, (double)t[e]);
-                atomicAdd(stats_mine + p.Cout + col + e,
-                          (double)p.bn_invstd[col + e] * ((double)t[2 + e] - (double)p.bn_mean[col + e] * (double)t[e]));
-              }
-            continue;
-          }
           if (col < p.Cout) {
             atomicAdd(stats_mine + col, (double)t[0]);
             atomicAdd(stats_mine + p.Cout + col, (double)t[2]);
@@ -386,7 +361,7 @@ conv_igemm_kernel(const __grid_constant__ CUtensorMap tmap_a,
     // is prefetched with cp.async into the warpgroup's residual tile while the current chunk is processed; only the
     // issuing thread reads it back, so no barrier is involved.
     const uint32_t rb_row = rbuf + (uint32_t)wg * kStageBuf + row_off;
-    const bool res_pf_ok = f_row && p.res_prefetch != 0;
+    const bool res_pf_ok = f_res && p.res_prefetch != 0;
     auto chunk_owner_ok = [&](const TileIter& ti_, int it_, int c_) -> bool {
       if (owner_of(it_, c_) != wg) return false;
       return ti_.nt * p.BN + c_ * 64 < p.Cout;
@@ -441,25 +416,15 @@ conv_igemm_kernel(const __grid_constant__ CUtensorMap tmap_a,
       const long long opix = (long long)b * p.o_bs + (long long)h * p.o_hs + (long long)w * p.o_ws;   // element offsets
       const long long rpix = (long long)b * p.r_bs + (long long)h * p.r_hs + (long long)w * p.r_ws;
       if (n0 != cur_n0) {
-        if (f_sums && cur_n0 >= 0) flush_stats(cur_n0);
-        if (f_aff || f_bndz) {
-          asm volatile("bar.sync 3, %0;" ::"n"(128 * NWG) : "memory");   // every reader of the previous channel tile is done
-          for (int i = threadIdx.x - 128; i < p.BN; i += 128 * NWG) {
+        if (f_stats && cur_n0 >= 0) flush_stats(cur_n0);
+        if (f_aff) {
+          asm volatile("bar.sync 3, %0;" ::"n"(128 * kEpiWG) : "memory");   // every reader of the previous channel tile is done
+          for (int i = threadIdx.x - 128; i < p.BN; i += 128 * kEpiWG) {
             const int n = n0 + i;
-            float sc_ = 0.f, sh_ = 0.f;
-            if (n < p.Cout) {
-              if (f_bndz) {            // the forward kernel's own scale / shift arithmetic (bn_train_apply_kernel): same ReLU mask
-                sc_ = p.bn_gamma[n] * p.bn_invstd[n];
-                sh_ = fmaf(-p.bn_mean[n], sc_, p.bn_beta[n]);
-              } else {
-                sc_ = p.scale[n];
-                sh_ = p.shift[n];
-              }
-            }
-            s_scale[i] = sc_;
-            s_shift[i] = sh_;
+            s_scale[i] = (n < p.Cout) ? p.scale[n] : 0.f;
+            s_shift[i] = (n < p.Cout) ? p.shift[n] : 0.f;
           }
-          asm volatile("bar.sync 3, %0;" ::"n"(128 * NWG) : "memory");
+          asm volatile("bar.sync 3, %0;" ::"n"(128 * kEpiWG) : "memory");
         }
         cur_n0 = n0;
       }
@@ -477,8 +442,8 @@ conv_igemm_kernel(const __grid_constant__ CUtensorMap tmap_a,
         tc::tmem_ld64(t_row + c64 * 64, v);
         // residual: this thread's row of the chunk (128 contiguous bytes) was prefetched into shared memory
         uint4 rr[8];
-        const bool res_vec = res_pf_ok ? pf_vec : (f_row && valid && ncols == 64 && (p.res_ld & 7) == 0);
-        if (f_row && !res_pf_ok && res_vec) {             // long-K convolution: direct loads, issued under the TMEM read
+        const bool res_vec = res_pf_ok ? pf_vec : (f_res && valid && ncols == 64 && (p.res_ld & 7) == 0);
+        if (f_res && !res_pf_ok && res_vec) {             // long-K convolution: direct loads, issued under the TMEM read
           const uint4* rp = reinterpret_cast<const uint4*>(p.res + rpix + nc);
 #pragma unroll
           for (int j = 0; j < 8; j++) rr[j] = rp[j];
@@ -538,26 +503,6 @@ conv_igemm_kernel(const __grid_constant__ CUtensorMap tmap_a,
               if (j < ncols && ((mbits >> j) & 1ull)) f[j] += __bfloat162float(rp[j]);
           }
         }
-        if (f_bndz) {
-          // dz = dout where the unit's ReLU was active: the mask is recomputed from the unit's pre-BN output (this
-          // thread's row of it, in rr) with the forward kernel's fma; rows outside the image / partial chunks carry nothing
-          const float4* sc4 = reinterpret_cast<const float4*>(s_scale + c64 * 64);
-          const float4* sh4 = reinterpret_cast<const float4*>(s_shift + c64 * 64);
-#pragma unroll
-          for (int j = 0; j < 8; j++) {
-            const uint32_t r4[4] = {rr[j].x, rr[j].y, rr[j].z, rr[j].w};
-            const float4 a0 = sc4[2 * j], a1 = sc4[2 * j + 1], c0 = sh4[2 * j], c1 = sh4[2 * j + 1];
-            const float as_[8] = {a0.x, a0.y, a0.z, a0.w, a1.x, a1.y, a1.z, a1.w};
-            const float cs_[8] = {c0.x, c0.y, c0.z, c0.w, c1.x, c1.y, c1.z, c1.w};
-#pragma unroll
-            for (int k = 0; k < 4; k++) {
-              float lo, hi;
-              unpack_bf16x2(r4[k], lo, hi);
-              f[8 * j + 2 * k] = (res_vec && fmaf(lo, as_[2 * k], cs_[2 * k]) > 0.f) ? f[8 * j + 2 * k] : 0.f;
-              f[8 * j + 2 * k + 1] = (res_vec && fmaf(hi, as_[2 * k + 1], cs_[2 * k + 1]) > 0.f) ? f[8 * j + 2 * k + 1] : 0.f;
-            }
-          }
-        }
         if (f_relu) {
 #pragma unroll
           for (int j = 0; j < 64; j++) f[j] = fmaxf(f[j], 0.f);
@@ -587,8 +532,8 @@ conv_igemm_kernel(const __grid_constant__ CUtensorMap tmap_a,
             tc::tma_store_commit();
           }
           TMARK(4)
-          if (f_sums) {
-            const int slot = (NWG == 2) ? (c64 >> 1) : c64;
+          if (f_stats) {
+            const int slot = c64 >> 1;
             // plain shared-memory loads (ordered after the barrier above by its memory clobber): 8 rows in flight,
             // then their sums, so the loads are not serialised behind the dependent adds
             const uint8_t* sbase = smem + (ob - ring) + (uint32_t)(q * 32) * 128u + (uint32_t)((lane & 3) << 2);
@@ -607,48 +552,6 @@ conv_igemm_kernel(const __grid_constant__ CUtensorMap tmap_a,
                 s0 += lo; s1 += hi;
                 q0 = fmaf(lo, lo, q0); q1 = fmaf(hi, hi, q1);
               }
-            }
-            if (f_bndz) {
-              // sum over this warp's 32 rows of dz * x per channel: every thread holds the 64 products of its own row
-              // (stored bf16 dz x bf16 pre-BN value, exact in fp32); five exchange-and-add rounds (recursive halving over
-              // the lane bits, fixed order) leave channels 2*lane, 2*lane+1 in this lane - the layout of s0 / s1 above
-              const uint32_t xm = res_vec ? 0xffffffffu : 0u;
-              auto prod2 = [&](int w_, float& plo, float& phi) {      // channel pair w_ (compile-time after unrolling)
-                const uint4 r = rr[w_ >> 2];
-                const uint32_t xw = ((w_ & 3) == 0 ? r.x : (w_ & 3) == 1 ? r.y : (w_ & 3) == 2 ? r.z : r.w) & xm;
-                float dl, dh_, xl, xh;
-                unpack_bf16x2(pk[w_], dl, dh_);
-                unpack_bf16x2(xw, xl, xh);
-                plo = dl * xl; phi = dh_ * xh;
-              };
-              float w32[32];
-              {
-                const bool up = lane & 16;
-#pragma unroll
-                for (int i = 0; i < 16; i++) {                      // channels 2i, 2i+1 against 2i+32, 2i+33
-                  float a0, a1, b0, b1;
-                  prod2(i, a0, a1);
-                  prod2(i + 16, b0, b1);
-                  const float k0 = up ? b0 : a0, k1 = up ? b1 : a1, s0_ = up ? a0 : b0, s1_ = up ? a1 : b1;
-                  w32[2 * i] = k0 + __shfl_xor_sync(0xffffffffu, s0_, 16);
-                  w32[2 * i + 1] = k1 + __shfl_xor_sync(0xffffffffu, s1_, 16);
-                }
-              }
-              float w16[16], w8[8], w4[4], w2[2];
-#define ISWM_HALVE(dst, src, n, bit)                                                          \
-              {                                                                               \
-                const bool up = lane & (bit);                                                 \
-                _Pragma("unroll") for (int i = 0; i < (n); i++) {                             \
-                  const float a = src[i], b = src[i + (n)];                                   \
-                  dst[i] = (up ? b : a) + __shfl_xor_sync(0xffffffffu, up ? a : b, (bit));    \
-                }                                                                             \
-              }
-              ISWM_HALVE(w16, w32, 16, 8)
-              ISWM_HALVE(w8, w16, 8, 4)
-              ISWM_HALVE(w4, w8, 4, 2)
-              ISWM_HALVE(w2, w4, 2, 1)
-#undef ISWM_HALVE
-              q0 = w2[0]; q1 = w2[1];
             }
             // predicated adds on statically indexed registers (a runtime index put the array in local memory)
 #pragma unroll
@@ -693,7 +596,7 @@ conv_igemm_kernel(const __grid_constant__ CUtensorMap tmap_a,
       as ^= 1;
       if (as == 0) aphase ^= 1;
     }
-    if (f_sums && cur_n0 >= 0) flush_stats(cur_n0);
+    if (f_stats && cur_n0 >= 0) flush_stats(cur_n0);
 #ifdef ISWM_EPI_TIMING
     // debug build only: [math+other, tfull wait, tmem load, staging free wait, stage+store, stats] cycles of thread 0/32 of each warpgroup
     if (blockIdx.x == 0 && (row == 0 || row == 32)) {
@@ -732,38 +635,15 @@ extern "C" int iswm_conv_igemm(const iswm_conv_desc* d, const void* d_in, const 
   return iswm_conv_igemm_ex(d, d_in, d_wgt, d_out, d_scale, d_shift, d_res, d_stats, nullptr, stream);
 }
 
-static int conv_igemm_launch(const iswm_conv_desc* d, const void* d_in, const void* d_wgt,
-                             void* d_out, const float* d_scale, const float* d_shift,
-                             const void* d_res, double* d_stats, const uint8_t* d_res_mask, const iswm_bn_dz* bn, void* stream);
-
 extern "C" int iswm_conv_igemm_ex(const iswm_conv_desc* d, const void* d_in, const void* d_wgt,
                                   void* d_out, const float* d_scale, const float* d_shift,
                                   const void* d_res, double* d_stats, const uint8_t* d_res_mask, void* stream) {
-  ISWM_REQUIRE(!(d && (d->flags & ISWM_EPI_BN_DZ)), "conv_igemm: ISWM_EPI_BN_DZ goes through iswm_conv_igemm_bn");
-  return conv_igemm_launch(d, d_in, d_wgt, d_out, d_scale, d_shift, d_res, d_stats, d_res_mask, nullptr, stream);
-}
-
-extern "C" int iswm_conv_igemm_bn(const iswm_conv_desc* d, const void* d_in, const void* d_wgt, void* d_out,
-                                  const iswm_bn_dz* bn, void* stream) {
-  ISWM_REQUIRE(d && bn && bn->raw && bn->mean && bn->invstd && bn->gamma && bn->beta && bn->sums, "conv_igemm_bn: null argument");
-  ISWM_REQUIRE((d->flags & ~ISWM_EPI_BN_DZ) == 0, "conv_igemm_bn: no other epilogue flag combines with ISWM_EPI_BN_DZ (flags=%d)", d->flags);
-  ISWM_REQUIRE((d->Cout % 64) == 0 && d->out_ld == d->Cout && d->out_ws == 0 && d->out_hs == 0 && d->out_bs == 0,
-               "conv_igemm_bn: needs a dense output with Cout %% 64 == 0 (Cout=%d out_ld=%d)", d->Cout, d->out_ld);
-  ISWM_REQUIRE((reinterpret_cast<uintptr_t>(bn->raw) & 15) == 0, "conv_igemm_bn: raw must be 16-byte aligned");
-  iswm_conv_desc dd = *d;
-  dd.flags = ISWM_EPI_BN_DZ;
-  dd.res_ld = d->Cout;                        // the pre-BN tensor rides in the residual slot: same geometry as the output
-  return conv_igemm_launch(&dd, d_in, d_wgt, d_out, nullptr, nullptr, bn->raw, bn->sums, nullptr, bn, stream);
-}
-
-static int conv_igemm_launch(const iswm_conv_desc* d, const void* d_in, const void* d_wgt,
-                             void* d_out, const float* d_scale, const float* d_shift,
-                             const void* d_res, double* d_stats, const uint8_t* d_res_mask, const iswm_bn_dz* bn, void* stream) {
   if (debug_skip(ISWM_SKIP_CONV_IGEMM)) return 0;
   ISWM_REQUIRE(!(d && (d->flags & ISWM_EPI_RES_MASK)) || (d_res_mask && (d->flags & ISWM_EPI_RESIDUAL) && (d->Cout % 64) == 0 &&
                                                           d->out_ws == 0 && d->out_hs == 0 && d->out_bs == 0),
                "conv_igemm: RES_MASK needs RESIDUAL, the bit tensor, Cout %% 64 == 0 and a dense output");
   ISWM_REQUIRE(d && d_in && d_wgt && d_out, "conv_igemm: null argument");
+  ISWM_REQUIRE((d->flags & ~63) == 0, "conv_igemm: unknown epilogue flags (flags=%d)", d->flags);
   ISWM_REQUIRE(d->ntaps >= 1 && d->ntaps <= ISWM_MAX_TAPS, "conv_igemm: ntaps=%d", d->ntaps);
   ISWM_REQUIRE(d->Cin >= 1 && d->Cout >= 1 && d->B >= 1 && d->Ho >= 1 && d->Wo >= 1, "conv_igemm: bad dims");
   ISWM_REQUIRE((d->in_ld % 8) == 0 && d->in_ld >= d->Cin, "conv_igemm: in_ld=%d must be a multiple of 8 and >= Cin=%d", d->in_ld, d->Cin);
@@ -807,8 +687,7 @@ static int conv_igemm_launch(const iswm_conv_desc* d, const void* d_in, const vo
     BN = std::min(256, (((d->Cout + nt - 1) / nt + 63) / 64) * 64);
     // without statistics / residual the tile's last 64-channel chunk may be narrow (written with plain 16-byte stores instead of
     // the TMA box): 304 channels run as 2 x 160 columns instead of 2 x 192 - a sixth less MMA work on the decoder's data gradient
-    static const int env_nt = [] { const char* e = getenv("ISWM_CONV_NARROW_TAIL"); return e ? atoi(e) : 1; }();
-    if (env_nt && !(d->flags & (ISWM_EPI_STATS | ISWM_EPI_RESIDUAL | ISWM_EPI_BN_DZ)) && (d->Cout % 8) == 0)
+    if (!(d->flags & (ISWM_EPI_STATS | ISWM_EPI_RESIDUAL)) && (d->Cout % 8) == 0)
       BN = std::min(BN, (((d->Cout + nt - 1) / nt + 31) / 32) * 32);
     p.narrow_tail = (BN % 64) != 0 ? 1 : 0;
   }
@@ -825,25 +704,13 @@ static int conv_igemm_launch(const iswm_conv_desc* d, const void* d_in, const vo
                    (reinterpret_cast<uintptr_t>(d_out) & 15) == 0) ? 1 : 0;
   ISWM_REQUIRE(!(d->flags & ISWM_EPI_RESIDUAL) || (reinterpret_cast<uintptr_t>(d_res) & 15) == 0 || (d->res_ld & 7) != 0,
                "conv_igemm: a residual with res_ld %% 8 == 0 must be 16-byte aligned");
-  ISWM_REQUIRE(!(d->flags & (ISWM_EPI_STATS | ISWM_EPI_BN_DZ)) || p.use_tma_out, "conv_igemm: STATS / BN_DZ need a bf16 output with out_ld %% 8 == 0 and a 16-byte aligned base");
-  ISWM_REQUIRE(!(d->flags & ISWM_EPI_BN_DZ) || bn, "conv_igemm: BN_DZ without its descriptor");
-  int fixed = 1024 /*align*/ + 256 /*barriers*/ + ((d->flags & (ISWM_EPI_AFFINE | ISWM_EPI_BN_DZ)) ? 2048 : 0);
-  // Epilogue warpgroups: two. A third one for short-K (epilogue-bound) convolutions was measured and LOST (cfg2
-  // 16.05 vs 15.64 ms/step, cfg4 27.1 vs 26.5): it costs a ring stage and 40 registers per thread, and the epilogue is
-  // paced by TMEM-read and barrier latency rather than by warp count. ISWM_CONV_NWG=3 / ISWM_CONV_NWG3_MAXK=<k-blocks>
-  // re-enable it for experiments.
-  static const int env_nwg = [] { const char* e = getenv("ISWM_CONV_NWG"); return e ? atoi(e) : 2; }();
-  static const int env_rpf = [] { const char* e = getenv("ISWM_RES_PREFETCH"); return e ? atoi(e) : -1; }();
-  static const int env_k3 = [] { const char* e = getenv("ISWM_CONV_NWG3_MAXK"); return e ? atoi(e) : 16; }();
-  int nwg = (env_nwg == 3 || (env_nwg == 0 && d->ntaps * p.kchunks <= env_k3)) ? 3 : 2;
-  if (d->flags & ISWM_EPI_BN_DZ) nwg = 2;
-  if (p.use_tma_out) fixed += nwg * kStageBuf;
+  ISWM_REQUIRE(!(d->flags & ISWM_EPI_STATS) || p.use_tma_out, "conv_igemm: STATS needs a bf16 output with out_ld %% 8 == 0 and a 16-byte aligned base");
+  int fixed = 1024 /*align*/ + 256 /*barriers*/ + ((d->flags & ISWM_EPI_AFFINE) ? 2048 : 0);
+  if (p.use_tma_out) fixed += kEpiWG * kStageBuf;
   // epilogue-bound (short-K) convolutions hide the residual read behind a shared-memory prefetch; long-K ones keep
   // the ring stage instead and load the residual directly under the TMEM read
-  p.res_prefetch = ((d->flags & (ISWM_EPI_RESIDUAL | ISWM_EPI_BN_DZ)) && (d->res_ld % 8) == 0 && d->ntaps * p.kchunks <= 16) ? 1 : 0;
-  if (env_rpf == 0) p.res_prefetch = 0;
-  if (env_rpf == 2 && nwg == 3) p.res_prefetch = 0;      // 2: prefetch only with two warpgroups
-  if (p.res_prefetch) fixed += nwg * kStageBuf;
+  p.res_prefetch = ((d->flags & ISWM_EPI_RESIDUAL) && (d->res_ld % 8) == 0 && d->ntaps * p.kchunks <= 16) ? 1 : 0;
+  if (p.res_prefetch) fixed += kEpiWG * kStageBuf;
   p.stages = std::max(2, std::min(kMaxStages, (kSmemMax - fixed) / stage_bytes));
   p.flags = d->flags;
   p.n_img_per_phase = B;
@@ -875,7 +742,6 @@ static int conv_igemm_launch(const iswm_conv_desc* d, const void* d_in, const vo
   p.stats = d_stats;
   p.stats_rep = ((d->flags & ISWM_EPI_STATS) && d->stats_replicas > 1) ? d->stats_replicas : 1;
   ISWM_REQUIRE(p.stats_rep <= 64, "conv_igemm: stats_replicas=%d (at most 64)", d->stats_replicas);
-  if (bn) { p.bn_mean = bn->mean; p.bn_invstd = bn->invstd; p.bn_gamma = bn->gamma; p.bn_beta = bn->beta; }
   p.abort_flag = abort_flag;
 
   CUtensorMap tmap_a, tmap_b;
@@ -916,9 +782,7 @@ static int conv_igemm_launch(const iswm_conv_desc* d, const void* d_in, const vo
   const int smem_bytes = p.stages * stage_bytes + fixed;
   static bool attr_set = false;
   if (!attr_set) {
-    cudaError_t e = cudaFuncSetAttribute(conv_igemm_kernel<2, false>, cudaFuncAttributeMaxDynamicSharedMemorySize, 232448);
-    if (e == cudaSuccess) e = cudaFuncSetAttribute(conv_igemm_kernel<3, false>, cudaFuncAttributeMaxDynamicSharedMemorySize, 232448);
-    if (e == cudaSuccess) e = cudaFuncSetAttribute(conv_igemm_kernel<2, true>, cudaFuncAttributeMaxDynamicSharedMemorySize, 232448);
+    const cudaError_t e = cudaFuncSetAttribute(conv_igemm_kernel, cudaFuncAttributeMaxDynamicSharedMemorySize, 232448);
     ISWM_REQUIRE(e == cudaSuccess, "conv_igemm: cudaFuncSetAttribute: %s", cudaGetErrorString(e));
     static_assert(kSmemMax == 232448, "opt-in shared memory limit of sm_100");
     attr_set = true;
@@ -934,16 +798,9 @@ static int conv_igemm_launch(const iswm_conv_desc* d, const void* d_in, const vo
     p.s_tb = r;
   }
   // second producer warp: pays off when a k-block's MMA time (128 x BN x 64) is short against the ~300-cycle issue path of
-  // one producer thread, i.e. for narrow N tiles; ISWM_CONV_NPROD=1/2 forces it
-  static const int env_np = [] { const char* e = getenv("ISWM_CONV_NPROD"); return e ? atoi(e) : 0; }();
-  p.nprod = (env_np == 1 || env_np == 2) ? env_np : ((BN <= 128 && p.stages >= 4 && nwg == 2) ? 2 : 1);
-  if (nwg != 2) p.nprod = 1;                              // with three epilogue warpgroups warp 3 does not exist as a spare
-  if (d->flags & ISWM_EPI_BN_DZ)
-    launch_k(conv_igemm_kernel<2, true>, dim3(grid), dim3(384), smem_bytes, static_cast<cudaStream_t>(stream), tmap_a, tmap_b, tmap_out, p);
-  else if (nwg == 3)
-    launch_k(conv_igemm_kernel<3, false>, dim3(grid), dim3(512), smem_bytes, static_cast<cudaStream_t>(stream), tmap_a, tmap_b, tmap_out, p);
-  else
-    launch_k(conv_igemm_kernel<2, false>, dim3(grid), dim3(384), smem_bytes, static_cast<cudaStream_t>(stream), tmap_a, tmap_b, tmap_out, p);
+  // one producer thread, i.e. for narrow N tiles
+  p.nprod = (BN <= 128 && p.stages >= 4) ? 2 : 1;
+  launch_k(conv_igemm_kernel, dim3(grid), dim3(kConvThreads), smem_bytes, static_cast<cudaStream_t>(stream), tmap_a, tmap_b, tmap_out, p);
   return check_launch("conv_igemm");
 }
 

@@ -22,7 +22,6 @@
 #include <algorithm>
 #include <array>
 #include <cmath>
-#include <stdlib.h>
 #include <vector>
 
 namespace iswm {
@@ -579,11 +578,10 @@ extern "C" int iswm_conv_wgrad_ex(const iswm_conv_desc* d, const void* d_in, con
   p.T = d->ntaps * p.cchunks;
   p.tail_cols = (d->Cin % 64) ? (((d->Cin % 64) + 15) / 16) * 16 : 64;
   {
-    // chunks per tile, by a small cost model fitted to tools/wgrad_g_sweep.py: a CTA streams its share of the pixel blocks at
+    // chunks per tile, by a small cost model fitted to the sweep recorded in DESIGN.md: a CTA streams its share of the pixel blocks at
     // max(MMA time, operand bytes at ~100 B/clk of L2 -> SM ingest) per block, then adds its partial tile into dW with
     // red.global (~2 TB/s device-wide, and EVERY split flushes the whole tile): wide tiles re-read dy less but need more
     // splits to fill the SMs, i.e. more reduction traffic - 1x1 and small 3x3 layers end up at 2 chunks, the decoder at 4-5.
-    static const int env_g = [] { const char* e = getenv("ISWM_WGRAD_G"); return e ? atoi(e) : 0; }();
     int G = 1;
     double best = 1e30;
     for (int g = 1; g <= std::min(kMaxG, p.T); g++) {
@@ -603,7 +601,6 @@ extern "C" int iswm_conv_wgrad_ex(const iswm_conv_desc* d, const void* d_in, con
       const double cost = t_stream + t_flush + ((p.T % g) ? 0.03 * t_stream : 0.0);
       if (cost < best) { best = cost; G = g; }
     }
-    if (env_g >= 1 && env_g <= kMaxG) G = std::min(env_g, p.T);
     p.G = G;
   }
   p.tiles_n = (p.T + p.G - 1) / p.G;
@@ -618,11 +615,9 @@ extern "C" int iswm_conv_wgrad_ex(const iswm_conv_desc* d, const void* d_in, con
     // split mode, ONE resident wave: as many splits as fit on the SMs next to each other. More CTAs than SMs (the former
     // "best fill of whole waves" rule picked e.g. 37 splits x 8 tiles = 2 waves) doubles the fp32 reduction traffic - every
     // CTA ends by adding its whole 128 x BN partial tile into dW with red.global, ~2 TB/s device-wide - for no gain in
-    // parallelism; measured sweep (tools/wgrad_split_sweep.py): 1024->256 at 32x32 32.8 -> 22.5 us, 2048->256 55.3 -> 31.6,
+    // parallelism; measured sweep (recorded in DESIGN.md): 1024->256 at 32x32 32.8 -> 22.5 us, 2048->256 55.3 -> 31.6,
     // 1024->2048 86.0 -> 66.6
-    int best = (int)std::max<int64_t>(1, std::min<int64_t>(pbs, sms / n_tiles));
-    static const int env_sp = [] { const char* e = getenv("ISWM_WGRAD_SPLITS"); return e ? atoi(e) : 0; }();
-    if (env_sp > 0) best = (int)std::min<int64_t>(env_sp, std::max<int64_t>(1, pbs));
+    const int best = (int)std::max<int64_t>(1, std::min<int64_t>(pbs, sms / n_tiles));
     p.split_len = (int)((pbs + best - 1) / best);
     p.splits = (int)((pbs + p.split_len - 1) / p.split_len);
     grid = (int)(n_tiles * p.splits);
@@ -636,8 +631,7 @@ extern "C" int iswm_conv_wgrad_ex(const iswm_conv_desc* d, const void* d_in, con
   const int stage_bytes = (2 + p.G) * kChunkBytes;
   p.stages = std::max(2, std::min(kWStages, kWSmemBudget / stage_bytes));
   p.n_img_per_phase = B;
-  static const int env_np = [] { const char* e = getenv("ISWM_WGRAD_NPROD"); return e ? atoi(e) : 0; }();
-  p.nprod = (env_np == 1 || env_np == 2) ? env_np : (p.stages >= 4 ? 2 : 1);
+  p.nprod = p.stages >= 4 ? 2 : 1;
   for (int t = 0; t < d->ntaps; t++) {
     p.dh[t] = d->dh[t]; p.dw[t] = d->dw[t]; p.phase[t] = d->phase[t];
     ISWM_REQUIRE(d->coff[t] == 0, "conv_wgrad: per-tap channel offsets are a forward / data-gradient feature");

@@ -651,186 +651,6 @@ bn_bwd_apply_kernel(const __nv_bfloat16* __restrict__ dout, int dout_ld,
   }
 }
 
-// BatchNorm backward, both passes in ONE launch: every block reduces its rows (pass 1), all blocks meet at a grid
-// barrier, then every block re-reads the SAME rows (still in L2 for all but the largest tensors) and writes dx
-// (pass 2). The grid is sized to be co-resident (<= 3 blocks per SM, enforced by the launch bounds), so the spin
-// barrier cannot deadlock; it is bounded anyway and records an abort code instead of hanging.
-__device__ __forceinline__ void bn_grid_barrier(unsigned* counter, unsigned nblocks, int* abort_flag) {
-  __threadfence();                       // this thread's fp64 atomics are visible device-wide before the block signals
-  __syncthreads();
-  if (threadIdx.x == 0) {
-    atomicAdd(counter, 1u);
-    const long long t0 = clock64();
-    while (true) {
-      unsigned v;
-      asm volatile("ld.acquire.gpu.global.u32 %0, [%1];" : "=r"(v) : "l"(counter) : "memory");
-      if (v >= nblocks) break;
-      __nanosleep(64);
-      if (clock64() - t0 > 4000000000ll) { atomicCAS(abort_flag, 0, 21); break; }
-    }
-  }
-  __syncthreads();
-}
-
-template <int MASK, bool DROP, bool DZ>
-__global__ void __launch_bounds__(kT, 3)
-bn_bwd_fused_kernel(const __nv_bfloat16* __restrict__ dout, int dout_ld,
-                    const __nv_bfloat16* __restrict__ x, int x_ld,
-                    const __nv_bfloat16* __restrict__ act, int act_ld, int64_t M, int C,
-                    const float* __restrict__ gamma, const float* __restrict__ beta, const float* __restrict__ mean,
-                    const float* __restrict__ invstd, double* sums, float drop_p, DropSeed drop_seed_in,
-                    __nv_bfloat16* __restrict__ dx, int dx_ld, __nv_bfloat16* __restrict__ dz, int dz_ld,
-                    float* dgamma, float* dbeta, int nx, int ny, int rows_per_block, int* abort_flag) {
-  pdl_wait();
-  pdl_launch();
-  const uint64_t drop_seed = DROP ? drop_seed_in.resolve() : 0ull;
-  __shared__ float s_red[kT * 16];
-  const int tx = threadIdx.x % nx, ty = threadIdx.x / nx;
-  const int c0 = tx << 3;
-  const float keep_scale = DROP ? 1.f / (1.f - drop_p) : 1.f;
-  const RowWalk w = (ty < ny) ? row_walk(M, rows_per_block, ty, ny) : RowWalk{0, 0};
-  const int64_t sg = (int64_t)ny * dout_ld, sx = (int64_t)ny * x_ld, sa_ = (int64_t)ny * act_ld;
-  const uint64_t sd = (uint64_t)ny * C;
-  float kk[8], sh[8];                      // k = gamma * invstd doubles as the mask scale of the forward kernel
-#pragma unroll
-  for (int j = 0; j < 8; j++) {
-    kk[j] = gamma[c0 + j] * invstd[c0 + j];
-    sh[j] = (MASK == 2) ? fmaf(-mean[c0 + j], kk[j], beta[c0 + j]) : 0.f;
-  }
-  auto masked = [&](const uint4& gr, const F8& xv, const uint4& orr, uint64_t di) -> F8 {
-    F8 g = unpack8(gr);
-    if (MASK == 1) {
-      const F8 o = unpack8(orr);
-#pragma unroll
-      for (int j = 0; j < 8; j++) g.v[j] = (o.v[j] > 0.f) ? g.v[j] : 0.f;
-    } else if (MASK == 2) {
-#pragma unroll
-      for (int j = 0; j < 8; j++) g.v[j] = (fmaf(xv.v[j], kk[j], sh[j]) > 0.f) ? g.v[j] : 0.f;
-    }
-    if (DROP) {
-#pragma unroll
-      for (int j = 0; j < 8; j++) g.v[j] = drop_keep(drop_seed, di + j, drop_p) ? g.v[j] * keep_scale : 0.f;
-    }
-    return g;
-  };
-  constexpr int U = 4;
-  // ---------------- pass 1: sum(dz), sum(dz * x) over this block's rows
-  {
-    float a[8], b[8];
-#pragma unroll
-    for (int j = 0; j < 8; j++) { a[j] = 0.f; b[j] = 0.f; }
-    const __nv_bfloat16* pg = dout + w.first * dout_ld + c0;
-    const __nv_bfloat16* px = x + w.first * x_ld + c0;
-    const __nv_bfloat16* pa = (MASK == 1) ? act + w.first * act_ld + c0 : nullptr;
-    uint64_t didx = (uint64_t)w.first * C + c0;
-    auto one = [&](const uint4& gr, const uint4& xr, const uint4& orr, uint64_t di) {
-      const F8 xv = unpack8(xr);
-      const F8 g = masked(gr, xv, orr, di);
-#pragma unroll
-      for (int j = 0; j < 8; j++) {
-        a[j] += g.v[j];
-        b[j] = fmaf(g.v[j], xv.v[j], b[j]);
-      }
-    };
-    int i = 0;
-    for (; i + U <= w.n; i += U) {
-      uint4 gr[U], xr[U], orr[U];
-#pragma unroll
-      for (int u = 0; u < U; u++) {
-        gr[u] = load_raw(pg + u * sg);
-        xr[u] = load_raw(px + u * sx);
-        if (MASK == 1) orr[u] = load_raw(pa + u * sa_); else orr[u] = gr[u];
-      }
-#pragma unroll
-      for (int u = 0; u < U; u++) one(gr[u], xr[u], orr[u], didx + u * sd);
-      pg += U * sg; px += U * sx; didx += U * sd;
-      if (MASK == 1) pa += U * sa_;
-    }
-    for (; i < w.n; i++) {
-      const uint4 gr = load_raw(pg), xr = load_raw(px);
-      uint4 orr = gr;
-      if (MASK == 1) orr = load_raw(pa);
-      one(gr, xr, orr, didx);
-      pg += sg; px += sx; didx += sd;
-      if (MASK == 1) pa += sa_;
-    }
-#pragma unroll
-    for (int j = 0; j < 8; j++) {
-      s_red[threadIdx.x * 16 + j] = a[j];
-      s_red[threadIdx.x * 16 + 8 + j] = b[j];
-    }
-    __syncthreads();
-    for (int o = threadIdx.x; o < nx * 8; o += kT) {
-      const int gx = o >> 3, j = o & 7;
-      float ta = 0.f, tb = 0.f;
-      for (int y = 0; y < ny; y++) {
-        ta += s_red[(y * nx + gx) * 16 + j];
-        tb += s_red[(y * nx + gx) * 16 + 8 + j];
-      }
-      const int c = (gx << 3) + j;
-      atomicAdd(sums + c, (double)ta);
-      atomicAdd(sums + C + c, (double)invstd[c] * ((double)tb - (double)mean[c] * (double)ta));
-    }
-  }
-  bn_grid_barrier(reinterpret_cast<unsigned*>(sums + 2 * C), gridDim.x, abort_flag);
-  if (ty >= ny) return;
-  // ---------------- pass 2: dx = k*dz + p*x + q  with  p = -k*invstd*mean(dz*xhat), q = -k*mean(dz) - p*mu
-  const float invM = 1.0f / (float)M;
-  float pp[8], qq[8];
-#pragma unroll
-  for (int j = 0; j < 8; j++) {
-    const int c = c0 + j;
-    const float sa = (float)__ldcg(sums + c), sb = (float)__ldcg(sums + C + c);
-    const float ma = sa * invM, mb = sb * invM;
-    pp[j] = -kk[j] * invstd[c] * mb;
-    qq[j] = -kk[j] * ma - pp[j] * mean[c];
-    if (blockIdx.x == 0 && ty == 0) {
-      if (dbeta) dbeta[c] += sa;
-      if (dgamma) dgamma[c] += sb;
-    }
-  }
-  const __nv_bfloat16* pg = dout + w.first * dout_ld + c0;
-  const __nv_bfloat16* px = x + w.first * x_ld + c0;
-  const __nv_bfloat16* pa = (MASK == 1) ? act + w.first * act_ld + c0 : nullptr;
-  __nv_bfloat16* pdx = dx + w.first * dx_ld + c0;
-  __nv_bfloat16* pdz = DZ ? dz + w.first * dz_ld + c0 : nullptr;
-  const int64_t sdx = (int64_t)ny * dx_ld, sdz = (int64_t)ny * dz_ld;
-  uint64_t didx = (uint64_t)w.first * C + c0;
-  auto two = [&](const uint4& gr, const uint4& xr, const uint4& orr, __nv_bfloat16* odx, __nv_bfloat16* odz, uint64_t di) {
-    const F8 xv = unpack8(xr);
-    const F8 g = masked(gr, xv, orr, di);
-    if (DZ) store8(odz, g);
-    F8 r;
-#pragma unroll
-    for (int j = 0; j < 8; j++) r.v[j] = fmaf(kk[j], g.v[j], fmaf(pp[j], xv.v[j], qq[j]));
-    store8(odx, r);
-  };
-  int i = 0;
-  for (; i + U <= w.n; i += U) {
-    uint4 gr[U], xr[U], orr[U];
-#pragma unroll
-    for (int u = 0; u < U; u++) {
-      gr[u] = load_raw(pg + u * sg);
-      xr[u] = load_raw(px + u * sx);
-      if (MASK == 1) orr[u] = load_raw(pa + u * sa_); else orr[u] = gr[u];
-    }
-#pragma unroll
-    for (int u = 0; u < U; u++) two(gr[u], xr[u], orr[u], pdx + u * sdx, DZ ? pdz + u * sdz : nullptr, didx + u * sd);
-    pg += U * sg; px += U * sx; pdx += U * sdx; didx += U * sd;
-    if (MASK == 1) pa += U * sa_;
-    if (DZ) pdz += U * sdz;
-  }
-  for (; i < w.n; i++) {
-    const uint4 gr = load_raw(pg), xr = load_raw(px);
-    uint4 orr = gr;
-    if (MASK == 1) orr = load_raw(pa);
-    two(gr, xr, orr, pdx, pdz, didx);
-    pg += sg; px += sx; pdx += sdx; didx += sd;
-    if (MASK == 1) pa += sa_;
-    if (DZ) pdz += sdz;
-  }
-}
-
 // ---------------------------------------------------------------------------
 // stem im2col: NCHW fp32 image -> [B*Ho*Wo][Kpad] bf16, col = (r*7+s)*Cin + c.
 // One block per (image, output row, 64-pixel strip): the 7-row input patch is staged in shared memory with
@@ -1733,9 +1553,8 @@ extern "C" int iswm_bn_train_apply(const void* d_x, int x_ld, const double* d_st
   int nx, ny, rpb, blocks;
   // blocks per SM the row range is cut for: 3 = exactly the resident blocks (80 registers x 256 threads), ONE wave.
   // Measured on B200 against 6 (two waves): 33.6 MB tensor 17.1 -> 12.3 us, 67 MB 30.0 -> 24.9 us, cfg2 1074 -> 1088
-  // img/s: a second wave is mostly a tail (each thread's life is one or two batches of loads). ISWM_BN_WAVES overrides.
-  static const int env_waves = [] { const char* e = getenv("ISWM_BN_WAVES"); return e ? atoi(e) : 3; }();
-  bn_row_grid(C, M, 4, nx, ny, rpb, blocks, env_waves);
+  // img/s: a second wave is mostly a tail (each thread's life is one or two batches of loads).
+  bn_row_grid(C, M, 4, nx, ny, rpb, blocks, 3);
   const bool has_res = d_res != nullptr, has_drop = drop_p > 0.f;
 #define ISWM_BN_APPLY(R, L, D)                                                                                     \
   launch_k(bn_train_apply_kernel<R, L, D>, dim3(blocks), dim3(kT), 0, ST(stream), BF(d_x), x_ld, d_stats, std::max(1, stats_replicas), M, C,    \
@@ -1773,19 +1592,16 @@ extern "C" int iswm_bn_bwd_reduce(const void* d_dout, int dout_ld, const void* d
   ISWM_REQUIRE(relu != 2 || d_out_act, "bn_bwd_reduce: relu mode 2 needs the packed sign bits in d_out_act");
   ISWM_REQUIRE(C <= 2048, "bn_bwd_reduce: C=%d > 2048 not supported", C);
   int nx, ny, rows_per_block, blocks, groups = 1;
-  static const int env_groups = [] { const char* e = getenv("ISWM_BN_RED_GROUPS"); return e ? atoi(e) : 1; }();
-  if (env_groups && C > 256) {
+  if (C > 256) {
     // channel groups of 256 (32 threads x 8 channels, 512 contiguous bytes per row) x row blocks, one resident wave in all
     nx = 32; ny = kT / nx;
     groups = (C / 8 + nx - 1) / nx;
     int64_t want = (M + (int64_t)ny * 8 - 1) / ((int64_t)ny * 8);
-    static const int env_rw0 = [] { const char* e = getenv("ISWM_BN_RED_WAVES"); return e ? atoi(e) : 3; }();
-    want = std::max<int64_t>(1, std::min<int64_t>(want, std::max(1, num_sms() * env_rw0 / groups)));
+    want = std::max<int64_t>(1, std::min<int64_t>(want, std::max(1, num_sms() * 3 / groups)));
     rows_per_block = (int)((M + want - 1) / want);
     blocks = (int)((M + rows_per_block - 1) / rows_per_block);
   } else {
-    static const int env_rw = [] { const char* e = getenv("ISWM_BN_RED_WAVES"); return e ? atoi(e) : 3; }();
-    bn_row_grid(C, M, 8, nx, ny, rows_per_block, blocks, env_rw);   // one wave: every block ends with fp64 atomics on the same 2C addresses
+    bn_row_grid(C, M, 8, nx, ny, rows_per_block, blocks, 3);   // one wave: every block ends with fp64 atomics on the same 2C addresses
   }
   const int mask = !relu ? 0 : (relu == 2 ? 3 : (d_out_act ? 1 : 2));
   const bool has_drop = drop_p > 0.f;
@@ -1814,8 +1630,7 @@ extern "C" int iswm_bn_bwd_apply(const void* d_dout, int dout_ld, const void* d_
   ISWM_REQUIRE(!d_dz || (dz_ld % 8) == 0, "bn_bwd_apply: dz_ld");
   ISWM_REQUIRE(C <= 2048, "bn_bwd_apply: C=%d > 2048 not supported", C);
   int nx, ny, rpb, blocks;
-  static const int env_waves = [] { const char* e = getenv("ISWM_BN_WAVES"); return e ? atoi(e) : 3; }();   // see iswm_bn_train_apply
-  bn_row_grid(C, M, 4, nx, ny, rpb, blocks, env_waves);
+  bn_row_grid(C, M, 4, nx, ny, rpb, blocks, 3);   // one wave, see iswm_bn_train_apply
   const int mask = !relu ? 0 : (relu == 2 ? 3 : (d_out_act ? 1 : 2));
   const bool has_drop = drop_p > 0.f, has_dz = d_dz != nullptr;
 #define ISWM_BN_BAP(MK, D, Z)                                                                                          \
@@ -1829,40 +1644,6 @@ extern "C" int iswm_bn_bwd_apply(const void* d_dout, int dout_ld, const void* d_
 #undef ISWM_BN_BAP_M
 #undef ISWM_BN_BAP
   return check_launch("bn_bwd_apply");
-}
-
-namespace iswm { int* abort_flag_ptr(); }   // tc_host.cu
-
-extern "C" int iswm_bn_bwd(const void* d_dout, int dout_ld, const void* d_x, int x_ld,
-                           const void* d_out_act, int act_ld, int64_t M, int C,
-                           const float* d_gamma, const float* d_beta, const float* d_save_mean,
-                           const float* d_save_invstd, double* d_sums, int relu, float drop_p, uint64_t drop_seed, const int64_t* d_drop_step,
-                           void* d_dx, int dx_ld, void* d_dz, int dz_ld, float* d_dgamma,
-                           float* d_dbeta, void* stream) {
-  REQ_C8(C, "bn_bwd"); REQ_LD8(dout_ld, "bn_bwd"); REQ_LD8(x_ld, "bn_bwd"); REQ_LD8(dx_ld, "bn_bwd");
-  ISWM_REQUIRE(d_dout && d_x && d_gamma && d_save_mean && d_save_invstd && d_sums && d_dx && M > 0, "bn_bwd: null/empty");
-  ISWM_REQUIRE(relu == 0 || relu == 1, "bn_bwd: relu mode %d (the packed-bit mask is a two-kernel feature)", relu);
-  ISWM_REQUIRE(!relu || (d_out_act && (act_ld % 8) == 0) || (!d_out_act && d_beta),
-               "bn_bwd: relu needs the activation (or beta to recompute the mask)");
-  ISWM_REQUIRE(!d_dz || (dz_ld % 8) == 0, "bn_bwd: dz_ld");
-  ISWM_REQUIRE(C <= 2048, "bn_bwd: C=%d > 2048 not supported", C);
-  int* abort_flag = iswm::abort_flag_ptr();
-  ISWM_REQUIRE(abort_flag, "bn_bwd: cannot allocate abort flag");
-  int nx, ny, rpb, blocks;
-  bn_row_grid(C, M, 4, nx, ny, rpb, blocks, 3);     // <= 3 blocks per SM: the whole grid is co-resident (grid barrier)
-  const int mask = !relu ? 0 : (d_out_act ? 1 : 2);
-  const bool has_drop = drop_p > 0.f, has_dz = d_dz != nullptr;
-#define ISWM_BN_F(MK, D, Z)                                                                                             \
-  launch_k(bn_bwd_fused_kernel<MK, D, Z>, dim3(blocks), dim3(kT), 0, ST(stream), BF(d_dout), dout_ld, BF(d_x), x_ld,     \
-           BF(d_out_act), act_ld, M, C, d_gamma, d_beta, d_save_mean, d_save_invstd, d_sums, drop_p, DropSeed{drop_seed, reinterpret_cast<const long long*>(d_drop_step)},         \
-           BFW(d_dx), dx_ld, BFW(d_dz), dz_ld, d_dgamma, d_dbeta, nx, ny, rpb, abort_flag)
-#define ISWM_BN_F_M(D, Z) \
-  do { if (mask == 0) ISWM_BN_F(0, D, Z); else if (mask == 1) ISWM_BN_F(1, D, Z); else ISWM_BN_F(2, D, Z); } while (0)
-  if (has_drop) { if (has_dz) ISWM_BN_F_M(true, true); else ISWM_BN_F_M(true, false); }
-  else          { if (has_dz) ISWM_BN_F_M(false, true); else ISWM_BN_F_M(false, false); }
-#undef ISWM_BN_F_M
-#undef ISWM_BN_F
-  return check_launch("bn_bwd");
 }
 
 extern "C" int iswm_stem_im2col(const float* d_img, int B, int Cin, int H, int W, int Ho, int Wo,

@@ -3,8 +3,6 @@
 #include "common.cuh"
 #include <stdarg.h>
 #include <stdlib.h>
-#include <mutex>
-#include <unordered_set>
 
 namespace iswm {
 static thread_local char t_err[512] = "";
@@ -23,23 +21,6 @@ bool pdl_enabled() {
     return !(e && e[0] == '0');
   }();
   return on;
-}
-void ensure_carveout(const void* kernel) {
-  // measured on B200 (r2f): OFF is faster - with the maximum-shared split the BatchNorm kernels lose their L1 and run 12-19 %
-  // slower (bn_train_apply 1.58 -> 1.89 ms per cfg2 step) while the convolution launches do not move, so the carve-out switch
-  // at a kernel boundary is not what the per-launch overhead consists of. ISWM_CARVEOUT=1 re-enables it for experiments.
-  static const bool on = [] {
-    const char* e = getenv("ISWM_CARVEOUT");
-    return e && e[0] == '1';
-  }();
-  if (!on) return;
-  static std::mutex mu;
-  static std::unordered_set<const void*> done;
-  std::lock_guard<std::mutex> lk(mu);
-  if (done.insert(kernel).second) {
-    if (cudaFuncSetAttribute(kernel, cudaFuncAttributePreferredSharedMemoryCarveout, cudaSharedmemCarveoutMaxShared) != cudaSuccess)
-      cudaGetLastError();                      // a hint only: never fail a launch over it
-  }
 }
 }  // namespace iswm
 

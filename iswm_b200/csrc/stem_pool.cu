@@ -1,34 +1,29 @@
-// stem_pool.cu — BatchNorm + ReLU + 3x3/s2 max pooling of the ResNet stem as ONE pass, forward and backward
+// stem_pool.cu — BatchNorm + ReLU + 3x3/s2 max pooling of the ResNet stem as ONE forward pass
 // (network/backbone/resnet.py:145-147: bn1 -> relu -> maxpool after the 7x7 convolution).
 //
-// Unfused, the 64-channel half-resolution stem activation (134 MB at cfg2) is written by the BatchNorm pass, read by the
-// pooling pass, and its gradient is written by the pooling backward and read twice by the BatchNorm backward. Here
-//   forward   reads the pre-BN convolution output (each element up to 4 times, from L1/L2), normalises + ReLUs on the fly,
-//             writes the pooled tensor and the per-channel argmax code (which of the 9 window positions won: first maximum in
-//             window order, the rule of maxpool_fwd_kernel)                                  -> the activation never exists
-//   backward  both BatchNorm passes gather the activation gradient of a 2x2 pixel block from the <= 4 pooled windows that
-//             cover it (argmax codes), gate it with the ReLU mask recomputed from the pre-BN value and reduce / apply
-//                                                                                           -> its gradient never exists
-// Same arithmetic as bn_train_apply / maxpool_fwd and maxpool_bwd / bn_bwd_reduce / bn_bwd_apply run one after the other
-// (the pooled values, codes and pre-BN gradients are bit-identical; the reduction sums differ by fp32 summation order).
+// Unfused, the 64-channel half-resolution stem activation (134 MB at cfg2) is written by the BatchNorm pass and read by the
+// pooling pass. Here the forward reads the pre-BN convolution output (each element up to 4 times, from L1/L2), normalises +
+// ReLUs on the fly, writes the pooled tensor and the per-channel argmax code (which of the 9 window positions won: first
+// maximum in window order, the rule of maxpool_fwd_kernel): the activation never exists. Same arithmetic as bn_train_apply
+// and maxpool_fwd run one after the other (the pooled values and codes are bit-identical). The backward runs maxpool_bwd,
+// bn_bwd_reduce and bn_bwd_apply on the argmax codes.
 #include "common.cuh"
 #include "ew_common.cuh"
 #include <math.h>
-#include <stdlib.h>
 
 namespace iswm {
 
 constexpr int kC = 64;          // stem width (8 channel groups of 8)
 
 struct StemBn {
-  const double* stats;          // forward: sum x, sum x^2 over the M stem pixels, `stats_rep` copies
+  const double* stats;          // sum x, sum x^2 over the M stem pixels, `stats_rep` copies
   int stats_rep;
   const float* gamma;
   const float* beta;
   float* running_mean;
   float* running_var;
   long long* nbt;
-  float* save_mean;             // forward: written; backward: read
+  float* save_mean;             // written for the backward's BatchNorm kernels
   float* save_invstd;
 };
 
@@ -117,264 +112,6 @@ stem_pool_fwd_kernel(const __nv_bfloat16* __restrict__ raw, StemBn bn, int B, in
   }
 }
 
-// Tiled form of the forward (ISWM_STEM_POOL_TILED=1; measured SLOWER than the gather form above, which stays the default): a block
-// normalises the (2 TPH + 1) x (2 TPW + 1) input pixels under a TPH x TPW tile of pooled outputs ONCE into shared memory
-// (bf16, what bn_train_apply would have stored; positions outside the image hold -inf, which never wins a strict `>`), then
-// every pooled output takes its nine candidates from there in window order. The gather form normalised every input element
-// 2.25 times with nine scattered 16-byte loads per output (92 us at cfg2 for 168 MB: 0.31 of the HBM peak); here an input
-// element is loaded and normalised 1.16 times, with coalesced 128-byte pixel rows - and the kernel takes 105 us: three
-// 40 KB blocks per SM, two block barriers per tile and a fill loop of dependent loads hide less latency than the gather
-// form's nine independent loads per thread at 75 registers. Pooled values and argmax codes are bit-identical (same
-// bn_relu_bf16, same first-maximum rule); kept as a tested alternative.
-constexpr int TPH = 4, TPW = 16;
-constexpr int TIH = 2 * TPH + 1, TIW = 2 * TPW + 1;
-
-__global__ void __launch_bounds__(kT)
-stem_pool_fwd_tiled_kernel(const __nv_bfloat16* __restrict__ raw, StemBn bn, int B, int H, int W, int Ho, int Wo, int64_t M,
-                           float eps, float momentum, int tiles_h, int tiles_w, __nv_bfloat16* __restrict__ out, uint8_t* __restrict__ idx) {
-  pdl_wait();
-  pdl_launch();
-  __shared__ double s_stat[2 * kC];
-  __shared__ uint4 s_act[TIH * TIW * 8];                // [input row][input column][channel group of 8] bf16
-  for (int i = threadIdx.x; i < 2 * kC; i += kT) {
-    double a = bn.stats[i];
-    for (int r = 1; r < bn.stats_rep; r++) a += bn.stats[(size_t)r * 2 * kC + i];
-    s_stat[i] = a;
-  }
-  __syncthreads();
-  const int cg = threadIdx.x & 7;                       // kT is a multiple of 8: a thread keeps its channel group in both phases
-  const int c0 = cg << 3;
-  const double invM = 1.0 / (double)M;
-  float sc[8], sh[8];
-#pragma unroll
-  for (int j = 0; j < 8; j++) {
-    const int c = c0 + j;
-    const double mean_d = s_stat[c] * invM;
-    const float mean = (float)mean_d;
-    const float var = fmaxf((float)(s_stat[kC + c] * invM - mean_d * mean_d), 0.f);
-    const float invstd = rsqrtf(var + eps);
-    sc[j] = bn.gamma[c] * invstd;
-    sh[j] = fmaf(-mean, sc[j], bn.beta[c]);
-    if (blockIdx.x == 0 && threadIdx.x < 8) {
-      bn.save_mean[c] = mean;
-      bn.save_invstd[c] = invstd;
-      if (bn.running_mean) {
-        const float unbiased = (M > 1) ? var * ((float)M / (float)(M - 1)) : var;
-        bn.running_mean[c] = (1.f - momentum) * bn.running_mean[c] + momentum * mean;
-        bn.running_var[c] = (1.f - momentum) * bn.running_var[c] + momentum * unbiased;
-      }
-    }
-  }
-  if (blockIdx.x == 0 && threadIdx.x == 0 && bn.nbt) *bn.nbt += 1;
-  const int tiles_per_img = tiles_h * tiles_w;
-  const int total_tiles = B * tiles_per_img;
-  const uint32_t ninf2 = 0xFF80FF80u;                   // two bf16 -inf
-  for (int tile = blockIdx.x; tile < total_tiles; tile += gridDim.x) {
-    const int b = tile / tiles_per_img, tr = tile - b * tiles_per_img;
-    const int ho0 = (tr / tiles_w) * TPH, wo0 = (tr % tiles_w) * TPW;
-    const int hi0 = 2 * ho0 - 1, wi0 = 2 * wo0 - 1;
-    const __nv_bfloat16* img = raw + (int64_t)b * H * W * kC + c0;
-    __syncthreads();                                    // the previous tile's readers are done with s_act
-    for (int it = threadIdx.x; it < TIH * TIW * 8; it += kT) {
-      const int px = it >> 3;
-      const int r = px / TIW, c = px - r * TIW;
-      const int hi = hi0 + r, wi = wi0 + c;
-      uint4 v = make_uint4(ninf2, ninf2, ninf2, ninf2);
-      if (hi >= 0 && hi < H && wi >= 0 && wi < W) {
-        const F8 x = unpack8(load_raw(img + ((int64_t)hi * W + wi) * kC));
-        v.x = pack_bf16x2(fmaxf(fmaf(x.v[0], sc[0], sh[0]), 0.f), fmaxf(fmaf(x.v[1], sc[1], sh[1]), 0.f));
-        v.y = pack_bf16x2(fmaxf(fmaf(x.v[2], sc[2], sh[2]), 0.f), fmaxf(fmaf(x.v[3], sc[3], sh[3]), 0.f));
-        v.z = pack_bf16x2(fmaxf(fmaf(x.v[4], sc[4], sh[4]), 0.f), fmaxf(fmaf(x.v[5], sc[5], sh[5]), 0.f));
-        v.w = pack_bf16x2(fmaxf(fmaf(x.v[6], sc[6], sh[6]), 0.f), fmaxf(fmaf(x.v[7], sc[7], sh[7]), 0.f));
-      }
-      s_act[it] = v;
-    }
-    __syncthreads();
-    for (int it = threadIdx.x; it < TPH * TPW * 8; it += kT) {
-      const int po = it >> 3;
-      const int pr = po / TPW, pc = po - pr * TPW;
-      const int ho = ho0 + pr, wo = wo0 + pc;
-      if (ho >= Ho || wo >= Wo) continue;
-      float best[8];
-      int arg[8];
-#pragma unroll
-      for (int j = 0; j < 8; j++) { best[j] = -INFINITY; arg[j] = 0; }
-#pragma unroll
-      for (int t = 0; t < 9; t++) {
-        const F8 v = unpack8(s_act[((2 * pr + t / 3) * TIW + 2 * pc + t % 3) * 8 + cg]);
-#pragma unroll
-        for (int j = 0; j < 8; j++)
-          if (v.v[j] > best[j]) { best[j] = v.v[j]; arg[j] = t; }
-      }
-      const int64_t m = ((int64_t)b * Ho + ho) * Wo + wo;
-      F8 o;
-#pragma unroll
-      for (int j = 0; j < 8; j++) o.v[j] = best[j];
-      store8(out + m * kC + c0, o);
-      uint2 pk;
-      pk.x = arg[0] | (arg[1] << 8) | (arg[2] << 16) | (arg[3] << 24);
-      pk.y = arg[4] | (arg[5] << 8) | (arg[6] << 16) | (arg[7] << 24);
-      *reinterpret_cast<uint2*>(idx + m * kC + c0) = pk;
-    }
-  }
-}
-
-// gradient of the (never stored) stem activation for the 2x2 pixel block (i, j) of image b, channels [c0, c0+8): sum of the
-// pooled gradients whose argmax code points at each pixel (the loop of maxpool_bwd_kernel)
-__device__ __forceinline__ void gather_block(const __nv_bfloat16* __restrict__ dpool, const uint8_t* __restrict__ idx, int b, int i, int j,
-                                             int Ho, int Wo, int c0, float (&acc)[2][2][8]) {
-#pragma unroll
-  for (int a = 0; a < 2; a++)
-#pragma unroll
-    for (int c = 0; c < 2; c++)
-#pragma unroll
-      for (int k = 0; k < 8; k++) acc[a][c][k] = 0.f;
-#pragma unroll
-  for (int dho = 0; dho < 2; dho++) {
-    const int ho = i + dho;
-    if (ho >= Ho) continue;
-#pragma unroll
-    for (int dwo = 0; dwo < 2; dwo++) {
-      const int wo = j + dwo;
-      if (wo >= Wo) continue;
-      const int64_t om = ((int64_t)b * Ho + ho) * Wo + wo;
-      const uint2 pk = *reinterpret_cast<const uint2*>(idx + om * kC + c0);
-      const F8 g = load8(dpool + om * kC + c0);
-#pragma unroll
-      for (int dy = dho; dy < 2; dy++) {
-        const int r = dho ? 0 : 1 + dy;
-#pragma unroll
-        for (int dxx = dwo; dxx < 2; dxx++) {
-          const int sx = dwo ? 0 : 1 + dxx;
-          const int code = r * 3 + sx;
-#pragma unroll
-          for (int k = 0; k < 8; k++) {
-            const int a = ((k < 4 ? pk.x : pk.y) >> (8 * (k & 3))) & 0xff;
-            if (a == code) acc[dy][dxx][k] += g.v[k];
-          }
-        }
-      }
-    }
-  }
-}
-
-// backward pass 1: sums[c] += sum dz, sums[64 + c] += sum dz * xhat over all stem pixels
-__global__ void __launch_bounds__(kT)
-stem_pool_bwd_reduce_kernel(const __nv_bfloat16* __restrict__ dpool, const uint8_t* __restrict__ idx, const __nv_bfloat16* __restrict__ raw,
-                            int B, int H, int W, int Ho, int Wo, const float* __restrict__ mean, const float* __restrict__ invstd,
-                            const float* __restrict__ gamma, const float* __restrict__ beta, double* __restrict__ sums) {
-  pdl_wait();
-  pdl_launch();
-  __shared__ float s_red[kT * 16];
-  const int cg = threadIdx.x & 7, c0 = cg << 3;
-  float sc[8], sh[8], a[8], bsum[8];
-#pragma unroll
-  for (int k = 0; k < 8; k++) {
-    sc[k] = gamma[c0 + k] * invstd[c0 + k];
-    sh[k] = fmaf(-mean[c0 + k], sc[k], beta[c0 + k]);
-    a[k] = 0.f; bsum[k] = 0.f;
-  }
-  const int Hb = (H + 1) >> 1, Wb = (W + 1) >> 1;
-  const int64_t total = (int64_t)B * Hb * Wb * 8;
-  for (int64_t it = (int64_t)blockIdx.x * kT + threadIdx.x; it < total; it += (int64_t)gridDim.x * kT) {
-    const int64_t m = it >> 3;
-    const int j = (int)(m % Wb), i = (int)((m / Wb) % Hb), b = (int)(m / ((int64_t)Wb * Hb));
-    float acc[2][2][8];
-    gather_block(dpool, idx, b, i, j, Ho, Wo, c0, acc);
-#pragma unroll
-    for (int dy = 0; dy < 2; dy++) {
-      const int hi = 2 * i + dy;
-      if (hi >= H) continue;
-#pragma unroll
-      for (int dxx = 0; dxx < 2; dxx++) {
-        const int wi = 2 * j + dxx;
-        if (wi >= W) continue;
-        const F8 xv = load8(raw + (((int64_t)b * H + hi) * W + wi) * kC + c0);
-#pragma unroll
-        for (int k = 0; k < 8; k++) {
-          // the unfused pair rounds the pooling gradient to bf16 before BatchNorm reads it
-          const float g = __bfloat162float(__float2bfloat16_rn(acc[dy][dxx][k]));
-          const float gz = (fmaf(xv.v[k], sc[k], sh[k]) > 0.f) ? g : 0.f;
-          a[k] += gz;
-          bsum[k] = fmaf(gz, xv.v[k], bsum[k]);
-        }
-      }
-    }
-  }
-#pragma unroll
-  for (int k = 0; k < 8; k++) {
-    s_red[threadIdx.x * 16 + k] = a[k];
-    s_red[threadIdx.x * 16 + 8 + k] = bsum[k];
-  }
-  __syncthreads();
-  if (threadIdx.x < kC) {
-    const int c = threadIdx.x, g8 = c >> 3, k = c & 7;
-    float ta = 0.f, tb = 0.f;
-    for (int y = 0; y < kT / 8; y++) {
-      ta += s_red[(y * 8 + g8) * 16 + k];
-      tb += s_red[(y * 8 + g8) * 16 + 8 + k];
-    }
-    atomicAdd(sums + c, (double)ta);
-    atomicAdd(sums + kC + c, (double)invstd[c] * ((double)tb - (double)mean[c] * (double)ta));
-  }
-}
-
-// backward pass 2: dy (gradient of the pre-BN convolution output), dgamma / dbeta
-__global__ void __launch_bounds__(kT)
-stem_pool_bwd_apply_kernel(const __nv_bfloat16* __restrict__ dpool, const uint8_t* __restrict__ idx, const __nv_bfloat16* __restrict__ raw,
-                           int B, int H, int W, int Ho, int Wo, int64_t M, const float* __restrict__ mean, const float* __restrict__ invstd,
-                           const float* __restrict__ gamma, const float* __restrict__ beta, const double* __restrict__ sums,
-                           __nv_bfloat16* __restrict__ dy, float* dgamma, float* dbeta) {
-  pdl_wait();
-  pdl_launch();
-  const int cg = threadIdx.x & 7, c0 = cg << 3;
-  const float invM = 1.0f / (float)M;
-  float kk[8], pp[8], qq[8], sh[8];
-#pragma unroll
-  for (int k = 0; k < 8; k++) {
-    const int c = c0 + k;
-    const float is = invstd[c], mu = mean[c];
-    const float kf = gamma[c] * is;
-    sh[k] = fmaf(-mu, kf, beta[c]);
-    const float sa = (float)sums[c], sb = (float)sums[kC + c];
-    kk[k] = kf;
-    pp[k] = -kf * is * (sb * invM);
-    qq[k] = -kf * (sa * invM) - pp[k] * mu;
-    if (blockIdx.x == 0 && threadIdx.x < 8) {
-      if (dbeta) dbeta[c] += sa;
-      if (dgamma) dgamma[c] += sb;
-    }
-  }
-  const int Hb = (H + 1) >> 1, Wb = (W + 1) >> 1;
-  const int64_t total = (int64_t)B * Hb * Wb * 8;
-  for (int64_t it = (int64_t)blockIdx.x * kT + threadIdx.x; it < total; it += (int64_t)gridDim.x * kT) {
-    const int64_t m = it >> 3;
-    const int j = (int)(m % Wb), i = (int)((m / Wb) % Hb), b = (int)(m / ((int64_t)Wb * Hb));
-    float acc[2][2][8];
-    gather_block(dpool, idx, b, i, j, Ho, Wo, c0, acc);
-#pragma unroll
-    for (int dyy = 0; dyy < 2; dyy++) {
-      const int hi = 2 * i + dyy;
-      if (hi >= H) continue;
-#pragma unroll
-      for (int dxx = 0; dxx < 2; dxx++) {
-        const int wi = 2 * j + dxx;
-        if (wi >= W) continue;
-        const int64_t off = (((int64_t)b * H + hi) * W + wi) * kC + c0;
-        const F8 xv = load8(raw + off);
-        F8 r;
-#pragma unroll
-        for (int k = 0; k < 8; k++) {
-          const float g = __bfloat162float(__float2bfloat16_rn(acc[dyy][dxx][k]));
-          const float gz = (fmaf(xv.v[k], kk[k], sh[k]) > 0.f) ? g : 0.f;
-          r.v[k] = fmaf(kk[k], gz, fmaf(pp[k], xv.v[k], qq[k]));
-        }
-        store8(dy + off, r);
-      }
-    }
-  }
-}
-
 }  // namespace iswm
 
 using namespace iswm;
@@ -397,35 +134,7 @@ extern "C" int iswm_stem_pool_fwd(const void* d_raw, const iswm_bn_side* bn, int
   ISWM_REQUIRE(Ho == (H - 1) / 2 + 1 && Wo == (W - 1) / 2 + 1 && B >= 1, "stem_pool_fwd: 3x3 / stride 2 / pad 1 geometry expected");
   const StemBn sb{bn->stats, bn->stats_replicas > 1 ? bn->stats_replicas : 1, bn->gamma, bn->beta, bn->running_mean, bn->running_var,
                   reinterpret_cast<long long*>(bn->num_batches_tracked), bn->save_mean, bn->save_invstd};
-  const char* tiled_env = getenv("ISWM_STEM_POOL_TILED"); // measured slower than the gather form (DESIGN 3b): off unless asked for;
-  const bool tiled = tiled_env && tiled_env[0] == '1';    // read per call (one launch per step) so that a test can switch it in-process
-  if (tiled) {
-    const int tiles_h = (Ho + TPH - 1) / TPH, tiles_w = (Wo + TPW - 1) / TPW;
-    const int64_t tiles = (int64_t)B * tiles_h * tiles_w;
-    ISWM_REQUIRE(tiles < (1ll << 31), "stem_pool_fwd: too many tiles");
-    const int grid = (int)std::min<int64_t>(tiles, (int64_t)resident_grid(stem_pool_fwd_tiled_kernel, kT));
-    launch_k(stem_pool_fwd_tiled_kernel, dim3((unsigned)grid), dim3(kT), 0, ST(stream), BF(d_raw), sb, B, H, W, Ho, Wo, (int64_t)B * H * W, eps,
-             momentum, tiles_h, tiles_w, BFW(d_out), d_idx);
-  } else {
-    launch_k(stem_pool_fwd_kernel, dim3(stem_grid((int64_t)B * Ho * Wo * 8)), dim3(kT), 0, ST(stream), BF(d_raw), sb, B, H, W, Ho, Wo,
-             (int64_t)B * H * W, eps, momentum, BFW(d_out), d_idx);
-  }
+  launch_k(stem_pool_fwd_kernel, dim3(stem_grid((int64_t)B * Ho * Wo * 8)), dim3(kT), 0, ST(stream), BF(d_raw), sb, B, H, W, Ho, Wo,
+           (int64_t)B * H * W, eps, momentum, BFW(d_out), d_idx);
   return check_launch("stem_pool_fwd");
-}
-
-extern "C" int iswm_stem_pool_bwd(const void* d_dpool, const uint8_t* d_idx, const void* d_raw, const iswm_bn_side* bn,
-                                  int B, int H, int W, int C, int Ho, int Wo, double* d_sums, void* d_dy,
-                                  float* d_dgamma, float* d_dbeta, void* stream) {
-  if (debug_skip(ISWM_SKIP_BN)) return 0;
-  ISWM_REQUIRE(d_dpool && d_idx && d_raw && bn && d_sums && d_dy && bn->gamma && bn->beta && bn->save_mean && bn->save_invstd, "stem_pool_bwd: null argument");
-  ISWM_REQUIRE(C == kC, "stem_pool_bwd: C=%d (the stem has %d channels)", C, kC);
-  ISWM_REQUIRE(Ho == (H - 1) / 2 + 1 && Wo == (W - 1) / 2 + 1 && B >= 1, "stem_pool_bwd: 3x3 / stride 2 / pad 1 geometry expected");
-  const int64_t items = (int64_t)B * ((H + 1) / 2) * ((W + 1) / 2) * 8;
-  launch_k(stem_pool_bwd_reduce_kernel, dim3(stem_grid(items)), dim3(kT), 0, ST(stream), BF(d_dpool), d_idx, BF(d_raw), B, H, W, Ho, Wo,
-           (const float*)bn->save_mean, (const float*)bn->save_invstd, bn->gamma, bn->beta, d_sums);
-  if (int rc = check_launch("stem_pool_bwd (reduce)")) return rc;
-  launch_k(stem_pool_bwd_apply_kernel, dim3(stem_grid(items)), dim3(kT), 0, ST(stream), BF(d_dpool), d_idx, BF(d_raw), B, H, W, Ho, Wo,
-           (int64_t)B * H * W, (const float*)bn->save_mean, (const float*)bn->save_invstd, bn->gamma, bn->beta, (const double*)d_sums,
-           BFW(d_dy), d_dgamma, d_dbeta);
-  return check_launch("stem_pool_bwd (apply)");
 }

@@ -26,6 +26,12 @@ BN_MOMENTUM = 0.1
 # channels per pixel of the x-unrolled stem rows (21 used): 32 = 64-byte pixels; 24 (48-byte, sector-straddling pixels) makes the
 # TMA loads of the 7-tap convolution 2.3x slower (tools/prof_stem.py: 231 vs 99 us)
 STEM_KPITCH = 32
+# weight gradients of these backbone layers are collected while the layer's backward runs and launched as ONE grouped kernel
+# when it ends (iswm_conv_wgrad_grouped: a layer's 13-19 small GEMMs side by side need almost no pixel-range splits, i.e.
+# almost no partial-tile reductions; layer3 325 -> 192 us, layer2 282 -> 230 us, tools/prof_wgrad_group.py). layer1
+# (operands far larger than L2: every tile would stream them from HBM again: 319 -> 374 us) keeps one launch per
+# convolution. conv_wgrad 2.63 -> 2.28 ms/step, step 12.50 -> 12.42.
+GROUP_WGRAD_LAYERS = ("layer2", "layer3", "layer4")
 
 
 class _StreamCache:
@@ -56,7 +62,7 @@ class _StreamScope:
 class Act:
     """NHWC bf16 activation: `t` is a [B,H,W,C] view whose row pitch is `ld` elements."""
 
-    __slots__ = ("t", "B", "H", "W", "C", "ld", "grad", "pending", "masked_ok", "bn_fold", "bn_sums", "phase_view")
+    __slots__ = ("t", "B", "H", "W", "C", "ld", "grad", "pending", "masked_ok", "phase_view")
 
     def __init__(self, t: torch.Tensor, B: int, H: int, W: int, Cc: int, ld: int):
         self.t, self.B, self.H, self.W, self.C, self.ld = t, B, H, W, Cc, ld
@@ -65,11 +71,6 @@ class Act:
         # the block's conv1 data gradient adds it, gated by the bits, in its epilogue (ISWM_EPI_RES_MASK)
         self.pending = None
         self.masked_ok = False                        # set on block inputs whose only other consumer is that conv1
-        # BatchNorm-backward pass 1 folded into the producer of this activation's gradient (ISWM_EPI_BN_DZ): `bn_fold` =
-        # (raw, save, bn) is set by the unit that owns the activation when its ONLY consumer is a stride-1 convolution,
-        # `bn_sums` by that consumer's data gradient once it has written dz (not dout) into `grad` and accumulated the sums
-        self.bn_fold = None
-        self.bn_sums = None
         self.phase_view = False                       # (H, W) are per-phase dims of a dense [B, 2H, 2W, ld] tensor read in place (stride-2 convs)
 
     @property
@@ -129,51 +130,28 @@ class Engine:
         self.weights_epoch = 0        # bumped by optimisers that update parameters behind autograd's back
         self.flat_w = None            # fp32 flat master weights (parameters become views of it)
         self.batched_pack = True      # repack all weights in one launch when any changed
-        # BatchNorm backward as ONE launch (iswm_bn_bwd: pass 1, grid barrier, pass 2) for tensors up to this many
-        # elements. Measured on B200 (cfg2): 15.58 ms/step with 0 (two launches everywhere), 15.74 / 15.92 / 16.03 with
-        # 4 Mi / 16 Mi / all -> the barrier and the 3-blocks-per-SM cap cost more than the saved launch; off by default.
-        self.bn_fused_max_elems = int(__import__("os").environ.get("ISWM_BN_FUSED_MAX", "0"))
-        self.bn_fused_min_elems = int(__import__("os").environ.get("ISWM_BN_FUSED_MIN", str(1 << 62)))
+        # The attributes below select between two implementations of one step; tests and the benchmark set them to time or
+        # compare the other form. All default to the faster one.
         # weight gradients feed nothing inside the backward sweep: they run on a second stream so that their
         # (tensor-core) kernels overlap the HBM-bound BatchNorm kernels and the launch / fill / drain gaps of the
-        # data-gradient chain; ISWM_ASYNC_WGRAD=0 puts them back in line
-        self.async_wgrad = __import__("os").environ.get("ISWM_ASYNC_WGRAD", "1") != "0"
-        self.relu_bits = __import__("os").environ.get("ISWM_RELU_BITS", "1") != "0"
-        self.fwd_overlap = __import__("os").environ.get("ISWM_FWD_OVERLAP", "1") != "0"
-        self.batch_unpack = __import__("os").environ.get("ISWM_BATCH_UNPACK", "1") != "0"
+        # data-gradient chain; False puts them back in line
+        self.async_wgrad = True
+        # forward branches nothing on the main chain consumes for a while run on that second stream too (_fwd_fork)
+        self.fwd_overlap = True
+        # k x k weight gradients are unpacked in one launch at the end of the sweep (_unpack_all)
+        self.batch_unpack = True
         # ASPP backward: one K-concatenated data-gradient GEMM over the four conv branches (iswm_aspp_bwd) instead of four
         # launches with three read-modify-write passes over the 2048-channel feature gradient
-        self.aspp_fused_bwd = __import__("os").environ.get("ISWM_ASPP_FUSED_BWD", "1") != "0"
+        self.aspp_fused_bwd = True
         # identity-path gradient of non-first bottleneck blocks folded into the block's conv1 data-gradient epilogue
-        # (ISWM_EPI_RES_MASK) instead of a tensor written by bn_bwd_apply and read back (ISWM_MASKED_IDENTITY=0: old form)
-        self.masked_identity = __import__("os").environ.get("ISWM_MASKED_IDENTITY", "1") != "0"
-        # BatchNorm-backward reductions (sum dz, sum dz.xhat) of conv -> BN -> ReLU units with a single stride-1 consumer can ride
-        # on that consumer's data-gradient epilogue (iswm_conv_igemm_bn) instead of a bn_bwd_reduce pass. OFF by default: kernel by
-        # kernel it saves 4-27 us per unit (tools/prof_bndz.py), but inside the step it LOSES (cfg2 12.95 -> 13.17 ms): the eight
-        # epilogue warps pay ~800 extra instructions per 128x64 chunk, and the longer persistent data-gradient kernels leave the
-        # weight-gradient stream fewer HBM-bound BatchNorm windows to run under (ISWM_BN_DZ_FOLD=1 enables; DESIGN 3b)
-        self.bn_dz_fold = __import__("os").environ.get("ISWM_BN_DZ_FOLD", "0") != "0"
+        # (ISWM_EPI_RES_MASK) instead of a tensor written by bn_bwd_apply and read back
+        self.masked_identity = True
         # blocks with a downsample branch: the closing BatchNorm and the downsample BatchNorm run as ONE kernel per pass
         # (csrc/bn_dual.cu; the normalised shortcut is never written, backward reads dout / sign bits once per pass for both)
-        self.dual_bn = __import__("os").environ.get("ISWM_DUAL_BN", "1") != "0"
-        self.ds_bwd_late = __import__("os").environ.get("ISWM_DS_BWD_LATE", "1") != "0"
-        # stem 7x7/s2: the image unrolled along x only (iswm_stem_rows, 48 B per pixel row) + the 7 kernel rows as 7 taps of the
-        # implicit GEMM over the two row-parity phases, instead of a full im2col matrix (320 B per pixel) + one GEMM
-        # (ISWM_STEM_ROWS=0: the im2col form)
-        self.stem_rows = __import__("os").environ.get("ISWM_STEM_ROWS", "1") != "0"
+        self.dual_bn = True
         # stem tail (train): BatchNorm + ReLU + maxpool as one forward pass (csrc/stem_pool.cu: the half-resolution activation is
-        # never written; ISWM_STEM_POOL=0: separate kernels). The fused backward (ISWM_STEM_POOL_BWD=1) exists and is tested but loses
-        self.stem_pool = __import__("os").environ.get("ISWM_STEM_POOL", "1") != "0"
-        self.stem_pool_bwd = __import__("os").environ.get("ISWM_STEM_POOL_BWD", "0") != "0"
-        # stride-2 convolutions read the parity phases of their dense input in place through a 5-D tensor map
-        # (iswm_conv_desc.in_phase_view) instead of phase_split / subsample2 copies (ISWM_PHASE_VIEW=0: the copies)
-        self.phase_view = __import__("os").environ.get("ISWM_PHASE_VIEW", "1") != "0"
-        # weight gradients of these backbone layers are collected while the layer's backward runs and launched as ONE grouped
-        # kernel when it ends (iswm_conv_wgrad_grouped: a layer's 13-19 small GEMMs side by side need almost no pixel-range
-        # splits, i.e. almost no partial-tile reductions; layer3 325 -> 192 us, layer2 282 -> 230 us, tools/prof_wgrad_group.py).
-        # layer1 (operands far larger than L2: every tile would stream them from HBM again: 319 -> 374 us)
-        # keeps one launch per convolution. conv_wgrad 2.63 -> 2.28 ms/step, step 12.50 -> 12.42. ISWM_WGRAD_GROUP="" turns it off.
-        self.group_wgrad = tuple(x for x in __import__("os").environ.get("ISWM_WGRAD_GROUP", "layer2,layer3,layer4").split(",") if x)
+        # never written); False: separate kernels
+        self.stem_pool = True
         self._wq, self._wq_layer = [], None
         self._fwd_keep = []
         self._wstream = None
@@ -213,6 +191,13 @@ class Engine:
         self.dec1 = S("classifier.classifier.0", cl[0], cl[1], 3, 1, 1)
         self.dec2 = S("classifier.classifier.3", cl[3], cl[4], 3, 1, 1)
         self.cls = S("classifier.classifier.6", cl[6], None, 1, 1, 1)
+
+    @property
+    def stem_rows(self) -> bool:
+        """The stem 7x7/s2 runs on the image unrolled along x only (iswm_stem_rows, 48 B per pixel row) with the 7 kernel rows
+        as 7 taps of the implicit GEMM over the two row-parity phases, instead of a full im2col matrix (320 B per pixel) + one
+        GEMM; the im2col form serves inputs of more than 3 channels."""
+        return self.stem.cin <= 3
 
     def _spec(self, name, conv, bn, k, stride, dilation) -> ConvSpec:
         s = ConvSpec(name, conv, bn, k, stride, dilation)
@@ -372,7 +357,7 @@ class Engine:
 
     def _aspp_cat_slot(self):
         """name -> (first tap, total taps) of the ASPP conv branches inside the concatenated dgrad operand; empty when the
-        fused ASPP backward is off (ISWM_ASPP_FUSED_BWD=0) or the branch widths do not allow it."""
+        fused ASPP backward is off (aspp_fused_bwd = False) or the branch widths do not allow it."""
         d = getattr(self, "_aspp_slots", None)
         if d is None:
             d = {}
@@ -492,7 +477,9 @@ class Engine:
             return x, ops.conv_taps(s.k, s.dilation), x.B, x.H, x.W
         assert s.stride == 2 and s.dilation == 1
         Ho, Wo = (x.H + 1) // 2, (x.W + 1) // 2
-        if self.phase_view and x.H % 2 == 0 and x.W % 2 == 0 and x.C % 64 == 0 and x.ld % 8 == 0:
+        # stride-2 convolutions read the parity phases of their dense input in place through a 5-D tensor map
+        # (iswm_conv_desc.in_phase_view); odd sizes and misaligned channels go through phase_split / subsample2 copies
+        if x.H % 2 == 0 and x.W % 2 == 0 and x.C % 64 == 0 and x.ld % 8 == 0:
             xv = Act(x.t, x.B, Ho, Wo, x.C, x.ld)
             xv.phase_view = True
             return xv, (ops.conv_taps(1, 1) if s.k == 1 else ops.conv_taps_s2_3x3()), x.B, Ho, Wo
@@ -535,11 +522,8 @@ class Engine:
 
     # ------------------------------------------------------------------ train-mode unit: conv(+stats) -> BN apply, taped
     def _unit_train(self, s: ConvSpec, x: Act, relu=True, residual: Optional[Act] = None, out: Optional[Act] = None,
-                    drop_p: float = 0.0, need_dx: bool = True, dy_into: Optional[Callable[[], torch.Tensor]] = None,
-                    single_consumer: bool = False) -> Act:
-        """`single_consumer`: the caller promises that exactly one convolution reads this unit's output (so that convolution's
-        data gradient IS the whole gradient of the activation and may carry the BatchNorm-backward reductions).
-        `dy_into`: called in backward, returns the [B,Ho,Wo,Cout] (possibly channel-sliced) view the BatchNorm backward
+                    drop_p: float = 0.0, need_dx: bool = True, dy_into: Optional[Callable[[], torch.Tensor]] = None) -> Act:
+        """`dy_into`: called in backward, returns the [B,Ho,Wo,Cout] (possibly channel-sliced) view the BatchNorm backward
         writes this unit's pre-activation gradient into instead of a private buffer (ASPP: slices of one concatenated buffer)."""
         L = _lib.lib()
         self._pack(s, need_dx)
@@ -560,8 +544,8 @@ class Engine:
         seed = (self.seed + len(self.tape)) & 0xFFFFFFFFFFFF
         step_ptr = self._step_dev.data_ptr() if drop_p > 0.0 else None
         # residual units: the ReLU sign bits go out as one byte per 8 channels, read back by the backward kernels
-        # instead of the block output (ISWM_RELU_BITS=0 restores the activation read)
-        bits = torch.empty((M, Cout // 8), dtype=torch.uint8, device=self.device) if (relu and residual is not None and self.relu_bits) else None
+        # instead of the block output
+        bits = torch.empty((M, Cout // 8), dtype=torch.uint8, device=self.device) if (relu and residual is not None) else None
         ev = self._prof_begin()
         check(L.iswm_bn_train_apply(raw.data_ptr(), Cout, stats.data_ptr(), rep, M, Cout, bn.weight.data_ptr(), bn.bias.data_ptr(),
                                     BN_EPS, BN_MOMENTUM, bn.running_mean.data_ptr(), bn.running_var.data_ptr(),
@@ -574,21 +558,16 @@ class Engine:
         self._tap(s.name, out)
         if self.debug_taps is not None:
             self.debug_taps[s.name + ":raw"] = raw.float().permute(0, 3, 1, 2).cpu()
-        if (single_consumer and self.bn_dz_fold and relu and residual is None and drop_p == 0.0 and out.ld == Cout and Cout % 64 == 0
-                and self.debug_units is None):
-            out.bn_fold = (raw, save, bn)
 
         def backward():
             dout = out.grad
             pend_bits = None
-            folded_sums, out.bn_sums, out.bn_fold = out.bn_sums, None, None
             if dout is None and out.pending is not None:
                 # this unit's output was the identity operand of a block-closing add + ReLU (downsample branch): its gradient is
                 # the block-output gradient gated by the block's ReLU sign bits, which the kernels apply on the fly (mode 2)
                 dout, pend_bits = out.pending
                 out.pending = None
             assert dout is not None, f"no gradient reached {s.name}"
-            use_mask = relu and folded_sums is None   # residual units: the mask comes from the block output (post add + ReLU)
             rec = None
             if self.debug_units is not None:
                 rec = dict(name=s.name, k=s.k, stride=s.stride, dilation=s.dilation, relu=relu, x=x.t.clone(), raw=raw.clone(),
@@ -597,12 +576,10 @@ class Engine:
                            residual=None if residual is None else residual.t.clone(),
                            xgrad_before=None if x.grad is None else x.grad.t.clone(),
                            resgrad_before=None if (residual is None or residual.grad is None) else residual.grad.t.clone())
-            # (folded: `dout` already holds dz and the sums were accumulated by the consumer's data-gradient epilogue)
-            sums = folded_sums if folded_sums is not None else self._stats_slot(2 * Cout + 2)        # + the grid barrier's arrival counter
-            # the ReLU mask is read from the block output only where a residual was added; otherwise the
-            # kernel recomputes it from raw (one tensor read less in each pass)
-            act_ptr = out.ptr if (use_mask and residual is not None) else None
-            relu_mode = 1 if use_mask else 0
+            sums = self._stats_slot(2 * Cout + 2)
+            # the ReLU mask comes from the sign bits where a residual was added (post add + ReLU); otherwise the kernel
+            # recomputes it from raw (one tensor read less in each pass)
+            act_ptr, relu_mode = None, (1 if relu else 0)
             if bits is not None:
                 act_ptr, relu_mode = bits.data_ptr(), 2
             if pend_bits is not None:
@@ -625,28 +602,19 @@ class Engine:
                     assert residual.grad.ld == residual.C
                     dz_tmp = torch.empty_like(residual.grad.t)
                     dz_ptr, dz_ld = dz_tmp.data_ptr(), residual.C
-            if folded_sums is None and bits is None and pend_bits is None and (M * Cout <= self.bn_fused_max_elems or M * Cout >= self.bn_fused_min_elems):
-                # small tensor (dout and raw stay in L2): reduce + apply in one launch, grid barrier between the passes
-                check(L.iswm_bn_bwd(dout.ptr, dout.ld, raw.data_ptr(), Cout, act_ptr, out.ld, M, Cout,
-                                    bn.weight.data_ptr(), bn.bias.data_ptr(), save.data_ptr(), save[Cout:].data_ptr(), sums.data_ptr(),
-                                    1 if use_mask else 0, drop_p, seed, step_ptr, dy.data_ptr(), dy_ld, dz_ptr, dz_ld,
-                                    self.grad_views[id(bn.weight)].data_ptr(), self.grad_views[id(bn.bias)].data_ptr(), _st()),
-                      "bn_bwd " + s.name)
-            else:
-                nmask = (1.0 / 16 if bits is not None else 1) if act_ptr is not None else 0
-                if folded_sums is None:
-                    ev = self._prof_begin()
-                    check(L.iswm_bn_bwd_reduce(dout.ptr, dout.ld, raw.data_ptr(), Cout, act_ptr, out.ld, M, Cout,
-                                               save.data_ptr(), save[Cout:].data_ptr(), bn.weight.data_ptr(), bn.bias.data_ptr(),
-                                               relu_mode, drop_p, seed, step_ptr, sums.data_ptr(), _st()), "bn_bwd_reduce " + s.name)
-                    self._prof_end(ev, "hbm:bn_bwd_reduce", 2.0 * M * Cout * (2 + nmask), "bn_bwd_reduce " + s.name)
-                ev = self._prof_begin()
-                check(L.iswm_bn_bwd_apply(dout.ptr, dout.ld, raw.data_ptr(), Cout, act_ptr, out.ld, M, Cout,
-                                          bn.weight.data_ptr(), bn.bias.data_ptr(), save.data_ptr(), save[Cout:].data_ptr(), sums.data_ptr(),
-                                          relu_mode, drop_p, seed, step_ptr, dy.data_ptr(), dy_ld, dz_ptr, dz_ld,
-                                          self.grad_views[id(bn.weight)].data_ptr(), self.grad_views[id(bn.bias)].data_ptr(), _st()),
-                      "bn_bwd_apply " + s.name)
-                self._prof_end(ev, "hbm:bn_bwd_apply", 2.0 * M * Cout * (3 + nmask + (1 if dz_ptr is not None else 0)), "bn_bwd_apply " + s.name)
+            nmask = (1.0 / 16 if bits is not None else 1) if act_ptr is not None else 0
+            ev = self._prof_begin()
+            check(L.iswm_bn_bwd_reduce(dout.ptr, dout.ld, raw.data_ptr(), Cout, act_ptr, out.ld, M, Cout,
+                                       save.data_ptr(), save[Cout:].data_ptr(), bn.weight.data_ptr(), bn.bias.data_ptr(),
+                                       relu_mode, drop_p, seed, step_ptr, sums.data_ptr(), _st()), "bn_bwd_reduce " + s.name)
+            self._prof_end(ev, "hbm:bn_bwd_reduce", 2.0 * M * Cout * (2 + nmask), "bn_bwd_reduce " + s.name)
+            ev = self._prof_begin()
+            check(L.iswm_bn_bwd_apply(dout.ptr, dout.ld, raw.data_ptr(), Cout, act_ptr, out.ld, M, Cout,
+                                      bn.weight.data_ptr(), bn.bias.data_ptr(), save.data_ptr(), save[Cout:].data_ptr(), sums.data_ptr(),
+                                      relu_mode, drop_p, seed, step_ptr, dy.data_ptr(), dy_ld, dz_ptr, dz_ld,
+                                      self.grad_views[id(bn.weight)].data_ptr(), self.grad_views[id(bn.bias)].data_ptr(), _st()),
+                  "bn_bwd_apply " + s.name)
+            self._prof_end(ev, "hbm:bn_bwd_apply", 2.0 * M * Cout * (3 + nmask + (1 if dz_ptr is not None else 0)), "bn_bwd_apply " + s.name)
             if dz_tmp is not None:
                 check(L.iswm_add_bf16(residual.grad.ptr, dz_tmp.data_ptr(), dz_tmp.numel(), residual.grad.ptr, _st()), "add_bf16")
             out.grad = None
@@ -675,12 +643,13 @@ class Engine:
                            bn.num_batches_tracked.data_ptr() if train_fwd else None, save.data_ptr(), save[Cc:].data_ptr(),
                            1 if stats is None else stats.numel() // (2 * Cc))
 
-    def _unit_train_dual(self, s: ConvSpec, x: Act, sds: ConvSpec, xds: Act, dsc) -> Act:
+    def _unit_train_dual(self, s: ConvSpec, x: Act, sds: ConvSpec, dsc) -> Act:
         """Closing unit of a bottleneck block with a downsample branch (resnet.py:110-118): out = relu(bn3(conv3(x)) +
-        bn_ds(conv_ds(xds))), both BatchNorms in one kernel per pass (csrc/bn_dual.cu). `dsc` = _conv_raw(sds, xds)."""
+        bn_ds(conv_ds(block input))), both BatchNorms in one kernel per pass (csrc/bn_dual.cu). `dsc` = _conv_raw(sds, block input)
+        + (list that receives the downsample branch's dy for its taped backward,)."""
         L = _lib.lib()
         raw, stats, xin, taps, n_img, Ho, Wo = self._conv_raw(s, x)
-        raw_ds, stats_ds, xin_ds, taps_ds, n_img_ds, Ho_ds, Wo_ds, ds_dy = dsc
+        raw_ds, stats_ds, _, _, _, Ho_ds, Wo_ds, ds_dy = dsc
         assert (Ho, Wo) == (Ho_ds, Wo_ds) and s.cout == sds.cout
         B, Cout = x.B, s.cout
         M = B * Ho * Wo
@@ -714,10 +683,7 @@ class Engine:
             self._prof_end(ev, "hbm:bn_bwd_apply", 2.0 * M * Cout * 5 + M * Cout / 8, "bn_bwd_apply " + s.name + "+ds")
             out.grad = None
             self._conv_backward(s, x, xin, taps, n_img, Ho, Wo, dy, True)
-            if self.ds_bwd_late:
-                ds_dy.append(dy_ds)                   # the downsample convolution's backward runs after conv1's (taped in forward())
-            else:
-                self._conv_backward(sds, xds, xin_ds, taps_ds, n_img_ds, Ho, Wo, dy_ds, True)
+            ds_dy.append(dy_ds)                       # the downsample convolution's backward runs after conv1's (taped in forward())
 
         self.tape.append(backward)
         return out
@@ -732,7 +698,7 @@ class Engine:
         dst = gview if s.k == 1 else self.wacc[self.wacc_off[s.name][0]:self.wacc_off[s.name][0] + self.wacc_off[s.name][1]]
         flops = 2.0 * B * Ho * Wo * Cout * s.cin * s.k * s.k
         layer = s.name.split(".")[1] if s.name.startswith("backbone.layer") else None
-        if layer in self.group_wgrad and self.debug_units is None:
+        if layer in GROUP_WGRAD_LAYERS and self.debug_units is None:
             if self._wq and self._wq_layer != layer:
                 self._flush_wgrad_group()
             self._wq_layer = layer
@@ -849,19 +815,6 @@ class Engine:
         L = _lib.lib()
         B, Cin, Cout = x.B, s.cin, s.cout
         flags, res, mask = 0, None, None
-        if x.grad is None and x.pending is None and x.bn_fold is not None and x.ld == x.C and Cin == x.C:
-            # x = relu(bn(raw)) has no other consumer: write dz = dout . relu_mask and accumulate the BatchNorm-backward sums here
-            raw, save, bn = x.bn_fold
-            x.new_grad()
-            g = x.grad
-            sums = self._stats_slot(2 * Cin + 2)
-            dd = ops.make_conv_desc(B, Hi, Wi, Cout, dy_ld, B, Ho, Wo, Cin, g.ld, dtaps, _lib.EPI_BN_DZ, g.ld)
-            bnd = _lib.BnDz(raw.data_ptr(), save.data_ptr(), save[Cin:].data_ptr(), bn.weight.data_ptr(), bn.bias.data_ptr(), sums.data_ptr())
-            ev = self._prof_begin()
-            check(L.iswm_conv_igemm_bn(C.byref(dd), dy.data_ptr(), s.packed_dgrad.data_ptr(), g.ptr, C.byref(bnd), _st()), "dgrad+bn " + s.name)
-            self._prof_end(ev, "conv_igemm", 2.0 * B * Ho * Wo * Cout * Cin * len(dtaps), "dgrad " + s.name)
-            x.bn_sums = sums
-            return
         if x.grad is None:
             x.new_grad()
             if x.pending is not None:              # + (block-output gradient where the block's ReLU was active)
@@ -908,7 +861,7 @@ class Engine:
         if not self.async_wgrad or self.debug_units is not None:      # the unit-replay recorder reads dW right away
             return Engine._NullCtx()
         if self._wstream is None or self._wstream.device != self.device:
-            self._wstream = torch.cuda.Stream(self.device, priority=int(__import__("os").environ.get("ISWM_WSTREAM_PRIO", "0")))
+            self._wstream = torch.cuda.Stream(self.device)
         main = torch.cuda.current_stream(self.device)
         self._wstream.wait_event(main.record_event())
         # held until the join below: their memory returns to the (main-stream) allocator pool only after the main
@@ -940,7 +893,7 @@ class Engine:
         if not (self.async_wgrad and self.fwd_overlap) or self.profile is not None or self.debug_units is not None or self.debug_taps is not None:
             return Engine._NullCtx()
         if self._wstream is None or self._wstream.device != self.device:
-            self._wstream = torch.cuda.Stream(self.device, priority=int(__import__("os").environ.get("ISWM_WSTREAM_PRIO", "0")))
+            self._wstream = torch.cuda.Stream(self.device)
         self._wstream.wait_event(torch.cuda.current_stream(self.device).record_event())
         self._fwd_forked = True
         return Engine._HandleCtx(self._wstream)
@@ -997,7 +950,7 @@ class Engine:
     def _stats_rep(cout: int) -> int:
         """Copies of a convolution's statistics accumulator (iswm_conv_desc.stats_replicas): narrow layers end every CTA on the
         same 2*Cout addresses, so their fp64 atomics are spread over 4 copies that the BatchNorm kernel folds (cfg2 same-box: 12.87 -> 12.65 ms/step; 8 copies: 12.73)."""
-        return int(__import__("os").environ.get("ISWM_STATS_REP", "4")) if cout <= 128 else 1
+        return 4 if cout <= 128 else 1
 
     def _stats_slot(self, n: int) -> torch.Tensor:
         """zeroed fp64 accumulator slot"""
@@ -1050,7 +1003,7 @@ class Engine:
 
         # ---- stem: 7x7/s2 conv as im2col GEMM -> BN -> ReLU -> maxpool 3x3/s2 (resnet.py:144-148)
         H1, W1 = (H + 1) // 2, (W + 1) // 2
-        if self.stem_rows and self.stem.cin <= 3:
+        if self.stem_rows:
             # x-unrolled rows, phase-major over the row parity: [2][B][H1][W1][kpitch]; the 7 kernel rows are the convolution's taps
             rows = torch.empty((2 * B, H1, W1, STEM_KPITCH), dtype=torch.bfloat16, device=dev)
             ev = self._prof_begin()
@@ -1090,8 +1043,7 @@ class Engine:
             for (c1, c2, c3, ds) in blocks:
                 if ds is None and c1.k == 1 and c1.stride == 1:
                     a.masked_ok = True            # consumers of this block input: conv1 and the identity add, nothing else
-                kw = dict(single_consumer=True) if train else {}
-                if (ds is not None and train and self.dual_bn and self.relu_bits and self.debug_units is None and self.debug_taps is None
+                if (ds is not None and train and self.dual_bn and self.debug_units is None and self.debug_taps is None
                         and c3.cout % 8 == 0):
                     dsc = self._conv_raw(ds, a)   # downsample convolution now; its BatchNorm rides on the block's closing one
                     # its backward is taped HERE, i.e. it runs after conv1's: conv1's data gradient then writes the block input's
@@ -1100,15 +1052,15 @@ class Engine:
                     ds_dy = []
                     self.tape.append(lambda ds=ds, a=a, dsc=dsc, ds_dy=ds_dy: ds_dy and self._conv_backward(ds, a, dsc[2], dsc[3], dsc[4], dsc[5], dsc[6], ds_dy.pop(), True))
                     dsc = dsc + (ds_dy,)
-                    y = unit(c1, a, **kw)
-                    y = unit(c2, y, **kw)
-                    a = self._unit_train_dual(c3, y, ds, a, dsc)
+                    y = unit(c1, a)
+                    y = unit(c2, y)
+                    a = self._unit_train_dual(c3, y, ds, dsc)
                     continue
                 idt = a if ds is None else unit(ds, a, relu=False)
                 if ds is not None:
                     idt.masked_ok = True          # the downsample output feeds the block-closing add only
-                y = unit(c1, a, **kw)
-                y = unit(c2, y, **kw)
+                y = unit(c1, a)
+                y = unit(c2, y)
                 a = unit(c3, y, relu=True, residual=idt)
             if li == 0:
                 low_level = a
@@ -1173,9 +1125,8 @@ class Engine:
                 up.grad = None
             self.tape.append(up_bwd)
             self._slice_grad_split(cat2, [(low_slice, 0), (up, 48)])
-        kw = dict(single_consumer=True) if train else {}
-        y = unit(self.dec1, cat2, **kw)
-        y = unit(self.dec2, y, **kw)
+        y = unit(self.dec1, cat2)
+        y = unit(self.dec2, y)
 
         # ---- classifier 1x1 (+bias) -> fp32 NHWC low-res logits -> bilinear to input size (utils.py:22)
         ncls = self.cls.cout
@@ -1244,22 +1195,13 @@ class Engine:
                 assert g is not None and g.ld == 64
                 sums = self._stats_slot(130)
                 dy = torch.empty((M, 64), dtype=torch.bfloat16, device=dev)
-                if self.stem_pool_bwd:
-                    # both BatchNorm-backward passes gather the activation gradient through the argmax codes: measured SLOWER than
-                    # the three separate kernels (281 vs 178 us at cfg2: the gather runs twice), so off by default
-                    side_b = self._bn_side(bn, None, save, 64, False)
-                    ev = self._prof_begin()
-                    check(L.iswm_stem_pool_bwd(g.ptr, idx.data_ptr(), raw.data_ptr(), C.byref(side_b), B, H1, W1, 64, H2, W2, sums.data_ptr(), dy.data_ptr(),
-                                               self.grad_views[id(bn.weight)].data_ptr(), self.grad_views[id(bn.bias)].data_ptr(), _st()), "stem_pool_bwd")
-                    self._prof_end(ev, "hbm:stem_pool_bwd", 2.0 * (2.0 * M * 64 + 3.0 * B * H2 * W2 * 64) + 2.0 * M * 64, "stem_pool_bwd")
-                else:
-                    dact = torch.empty((M, 64), dtype=torch.bfloat16, device=dev)
-                    check(L.iswm_maxpool_bwd(g.ptr, idx.data_ptr(), B, H1, W1, 64, H2, W2, dact.data_ptr(), _st()), "maxpool_bwd")
-                    check(L.iswm_bn_bwd_reduce(dact.data_ptr(), 64, raw.data_ptr(), 64, None, 64, M, 64, save.data_ptr(), save[64:].data_ptr(),
-                                               bn.weight.data_ptr(), bn.bias.data_ptr(), 1, 0.0, 0, None, sums.data_ptr(), _st()), "bn_bwd_reduce stem")
-                    check(L.iswm_bn_bwd_apply(dact.data_ptr(), 64, raw.data_ptr(), 64, None, 64, M, 64, bn.weight.data_ptr(), bn.bias.data_ptr(), save.data_ptr(),
-                                              save[64:].data_ptr(), sums.data_ptr(), 1, 0.0, 0, None, dy.data_ptr(), 64, None, 0,
-                                              self.grad_views[id(bn.weight)].data_ptr(), self.grad_views[id(bn.bias)].data_ptr(), _st()), "bn_bwd_apply stem")
+                dact = torch.empty((M, 64), dtype=torch.bfloat16, device=dev)
+                check(L.iswm_maxpool_bwd(g.ptr, idx.data_ptr(), B, H1, W1, 64, H2, W2, dact.data_ptr(), _st()), "maxpool_bwd")
+                check(L.iswm_bn_bwd_reduce(dact.data_ptr(), 64, raw.data_ptr(), 64, None, 64, M, 64, save.data_ptr(), save[64:].data_ptr(),
+                                           bn.weight.data_ptr(), bn.bias.data_ptr(), 1, 0.0, 0, None, sums.data_ptr(), _st()), "bn_bwd_reduce stem")
+                check(L.iswm_bn_bwd_apply(dact.data_ptr(), 64, raw.data_ptr(), 64, None, 64, M, 64, bn.weight.data_ptr(), bn.bias.data_ptr(), save.data_ptr(),
+                                          save[64:].data_ptr(), sums.data_ptr(), 1, 0.0, 0, None, dy.data_ptr(), 64, None, 0,
+                                          self.grad_views[id(bn.weight)].data_ptr(), self.grad_views[id(bn.bias)].data_ptr(), _st()), "bn_bwd_apply stem")
                 pooled.grad = None
                 self._stem_wgrad(s, bn, colA, dy, B, H1, W1, M, taps, row_taps, n_img)
 
@@ -1274,7 +1216,6 @@ class Engine:
             dout = out.grad
             sums = self._stats_slot(130)
             dy = torch.empty((M, 64), dtype=torch.bfloat16, device=dev)
-            # two launches: the single-launch grid-barrier version costs more than the boundary it saves (DESIGN 3b)
             check(L.iswm_bn_bwd_reduce(dout.ptr, dout.ld, raw.data_ptr(), 64, None, 64, M, 64, save.data_ptr(), save[64:].data_ptr(),
                                        bn.weight.data_ptr(), bn.bias.data_ptr(), 1, 0.0, 0, None, sums.data_ptr(), _st()), "bn_bwd_reduce stem")
             check(L.iswm_bn_bwd_apply(dout.ptr, dout.ld, raw.data_ptr(), 64, None, 64, M, 64, bn.weight.data_ptr(), bn.bias.data_ptr(), save.data_ptr(),

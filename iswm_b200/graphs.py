@@ -94,10 +94,8 @@ class GraphedTrainStep:
         self.graph = torch.cuda.CUDAGraph()
         # Stream priorities were measured and do NOT help (cfg2, same box): capturing on a high-priority stream (weight-gradient
         # stream lowest) 12.60 -> 13.09 ms/step, the reverse 12.61 -> 12.77; long weight gradients cut into batch slices on top
-        # of either: no better. Equal priorities stay (ISWM_GRAPH_PRIO=1 / ISWM_WSTREAM_PRIO=-1 re-enable the experiments).
-        import os
-        cap = torch.cuda.Stream(x.device, priority=-1) if os.environ.get("ISWM_GRAPH_PRIO", "0") != "0" else None
-        with torch.cuda.graph(self.graph, stream=cap):
+        # of either: no better. Both streams keep the default priority.
+        with torch.cuda.graph(self.graph):
             self.loss = self._eager(self.images, self.labels)
         self.launches_per_replay = _lib.launch_count() - n0      # library kernels recorded in the graph
         # did the captured optimiser step repack the operands itself (FusedSGD with iswm_sgd_pack_batched)? then the graph holds no

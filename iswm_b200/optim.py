@@ -21,9 +21,9 @@ class FusedSGD:
         self.param_groups = [{"lr": lr, "momentum": momentum, "weight_decay": weight_decay, "nesterov": nesterov}]
         self._mom = None
         self._steps = 0
-        # the step also rewrites the packed bf16 convolution operands (one pass over the weights instead of two; ISWM_SGD_PACK=0:
+        # the step also rewrites the packed bf16 convolution operands (one pass over the weights instead of two; False:
         # iswm_sgd_step, and the next forward repacks)
-        self.fuse_pack = __import__("os").environ.get("ISWM_SGD_PACK", "1") != "0"
+        self.fuse_pack = True
         self.lr_dev = None                 # device copy of the learning rate (enable_device_state: CUDA-graph replays)
         self.step_dev = None
 

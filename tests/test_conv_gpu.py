@@ -271,72 +271,6 @@ def test_stride2_3x3_dgrad_by_parity_phases(B, Cin, H, W, Cout, accumulate):
     assert _rel_err(dx.float().cpu().permute(0, 3, 1, 2), want) < 1e-2
 
 
-@pytest.mark.parametrize("B,Cu,H,W,Cv,k,dil", [(2, 64, 16, 16, 64, 3, 1),        # c2 <- c1 of layer1: long K, operand row loaded directly
-                                                (2, 64, 16, 16, 256, 1, 1),       # c3 <- c2: short K, operand row prefetched via cp.async
-                                                (1, 128, 13, 11, 512, 1, 1),      # rows outside the 128-pixel tile grid
-                                                (3, 256, 9, 7, 256, 3, 2),        # dilated 3x3, several channel chunks per tile
-                                                (2, 512, 8, 8, 2048, 1, 1),       # two channel tiles (BN 256) -> statistics flushed twice per CTA
-                                                (2, 256, 24, 24, 8, 1, 1)])       # classifier-like: K = 2 channels in a pitch-8 buffer
-def test_conv_dgrad_carrying_the_bn_backward_reduction(B, Cu, H, W, Cv, k, dil):
-    """iswm_conv_igemm_bn: data gradient of conv V (Cu -> Cv) whose input is relu(bn(raw)) of a unit with Cu channels; the
-    epilogue writes dz = dout . relu_mask and accumulates sum(dz), sum(dz . xhat). Against the unfused pair: plain data
-    gradient, then bn_bwd_reduce / bn_bwd_apply (mask recomputed from raw). dz bit-exact; sums to fp32 summation order."""
-    import ctypes as C
-    real_cv = 2 if Cv == 8 else Cv
-    x, w = _mk(B, Cu, H, W, real_cv, k, seed=21)
-    g = torch.Generator().manual_seed(22)
-    dy = torch.randn((B, real_cv, H, W), generator=g).to(torch.bfloat16)
-    raw = (torch.randn((B, H, W, Cu), generator=g) * 1.5 + 0.2).to(torch.bfloat16).to(DEV)
-    gamma = (torch.rand(Cu, generator=g) + 0.5).to(DEV)
-    beta = (torch.randn(Cu, generator=g) * 0.3).to(DEV)
-    M = B * H * W
-    mean = raw.float().reshape(M, Cu).mean(0)
-    invstd = torch.rsqrt(raw.float().reshape(M, Cu).var(0, unbiased=False) + 1e-5)
-    save = torch.cat([mean, invstd]).contiguous()
-    dy_ld = ((real_cv + 7) // 8) * 8
-    dyd = torch.zeros((B, H, W, dy_ld), dtype=torch.bfloat16, device=DEV)
-    dyd[..., :real_cv] = _nhwc(dy).to(DEV)
-    wd = ops.pack_weight_dgrad(w.to(DEV))
-    taps = [(-a, -b, 0) for (a, b, _) in ops.conv_taps(k, dil)]
-    L, st = _lib.lib(), torch.cuda.current_stream().cuda_stream
-    # unfused: dout, then the reduction and the masked gradient from the BatchNorm kernels
-    dout = torch.zeros((B, H, W, Cu), dtype=torch.bfloat16, device=DEV)
-    ops.conv_igemm(ops.make_conv_desc(B, H, W, real_cv, dy_ld, B, H, W, Cu, Cu, taps), dyd, wd, dout)
-    sums_ref = torch.zeros(2 * Cu, dtype=torch.float64, device=DEV)
-    _lib.check(L.iswm_bn_bwd_reduce(dout.data_ptr(), Cu, raw.data_ptr(), Cu, None, Cu, M, Cu, save.data_ptr(), save[Cu:].data_ptr(),
-                                    gamma.data_ptr(), beta.data_ptr(), 1, 0.0, 0, None, sums_ref.data_ptr(), st))
-    dx_ref = torch.empty_like(dout); dz_ref = torch.empty_like(dout)
-    dg = torch.zeros(Cu, device=DEV); db = torch.zeros(Cu, device=DEV)
-    _lib.check(L.iswm_bn_bwd_apply(dout.data_ptr(), Cu, raw.data_ptr(), Cu, None, Cu, M, Cu, gamma.data_ptr(), beta.data_ptr(), save.data_ptr(),
-                                   save[Cu:].data_ptr(), sums_ref.data_ptr(), 1, 0.0, 0, None, dx_ref.data_ptr(), Cu, dz_ref.data_ptr(), Cu,
-                                   dg.data_ptr(), db.data_ptr(), st))
-    # fused
-    dz = torch.full((B, H, W, Cu), 7.0, dtype=torch.bfloat16, device=DEV)
-    sums = torch.zeros(2 * Cu, dtype=torch.float64, device=DEV)
-    d = ops.make_conv_desc(B, H, W, real_cv, dy_ld, B, H, W, Cu, Cu, taps, flags=_lib.EPI_BN_DZ)
-    bnd = _lib.BnDz(raw.data_ptr(), save.data_ptr(), save[Cu:].data_ptr(), gamma.data_ptr(), beta.data_ptr(), sums.data_ptr())
-    _lib.check(L.iswm_conv_igemm_bn(C.byref(d), dyd.data_ptr(), wd.data_ptr(), dz.data_ptr(), C.byref(bnd), st), "conv_igemm_bn")
-    _assert_healthy()
-    assert torch.equal(dz, dz_ref)
-    frac_on = float((dz_ref != 0).float().mean())
-    assert 0.2 < frac_on < 0.9                       # the mask really gates something
-    s, r = sums.cpu().numpy(), sums_ref.cpu().numpy()
-    scale = np.abs(dz_ref.float().cpu().numpy()).reshape(M, Cu).sum(0)          # magnitude of the summands per channel
-    np.testing.assert_allclose(s[:Cu], r[:Cu], rtol=1e-5, atol=2e-6 * scale.max())
-    np.testing.assert_allclose(s[Cu:], r[Cu:], rtol=1e-5, atol=2e-5 * scale.max())
-    # the second pass on the fused outputs (mask already applied) gives the unfused result
-    dx = torch.empty_like(dout)
-    dg2 = torch.zeros(Cu, device=DEV); db2 = torch.zeros(Cu, device=DEV)
-    _lib.check(L.iswm_bn_bwd_apply(dz.data_ptr(), Cu, raw.data_ptr(), Cu, None, Cu, M, Cu, gamma.data_ptr(), beta.data_ptr(), save.data_ptr(),
-                                   save[Cu:].data_ptr(), sums.data_ptr(), 0, 0.0, 0, None, dx.data_ptr(), Cu, None, 0,
-                                   dg2.data_ptr(), db2.data_ptr(), st))
-    torch.cuda.synchronize()
-    amax = float(dx_ref.float().abs().max())
-    assert float((dx.float() - dx_ref.float()).abs().max()) <= 8e-3 * amax      # one bf16 ulp where a sum's last bits moved
-    np.testing.assert_allclose(dg2.cpu().numpy(), dg.cpu().numpy(), rtol=1e-4, atol=1e-4 * scale.max())
-    np.testing.assert_allclose(db2.cpu().numpy(), db.cpu().numpy(), rtol=1e-4, atol=1e-4 * scale.max())
-
-
 @pytest.mark.parametrize("Cout,rep", [(64, 8), (48, 8), (128, 3), (256, 2)])
 def test_conv_stats_replicas_sum_to_the_single_accumulator(Cout, rep):
     """iswm_conv_desc.stats_replicas: CTA i adds its per-channel sums into copy i % replicas of the fp64 accumulator; the copies

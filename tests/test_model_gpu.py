@@ -384,7 +384,7 @@ def test_batched_unpack_equals_per_layer_and_accumulates():
 
 def test_fused_aspp_backward_matches_the_four_launch_form():
     """ASPP backward as one K-concatenated data-gradient GEMM (iswm_aspp_bwd, the default) against the four separate
-    launches (ISWM_ASPP_FUSED_BWD=0 semantics: engine.aspp_fused_bwd = False): same loss bit for bit (the forward is
+    launches (engine.aspp_fused_bwd = False): same loss bit for bit (the forward is
     untouched); the fused form accumulates the four branches in fp32 where the unfused one rounds to bf16 three times, so the
     parameter gradients agree to bf16 noise."""
     x = torch.randn((4, 3, 96, 96), generator=torch.Generator().manual_seed(5))
@@ -440,35 +440,6 @@ def test_masked_identity_gradient_equals_the_materialised_form():
     assert rel_l2(res[0][2], res[1][2]) <= 1e-5          # the very last gradient of the sweep (stem BatchNorm weight)
 
 
-def test_bn_backward_reduction_folded_into_dgrad_matches_the_separate_pass():
-    """conv -> BN -> ReLU units with one stride-1 consumer (conv1 / conv2 of every bottleneck, both decoder 3x3s): the
-    BatchNorm-backward sums ride on the consumer's data-gradient epilogue (iswm_conv_igemm_bn, Engine.bn_dz_fold) against the separate
-    bn_bwd_reduce pass. Same summands (the stored bf16 dz and raw values), different fp32 partial-sum order: gradients agree
-    to that noise amplified by the occasional bf16 rounding flip downstream."""
-    x = torch.randn((4, 3, 96, 96), generator=torch.Generator().manual_seed(25))
-    y = synth_labels((4, 96, 96), seed=26, fg=0.2, ign=0.05)
-    w = torch.tensor([1.0, 3.0])
-    res = []
-    for fold in (True, False):
-        m, _ = build("resnet50", 16, seed=79)
-        m.to(DEV).train()
-        eng = m.engine()
-        eng.dropout_p = 0.0
-        eng.bn_dz_fold = fold
-        crit = CrossEntropyLoss(weight=w, ignore_index=255).to(DEV)
-        n0 = _lib.launch_count()
-        loss = crit(m(x.to(DEV)), y.to(DEV))
-        loss.backward()
-        torch.cuda.synchronize()
-        res.append((float(loss.detach()), eng.flat_g.clone(), _lib.launch_count() - n0))
-    assert res[0][0] == res[1][0]
-    rel = rel_l2(res[0][1], res[1][1])
-    cos = cosine(res[0][1], res[1][1])
-    report("bn_dz_fold_vs_separate_reduce", flat_grad_rel_l2=rel, cosine=cos, launches_folded=res[0][2], launches_separate=res[1][2])
-    assert res[1][2] - res[0][2] >= 30          # 16 conv1 + 16 conv2 (minus stride-2 consumers) + 2 decoder reductions are gone
-    assert rel <= 3e-2 and cos >= 0.999
-
-
 def test_dual_batchnorm_blocks_match_the_two_kernel_form():
     """First block of every ResNet layer (resnet.py:176-186): closing BatchNorm + downsample BatchNorm as one kernel per pass
     (csrc/bn_dual.cu, the default) against the separate kernels. The fused forward adds the shortcut in fp32 instead of
@@ -512,10 +483,9 @@ def test_dual_batchnorm_blocks_match_the_two_kernel_form():
         assert rel_l2(a, b) <= 2e-2, (k, rel_l2(a, b))
 
 
-def test_fused_stem_tail_matches_the_separate_kernels():
-    """Stem BatchNorm + ReLU + maxpool as one pass (csrc/stem_pool.cu, the default) against bn_train_apply + maxpool_fwd and
-    their three backward kernels: the forward is bit-identical (same logits, same loss); gradients differ by the fp32 order of
-    the stem BatchNorm's two reduction sums only."""
+def test_fused_stem_tail_forward_matches_the_separate_kernels():
+    """Stem BatchNorm + ReLU + maxpool as one forward pass (csrc/stem_pool.cu, the default) against bn_train_apply + maxpool_fwd:
+    the forward is bit-identical (same logits, same loss); both forms run the same three backward kernels."""
     x = torch.randn((4, 3, 96, 96), generator=torch.Generator().manual_seed(45))
     y = synth_labels((4, 96, 96), seed=46, fg=0.2, ign=0.05)
     w = torch.tensor([1.0, 3.0])
@@ -526,7 +496,6 @@ def test_fused_stem_tail_matches_the_separate_kernels():
         eng = m.engine()
         eng.dropout_p = 0.0
         eng.stem_pool = fused
-        eng.stem_pool_bwd = fused                       # the fused backward too (off by default: it is slower)
         crit = CrossEntropyLoss(weight=w, ignore_index=255).to(DEV)
         n0 = _lib.launch_count()
         logits = m(x.to(DEV))
@@ -537,7 +506,7 @@ def test_fused_stem_tail_matches_the_separate_kernels():
                     m.backbone.bn1.running_var.clone(), m.backbone.conv1.weight.grad.clone(), m.backbone.bn1.weight.grad.clone()))
     assert torch.equal(res[0][3], res[1][3]) and res[0][0] == res[1][0]
     assert torch.equal(res[0][4], res[1][4])
-    assert res[1][2] - res[0][2] == 2                    # (apply + maxpool) -> 1, (maxpool_bwd + reduce + apply) -> 2
+    assert res[1][2] - res[0][2] == 1                    # (apply + maxpool) -> 1
     rel = rel_l2(res[0][1], res[1][1])
     report("fused_stem_tail_vs_separate", flat_grad_rel_l2=rel, stem_weight_grad_rel_l2=rel_l2(res[0][5], res[1][5]),
            bn1_weight_grad_rel_l2=rel_l2(res[0][6], res[1][6]))

@@ -20,6 +20,6 @@ for r in range(reps):
     torch.cuda.synchronize()
     rows.append(([float(l) for l in losses], m.engine().flat_w.clone()))
 ref = rows[0]
-print({k: os.environ.get(k) for k in ("ISWM_PDL", "ISWM_ASYNC_WGRAD", "ISWM_BN_WAVES", "PDROP") if os.environ.get(k) is not None})
+print({k: os.environ.get(k) for k in ("ISWM_PDL", "PDROP") if os.environ.get(k) is not None})
 for i, (l, w) in enumerate(rows):
     print(f"  rep {i}: losses {' '.join(f'{v:.6f}' for v in l)}  w vs rep0 {float((w - ref[1]).norm() / ref[1].norm()):.2e}")
