@@ -46,7 +46,7 @@ void iswm_debug_set_skip(int mask);
 /* element type codes for label / prediction buffers */
 enum { ISWM_U8 = 0, ISWM_I32 = 1, ISWM_I64 = 2 };
 /* element type codes for floating tensors */
-enum { ISWM_F32 = 0, ISWM_BF16 = 1 };
+enum { ISWM_F32 = 0, ISWM_BF16 = 1, ISWM_E4M3 = 2 };
 
 /* ---- loss / histogram / metric (HBM-bound) ----------------------------- */
 
@@ -193,6 +193,16 @@ int iswm_conv_igemm(const iswm_conv_desc* desc, const void* d_in, const void* d_
 int iswm_conv_igemm_ex(const iswm_conv_desc* desc, const void* d_in, const void* d_wgt,
                        void* d_out, const float* d_scale, const float* d_shift,
                        const void* d_res, double* d_stats, const uint8_t* d_res_mask, void* stream);
+
+/* FP8 (e4m3) inference form of iswm_conv_igemm (iswm_b200/quant.py): d_in e4m3 NHWC activations (in_ld %% 16 == 0), d_wgt
+ * e4m3 [Cout][ntaps][Cin_pad] with Cin_pad = Cin rounded up to 128 (iswm_pack_weight_f8), tcgen05 kind::f8f6f4 with fp32
+ * accumulation. Epilogue, in this order: y = acc * scale[c] + shift[c] (AFFINE), y += res_scale * res (RESIDUAL, d_res e4m3 of
+ * the output geometry, pitch res_ld), ReLU (RELU), then the store as out_type: ISWM_E4M3 (round to nearest even, saturating
+ * to +-448), ISWM_BF16 or ISWM_F32. Statistics, residual masks, ISWM_EPI_OUT_F32 and strided outputs are rejected; a
+ * stride-2 convolution's in_phase_view needs Cin %% 128 == 0. */
+int iswm_conv_igemm_f8(const iswm_conv_desc* desc, const void* d_in, const void* d_wgt, void* d_out,
+                       const float* d_scale, const float* d_shift, const void* d_res, float res_scale,
+                       int out_type, void* stream);
 
 /* ASPP backward, data-gradient half (network/_deeplab.py:143-172: the 1x1 branch and the three dilated 3x3 branches all
  * read the SAME 2048-channel feature map): ONE K-concatenated implicit GEMM
@@ -422,6 +432,25 @@ int iswm_logits_up_fwd(const float* d_x, int B, int Hi, int Wi, int C, int Ho, i
  * (network/_deeplab.py:51 Conv2d(256, C, 1) bias) from the same sweep over dlogits */
 int iswm_logits_up_bwd(const float* d_dout, int B, int Hi, int Wi, int C, int Ho, int Wo, void* d_dx, int dx_ld,
                        float* d_bias_grad, void* stream);
+/* ---- FP8 (e4m3) inference path (csrc/quant.cu, iswm_b200/quant.py) ----------------------------------------------------
+ * An e4m3 activation q stands for q * s with one fp32 scale s per tensor; every conversion to e4m3 is
+ * cvt.rn.satfinite(x / s) with an IEEE fp32 division.
+ * iswm_pack_weight_f8: fp32 OIHW -> d_sw[o] = max_i |w[o,i]| / 448 (1 for an all-zero channel) and e4m3
+ *   d_out [Cout][RS][cin_pad] = e4m3(w[o][c][t] / d_sw[o]), zero for c >= Cin; cin_pad a multiple of 128.
+ * iswm_maxpool_fwd_f8: MaxPool2d(3,2,1) of bf16 NHWC [B,H,W,C] -> e4m3 [B,Ho,Wo,C] with scale s.
+ * iswm_gap_fwd_f8: e4m3 [B,HW,x_ld] (scale s) -> bf16 [B,C] = (sum over HW) / HW * s.
+ * iswm_broadcast_hw_f8: bf16 [B,C] -> e4m3 channel slice [B,HW,out_ld] with scale s.
+ * iswm_bilinear_fwd_f8: as iswm_bilinear_fwd (generic kernel), bf16 in, e4m3 channel slice out with scale s.
+ * iswm_phase_split_b8 / iswm_subsample2_b8: iswm_phase_split / iswm_subsample2 over one-byte elements (C, x_ld multiples of 16). */
+int iswm_pack_weight_f8(const float* d_w, int Cout, int Cin, int RS, int cin_pad, void* d_out, float* d_sw, void* stream);
+int iswm_maxpool_fwd_f8(const void* d_x, int B, int H, int W, int C, int Ho, int Wo, float s, void* d_out, void* stream);
+int iswm_gap_fwd_f8(const void* d_x, int x_ld, int B, int64_t HW, int C, float s, void* d_out, void* stream);
+int iswm_broadcast_hw_f8(const void* d_x, int B, int64_t HW, int C, float s, void* d_out, int out_ld, void* stream);
+int iswm_bilinear_fwd_f8(const void* d_x, int x_ld, int B, int Hi, int Wi, int C, int Ho, int Wo, float s, void* d_out,
+                         int out_ld, void* stream);
+int iswm_phase_split_b8(const void* d_x, int x_ld, int B, int H, int W, int C, void* d_out, void* stream);
+int iswm_subsample2_b8(const void* d_x, int x_ld, int B, int H, int W, int C, void* d_out, void* stream);
+
 /* strided helpers for stride-2 convolutions */
 int iswm_phase_split(const void* d_x, int x_ld, int B, int H, int W, int C, void* d_out, void* stream);   /* -> [4][B][ceil(H/2)][ceil(W/2)][C], phase = (h&1)*2 + (w&1) */
 int iswm_subsample2(const void* d_x, int x_ld, int B, int H, int W, int C, void* d_out, void* stream);    /* -> [B][ceil(H/2)][ceil(W/2)][C] */

@@ -16,7 +16,7 @@ LIB_PATH = os.environ.get("ISWM_B200_LIB") or os.path.join(_HERE, "libiswm_b200.
 
 MAX_TAPS = 32
 U8, I32, I64 = 0, 1, 2
-F32, BF16 = 0, 1
+F32, BF16, E4M3 = 0, 1, 2
 EPI_AFFINE, EPI_RELU, EPI_RESIDUAL, EPI_STATS, EPI_OUT_F32, EPI_RES_MASK = 1, 2, 4, 8, 16, 32
 
 
@@ -109,6 +109,7 @@ SIGNATURES = {
     "iswm_focal_fwd_bwd": (_i, [_p, _i, _p, _i, _p, _i64, _i, _i64, _i, _f, _f, _i, _p, _p, _p, _p]),
     "iswm_conv_igemm": (_i, [C.POINTER(ConvDesc), _p, _p, _p, _p, _p, _p, _p, _p]),
     "iswm_conv_igemm_ex": (_i, [C.POINTER(ConvDesc), _p, _p, _p, _p, _p, _p, _p, _p, _p]),
+    "iswm_conv_igemm_f8": (_i, [C.POINTER(ConvDesc), _p, _p, _p, _p, _p, _p, _f, _i, _p]),
     "iswm_aspp_bwd": (_i, [_p, _i, _p, _i, _i, _i, _i, _i, C.POINTER(C.c_int), _p, _i, _i, _p]),
     "iswm_peer_barrier": (_i, [C.POINTER(_p), _i, _i, _p, _p]),
     "iswm_peer_allreduce_f32": (_i, [C.POINTER(_p), _i, _i, _i64, _i64, _i, _p]),
@@ -145,6 +146,13 @@ SIGNATURES = {
     "iswm_bilinear_bwd": (_i, [_p, _i, _i, _i, _i, _i, _i, _i, _p, _i, _p]),
     "iswm_logits_up_fwd": (_i, [_p, _i, _i, _i, _i, _i, _i, _p, _p]),
     "iswm_logits_up_bwd": (_i, [_p, _i, _i, _i, _i, _i, _i, _p, _i, _p, _p]),
+    "iswm_pack_weight_f8": (_i, [_p, _i, _i, _i, _i, _p, _p, _p]),
+    "iswm_maxpool_fwd_f8": (_i, [_p, _i, _i, _i, _i, _i, _i, _f, _p, _p]),
+    "iswm_gap_fwd_f8": (_i, [_p, _i, _i, _i64, _i, _f, _p, _p]),
+    "iswm_broadcast_hw_f8": (_i, [_p, _i, _i64, _i, _f, _p, _i, _p]),
+    "iswm_bilinear_fwd_f8": (_i, [_p, _i, _i, _i, _i, _i, _i, _i, _f, _p, _i, _p]),
+    "iswm_phase_split_b8": (_i, [_p, _i, _i, _i, _i, _i, _p, _p]),
+    "iswm_subsample2_b8": (_i, [_p, _i, _i, _i, _i, _i, _p, _p]),
     "iswm_phase_split": (_i, [_p, _i, _i, _i, _i, _i, _p, _p]),
     "iswm_subsample2": (_i, [_p, _i, _i, _i, _i, _i, _p, _p]),
     "iswm_zero_stuff2": (_i, [_p, _i, _i, _i, _i, _i, _i, _p, _p]),

@@ -23,8 +23,14 @@
 // Forward convs of network/backbone/resnet.py:27-35 (conv3x3 / conv1x1, all dilations)
 // and network/_deeplab.py:37-51,124,134,149,162; their data gradients run through the
 // same kernel with transposed packed weights and negated tap offsets.
+//
+// conv_igemm_f8_kernel is the same body over e4m3 operands (tcgen05.mma kind::f8f6f4, E4M3 x E4M3 -> fp32) for the
+// post-training-quantised inference path (iswm_b200/quant.py): a k-block is still one 128-byte swizzle row, now 128
+// channels, and each of its four MMAs still advances the operand descriptors by 32 bytes (K = 32 instead of 16). Its
+// epilogue reads an e4m3 residual scaled by a per-call factor and writes e4m3 / bf16 / fp32 with direct stores.
 #include "tc_common.cuh"
 #include <algorithm>
+#include <cuda_fp8.h>
 
 namespace iswm {
 
@@ -62,7 +68,22 @@ struct ConvKParams {
   double* stats;                 // fp64 accumulators: cross-CTA summation order no longer shows up in fp32 results
   int stats_rep;                 // copies of the accumulator vector; this CTA adds into copy blockIdx.x % stats_rep
   int* abort_flag;
+  float res_scale;               // e4m3 kernel: the residual is added as res_scale * residual
+  int out_f8;                    // e4m3 kernel: write e4m3 (satfinite) instead of bf16 / fp32
 };
+
+// four fp32 values -> four e4m3 bytes (round to nearest even, saturating to +-448), first value in the lowest byte
+__device__ __forceinline__ uint32_t pack_e4m3x4(float a, float b, float c, float d) {
+  const uint32_t lo = __nv_cvt_float2_to_fp8x2(make_float2(a, b), __NV_SATFINITE, __NV_E4M3);
+  const uint32_t hi = __nv_cvt_float2_to_fp8x2(make_float2(c, d), __NV_SATFINITE, __NV_E4M3);
+  return lo | (hi << 16);
+}
+__device__ __forceinline__ void unpack_e4m3x2(uint32_t v, float& lo, float& hi) {
+  const __half2_raw h = __nv_cvt_fp8x2_to_halfraw2((__nv_fp8x2_storage_t)(v & 0xffffu), __NV_E4M3);
+  const float2 f = __half22float2(*reinterpret_cast<const __half2*>(&h));
+  lo = f.x;
+  hi = f.y;
+}
 
 // A CTA's tile schedule (tile = blockIdx.x, += gridDim.x ...) decoded into (n tile, w / h / image tile) coordinates. The decode
 // of the first tile uses integer divisions once; every later tile adds the precomputed mixed-radix digits of the grid size with
@@ -100,10 +121,12 @@ struct TileIter {
 constexpr int kEpiWG = 2;
 constexpr int kConvThreads = 128 * (kEpiWG + 1);
 
-__global__ void __launch_bounds__(kConvThreads, 1)
-conv_igemm_kernel(const __grid_constant__ CUtensorMap tmap_a,
-                  const __grid_constant__ CUtensorMap tmap_b,
-                  const __grid_constant__ CUtensorMap tmap_out, const ConvKParams p) {
+// F8 = false: bf16 operands, 64 channels per k-block; true: e4m3 operands, 128 channels per k-block (no statistics,
+// residual mask, strided output or TMA store: the host rejects or disables them)
+template <bool F8>
+__device__ __forceinline__ void conv_igemm_body(const CUtensorMap& tmap_a, const CUtensorMap& tmap_b,
+                                                const CUtensorMap& tmap_out, const ConvKParams& p) {
+  constexpr int KB = F8 ? 128 : kKBlock;      // elements per k-block
   extern __shared__ uint8_t smem_raw[];
 #ifdef ISWM_EPI_TIMING
   unsigned long long gt_entry, gt_prol = 0, gt_dep = 0;
@@ -115,12 +138,12 @@ conv_igemm_kernel(const __grid_constant__ CUtensorMap tmap_a,
   const uint32_t b_bytes = (uint32_t)p.BN * 128u;
   const uint32_t stage_bytes = kABytes + b_bytes;
   // [ring stages][out staging: one 16K tile per epilogue warpgroup, if TMA out][residual prefetch: same][barriers][scale, shift]
-  const bool tma_out = p.use_tma_out != 0;
+  const bool tma_out = !F8 && p.use_tma_out != 0;
   uint32_t off = (uint32_t)p.stages * stage_bytes;
   const uint32_t obuf = ring + off;
   if (tma_out) off += kEpiWG * kStageBuf;
   const uint32_t rbuf = ring + off;                        // residual prefetch tile, one per epilogue warpgroup
-  if (p.res_prefetch) off += kEpiWG * kStageBuf;
+  if (!F8 && p.res_prefetch) off += kEpiWG * kStageBuf;
   uint8_t* tail = smem + off;
   uint64_t* bars = reinterpret_cast<uint64_t*>(tail);      // full[8] empty[8] tfull[2] tempty[2]
   uint32_t* tmem_slot = reinterpret_cast<uint32_t*>(bars + 2 * kMaxStages + 6);
@@ -213,10 +236,10 @@ conv_igemm_kernel(const __grid_constant__ CUtensorMap tmap_a,
           const uint32_t a_dst = ring + stage * stage_bytes;
           tc::mbar_expect_tx(bar_full + 8 * stage, stage_bytes);
           if (p.phase_view)
-            tc::tma_load_5d(a_dst, &tmap_a, bar_full + 8 * stage, (p.phase[t] & 1) * p.pv_ld + p.coff[t] + kc * kKBlock, cw, p.phase[t] >> 1, ch, b0);
+            tc::tma_load_5d(a_dst, &tmap_a, bar_full + 8 * stage, (p.phase[t] & 1) * p.pv_ld + p.coff[t] + kc * KB, cw, p.phase[t] >> 1, ch, b0);
           else
-            tc::tma_load_4d(a_dst, &tmap_a, bar_full + 8 * stage, p.coff[t] + kc * kKBlock, cw, ch, cb);
-          tc::tma_load_2d(a_dst + kABytes, &tmap_b, bar_full + 8 * stage, p.wtap[t] * p.cin_pad + kc * kKBlock, n0);
+            tc::tma_load_4d(a_dst, &tmap_a, bar_full + 8 * stage, p.coff[t] + kc * KB, cw, ch, cb);
+          tc::tma_load_2d(a_dst + kABytes, &tmap_b, bar_full + 8 * stage, p.wtap[t] * p.cin_pad + kc * KB, n0);
           stage += np;
           if (stage >= p.stages) { stage -= p.stages; phase ^= 1; }
           kc += np;
@@ -232,7 +255,7 @@ conv_igemm_kernel(const __grid_constant__ CUtensorMap tmap_a,
   } else if (warp == 1) {
     // ===================== MMA issuer =====================
     if (tc::elect_one()) {
-      const uint32_t idesc = tc::make_idesc_bf16(kTileM, p.BN, 0, 0);
+      const uint32_t idesc = F8 ? tc::make_idesc_e4m3(kTileM, p.BN) : tc::make_idesc_bf16(kTileM, p.BN, 0, 0);
       int stage = 0, as = 0;
       uint32_t phase = 0, aphase = 0;
       bool ok = true;
@@ -265,8 +288,10 @@ conv_igemm_kernel(const __grid_constant__ CUtensorMap tmap_a,
           const uint64_t da = tc::make_smem_desc_sw128(a_addr, 16, 1024);
           const uint64_t db = tc::make_smem_desc_sw128(a_addr + kABytes, 16, 1024);
 #pragma unroll
-          for (int k = 0; k < kKBlock / 16; k++)
-            tc::umma_bf16(d_tmem, da + 2 * k, db + 2 * k, idesc, (kb | k) != 0);
+          for (int k = 0; k < 4; k++) {                // 32 bytes of K per MMA: 16 bf16 or 32 e4m3 channels
+            if constexpr (F8) tc::umma_f8(d_tmem, da + 2 * k, db + 2 * k, idesc, (kb | k) != 0);
+            else tc::umma_bf16(d_tmem, da + 2 * k, db + 2 * k, idesc, (kb | k) != 0);
+          }
           tc::umma_commit(bar_empty + 8 * stage);     // frees this smem stage when the MMAs retire
           if (++stage == p.stages) { stage = 0; phase ^= 1; }
         }
@@ -294,7 +319,7 @@ conv_igemm_kernel(const __grid_constant__ CUtensorMap tmap_a,
     const int hh = (row >> p.lgBW) & (BH - 1);
     const int ww = row & (BW - 1);
     const bool f_aff = p.flags & ISWM_EPI_AFFINE, f_relu = p.flags & ISWM_EPI_RELU, f_res = p.flags & ISWM_EPI_RESIDUAL,
-               f_stats = p.flags & ISWM_EPI_STATS, f_mask = p.flags & ISWM_EPI_RES_MASK, f_f32 = p.flags & ISWM_EPI_OUT_F32;
+               f_stats = !F8 && (p.flags & ISWM_EPI_STATS), f_mask = !F8 && (p.flags & ISWM_EPI_RES_MASK), f_f32 = p.flags & ISWM_EPI_OUT_F32;
     // Each epilogue WARP is independent between channel-tile changes: it stages its own 32 rows (a 4 KiB, 1 KiB-aligned
     // slice of the warpgroup's staging tile), issues its own TMA store (a 32-pixel sub-box of the tile) and sums its own
     // rows for the statistics - __syncwarp() instead of three 128-thread named barriers per chunk, so the eight warps
@@ -361,7 +386,7 @@ conv_igemm_kernel(const __grid_constant__ CUtensorMap tmap_a,
     // is prefetched with cp.async into the warpgroup's residual tile while the current chunk is processed; only the
     // issuing thread reads it back, so no barrier is involved.
     const uint32_t rb_row = rbuf + (uint32_t)wg * kStageBuf + row_off;
-    const bool res_pf_ok = f_res && p.res_prefetch != 0;
+    const bool res_pf_ok = !F8 && f_res && p.res_prefetch != 0;
     auto chunk_owner_ok = [&](const TileIter& ti_, int it_, int c_) -> bool {
       if (owner_of(it_, c_) != wg) return false;
       return ti_.nt * p.BN + c_ * 64 < p.Cout;
@@ -442,11 +467,17 @@ conv_igemm_kernel(const __grid_constant__ CUtensorMap tmap_a,
         tc::tmem_ld64(t_row + c64 * 64, v);
         // residual: this thread's row of the chunk (128 contiguous bytes) was prefetched into shared memory
         uint4 rr[8];
-        const bool res_vec = res_pf_ok ? pf_vec : (f_res && valid && ncols == 64 && (p.res_ld & 7) == 0);
+        const bool res_vec = res_pf_ok ? pf_vec : (f_res && valid && ncols == 64 && (p.res_ld & (F8 ? 15 : 7)) == 0);
         if (f_res && !res_pf_ok && res_vec) {             // long-K convolution: direct loads, issued under the TMEM read
-          const uint4* rp = reinterpret_cast<const uint4*>(p.res + rpix + nc);
+          if constexpr (F8) {
+            const uint4* rp = reinterpret_cast<const uint4*>(reinterpret_cast<const uint8_t*>(p.res) + rpix + nc);
 #pragma unroll
-          for (int j = 0; j < 8; j++) rr[j] = rp[j];
+            for (int j = 0; j < 4; j++) rr[j] = rp[j];
+          } else {
+            const uint4* rp = reinterpret_cast<const uint4*>(p.res + rpix + nc);
+#pragma unroll
+            for (int j = 0; j < 8; j++) rr[j] = rp[j];
+          }
         }
         if (res_pf_ok) {                                   // (pf_ti.tile, pf_c) == (ti.tile, c64) by construction
           asm volatile("cp.async.wait_group 0;" ::: "memory");
@@ -479,7 +510,34 @@ conv_igemm_kernel(const __grid_constant__ CUtensorMap tmap_a,
             f[4 * j + 3] = fmaf(f[4 * j + 3], a.w, c.w);
           }
         }
-        if (f_res) {
+        if (F8 && f_res) {                                 // f += res_scale * residual (e4m3)
+          if (res_vec) {
+#pragma unroll
+            for (int j = 0; j < 4; j++) {
+              const uint32_t r4[4] = {rr[j].x, rr[j].y, rr[j].z, rr[j].w};
+#pragma unroll
+              for (int k = 0; k < 4; k++) {
+                float a0, a1, a2, a3;
+                unpack_e4m3x2(r4[k], a0, a1);
+                unpack_e4m3x2(r4[k] >> 16, a2, a3);
+                f[16 * j + 4 * k] = fmaf(a0, p.res_scale, f[16 * j + 4 * k]);
+                f[16 * j + 4 * k + 1] = fmaf(a1, p.res_scale, f[16 * j + 4 * k + 1]);
+                f[16 * j + 4 * k + 2] = fmaf(a2, p.res_scale, f[16 * j + 4 * k + 2]);
+                f[16 * j + 4 * k + 3] = fmaf(a3, p.res_scale, f[16 * j + 4 * k + 3]);
+              }
+            }
+          } else if (valid) {
+            const uint8_t* rp = reinterpret_cast<const uint8_t*>(p.res) + rpix + nc;
+#pragma unroll
+            for (int j = 0; j < 64; j += 2)
+              if (j < ncols) {
+                float a0, a1;
+                unpack_e4m3x2(rp[j] | ((j + 1 < ncols ? (uint32_t)rp[j + 1] : 0u) << 8), a0, a1);
+                f[j] = fmaf(a0, p.res_scale, f[j]);
+                if (j + 1 < ncols) f[j + 1] = fmaf(a1, p.res_scale, f[j + 1]);
+              }
+          }
+        } else if (f_res) {
           if (res_vec) {
 #pragma unroll
             for (int j = 0; j < 8; j++) {
@@ -573,6 +631,22 @@ conv_igemm_kernel(const __grid_constant__ CUtensorMap tmap_a,
               for (int j = 0; j < 64; j++)
                 if (j < ncols) op[j] = f[j];
             }
+          } else if (F8 && p.out_f8) {
+            uint8_t* op = reinterpret_cast<uint8_t*>(p.out) + opix + nc;
+            if ((ncols & 15) == 0 && (p.out_ld & 15) == 0 && (nc & 15) == 0 && (reinterpret_cast<uintptr_t>(p.out) & 15) == 0) {
+              // 16-byte stores; a narrow chunk (the 48-channel slice of the decoder concat) writes its first ncols bytes
+#pragma unroll
+              for (int j = 0; j < 4; j++)
+                if (16 * j < ncols)
+                  *reinterpret_cast<uint4*>(op + 16 * j) = make_uint4(pack_e4m3x4(f[16 * j], f[16 * j + 1], f[16 * j + 2], f[16 * j + 3]),
+                                                                      pack_e4m3x4(f[16 * j + 4], f[16 * j + 5], f[16 * j + 6], f[16 * j + 7]),
+                                                                      pack_e4m3x4(f[16 * j + 8], f[16 * j + 9], f[16 * j + 10], f[16 * j + 11]),
+                                                                      pack_e4m3x4(f[16 * j + 12], f[16 * j + 13], f[16 * j + 14], f[16 * j + 15]));
+            } else {
+#pragma unroll
+              for (int j = 0; j < 64; j++)
+                if (j < ncols) op[j] = (uint8_t)(pack_e4m3x4(f[j], 0.f, 0.f, 0.f) & 0xffu);
+            }
           } else {
             __nv_bfloat16* op = reinterpret_cast<__nv_bfloat16*>(p.out) + opix + nc;
             if ((ncols & 7) == 0 && (p.out_ld & 7) == 0 && (nc & 7) == 0 && (reinterpret_cast<uintptr_t>(p.out) & 15) == 0) {
@@ -619,6 +693,20 @@ conv_igemm_kernel(const __grid_constant__ CUtensorMap tmap_a,
 #endif
 }
 
+__global__ void __launch_bounds__(kConvThreads, 1)
+conv_igemm_kernel(const __grid_constant__ CUtensorMap tmap_a,
+                  const __grid_constant__ CUtensorMap tmap_b,
+                  const __grid_constant__ CUtensorMap tmap_out, const ConvKParams p) {
+  conv_igemm_body<false>(tmap_a, tmap_b, tmap_out, p);
+}
+
+__global__ void __launch_bounds__(kConvThreads, 1)
+conv_igemm_f8_kernel(const __grid_constant__ CUtensorMap tmap_a,
+                     const __grid_constant__ CUtensorMap tmap_b,
+                     const __grid_constant__ CUtensorMap tmap_out, const ConvKParams p) {
+  conv_igemm_body<true>(tmap_a, tmap_b, tmap_out, p);
+}
+
 static int ilog2_ceil(int v) {
   int l = 0;
   while ((1 << l) < v) l++;
@@ -635,10 +723,18 @@ extern "C" int iswm_conv_igemm(const iswm_conv_desc* d, const void* d_in, const 
   return iswm_conv_igemm_ex(d, d_in, d_wgt, d_out, d_scale, d_shift, d_res, d_stats, nullptr, stream);
 }
 
-extern "C" int iswm_conv_igemm_ex(const iswm_conv_desc* d, const void* d_in, const void* d_wgt,
-                                  void* d_out, const float* d_scale, const float* d_shift,
-                                  const void* d_res, double* d_stats, const uint8_t* d_res_mask, void* stream) {
-  if (debug_skip(ISWM_SKIP_CONV_IGEMM)) return 0;
+// f8: e4m3 operands / residual (conv_igemm_f8_kernel), output type out_type (ISWM_E4M3 / ISWM_BF16 / ISWM_F32)
+static int conv_igemm_launch(const iswm_conv_desc* d, const void* d_in, const void* d_wgt, void* d_out, const float* d_scale,
+                             const float* d_shift, const void* d_res, double* d_stats, const uint8_t* d_res_mask, bool f8,
+                             float res_scale, int out_type, void* stream) {
+  const int KB = f8 ? 128 : kKBlock;                       // channels per k-block
+  if (f8) {
+    ISWM_REQUIRE(d && (d->flags & ~(ISWM_EPI_AFFINE | ISWM_EPI_RELU | ISWM_EPI_RESIDUAL)) == 0,
+                 "conv_igemm_f8: only AFFINE, RELU and RESIDUAL (statistics, residual masks and fp32 output flags are training-side)");
+    ISWM_REQUIRE(d->out_ws == 0 && d->out_hs == 0 && d->out_bs == 0, "conv_igemm_f8: strided outputs are not supported");
+    ISWM_REQUIRE(out_type == ISWM_E4M3 || out_type == ISWM_BF16 || out_type == ISWM_F32, "conv_igemm_f8: out_type %d", out_type);
+    ISWM_REQUIRE((d->in_ld % 16) == 0, "conv_igemm_f8: in_ld=%d must be a multiple of 16 (tensor-map row pitch in bytes)", d->in_ld);
+  }
   ISWM_REQUIRE(!(d && (d->flags & ISWM_EPI_RES_MASK)) || (d_res_mask && (d->flags & ISWM_EPI_RESIDUAL) && (d->Cout % 64) == 0 &&
                                                           d->out_ws == 0 && d->out_hs == 0 && d->out_bs == 0),
                "conv_igemm: RES_MASK needs RESIDUAL, the bit tensor, Cout %% 64 == 0 and a dense output");
@@ -659,7 +755,7 @@ extern "C" int iswm_conv_igemm_ex(const iswm_conv_desc* d, const void* d_in, con
   int B = d->B, Hi = d->Hi, Wi = d->Wi, Ho = d->Ho, Wo = d->Wo, n_img = d->n_img;
   const bool strided_out = d->out_ws != 0 || d->out_hs != 0 || d->out_bs != 0;
   const bool phase_view = d->in_phase_view != 0;
-  ISWM_REQUIRE(!phase_view || ((d->Cin % kKBlock) == 0 && n_img == B), "conv_igemm: in_phase_view needs Cin %% 64 == 0 and n_img == B (Cin=%d n_img=%d B=%d)", d->Cin, n_img, B);
+  ISWM_REQUIRE(!phase_view || ((d->Cin % KB) == 0 && n_img == B), "conv_igemm: in_phase_view needs Cin %% %d == 0 and n_img == B (Cin=%d n_img=%d B=%d)", KB, d->Cin, n_img, B);
   bool pointwise = (d->ntaps == 1 && d->dh[0] == 0 && d->dw[0] == 0 && d->phase[0] == 0 &&
                     Hi == Ho && Wi == Wo && n_img == B && !strided_out && !phase_view);
   if (pointwise) {  // a 1x1 convolution is a plain GEMM over all pixels: no tile-edge waste
@@ -696,11 +792,11 @@ extern "C" int iswm_conv_igemm_ex(const iswm_conv_desc* d, const void* d_in, con
   const int64_t total = (int64_t)p.tiles_w * p.tiles_h * p.tiles_b * p.tiles_n;
   ISWM_REQUIRE(total < (1ll << 31), "conv_igemm: too many tiles");
   p.total_tiles = (int)total;
-  p.kchunks = (d->Cin + kKBlock - 1) / kKBlock;
-  p.cin_pad = p.kchunks * kKBlock;
+  p.kchunks = (d->Cin + KB - 1) / KB;
+  p.cin_pad = p.kchunks * KB;
   p.ntaps = d->ntaps;
   const int stage_bytes = kABytes + BN * 128;
-  p.use_tma_out = (!(d->flags & ISWM_EPI_OUT_F32) && (d->out_ld % 8) == 0 &&
+  p.use_tma_out = (!f8 && !(d->flags & ISWM_EPI_OUT_F32) && (d->out_ld % 8) == 0 &&
                    (reinterpret_cast<uintptr_t>(d_out) & 15) == 0) ? 1 : 0;
   ISWM_REQUIRE(!(d->flags & ISWM_EPI_RESIDUAL) || (reinterpret_cast<uintptr_t>(d_res) & 15) == 0 || (d->res_ld & 7) != 0,
                "conv_igemm: a residual with res_ld %% 8 == 0 must be 16-byte aligned");
@@ -709,10 +805,12 @@ extern "C" int iswm_conv_igemm_ex(const iswm_conv_desc* d, const void* d_in, con
   if (p.use_tma_out) fixed += kEpiWG * kStageBuf;
   // epilogue-bound (short-K) convolutions hide the residual read behind a shared-memory prefetch; long-K ones keep
   // the ring stage instead and load the residual directly under the TMEM read
-  p.res_prefetch = ((d->flags & ISWM_EPI_RESIDUAL) && (d->res_ld % 8) == 0 && d->ntaps * p.kchunks <= 16) ? 1 : 0;
+  p.res_prefetch = (!f8 && (d->flags & ISWM_EPI_RESIDUAL) && (d->res_ld % 8) == 0 && d->ntaps * p.kchunks <= 16) ? 1 : 0;
   if (p.res_prefetch) fixed += kEpiWG * kStageBuf;
   p.stages = std::max(2, std::min(kMaxStages, (kSmemMax - fixed) / stage_bytes));
-  p.flags = d->flags;
+  p.flags = d->flags | ((f8 && out_type == ISWM_F32) ? ISWM_EPI_OUT_F32 : 0);
+  p.res_scale = res_scale;
+  p.out_f8 = (f8 && out_type == ISWM_E4M3) ? 1 : 0;
   p.n_img_per_phase = B;
   p.out_ld = d->out_ld;
   p.res_ld = d->res_ld;
@@ -733,7 +831,7 @@ extern "C" int iswm_conv_igemm_ex(const iswm_conv_desc* d, const void* d_in, con
     p.wtap[t] = d->wtap[t] > 0 ? (int8_t)(d->wtap[t] - 1) : (int8_t)t;
     ISWM_REQUIRE(d->coff[t] >= 0 && (d->coff[t] % 8) == 0 && d->coff[t] + d->Cin <= d->in_ld,
                  "conv_igemm: tap %d channel offset %d (must be a multiple of 8 with offset + Cin <= in_ld)", t, (int)d->coff[t]);
-    ISWM_REQUIRE(d->coff[t] == 0 || (d->Cin % kKBlock) == 0, "conv_igemm: channel-offset taps need Cin %% 64 == 0 (the K tail is zero-filled by the tensor map's edge)");
+    ISWM_REQUIRE(d->coff[t] == 0 || (d->Cin % KB) == 0, "conv_igemm: channel-offset taps need Cin %% %d == 0 (the K tail is zero-filled by the tensor map's edge)", KB);
     in_c = std::max(in_c, d->coff[t] + d->Cin);
   }
   p.out = d_out; p.scale = d_scale; p.shift = d_shift;
@@ -744,21 +842,22 @@ extern "C" int iswm_conv_igemm_ex(const iswm_conv_desc* d, const void* d_in, con
   ISWM_REQUIRE(p.stats_rep <= 64, "conv_igemm: stats_replicas=%d (at most 64)", d->stats_replicas);
   p.abort_flag = abort_flag;
 
+  auto encode = f8 ? encode_tmap_u8 : encode_tmap_bf16;
   CUtensorMap tmap_a, tmap_b;
   if (phase_view) {
     // dense [B, 2Hi, 2Wi, ld] read as four parity phases: {column parity * ld + channel, w, row parity, h, image}
     const uint64_t ld = (uint64_t)d->in_ld, Wf = 2ull * Wi, Hf = 2ull * Hi;
     const uint64_t dims[5] = {ld + (uint64_t)in_c, (uint64_t)Wi, 2, (uint64_t)Hi, (uint64_t)B};
     const uint64_t str[5] = {1, 2 * ld, Wf * ld, 2 * Wf * ld, Hf * Wf * ld};
-    const uint32_t box[5] = {(uint32_t)kKBlock, (uint32_t)BW, 1, (uint32_t)BH, (uint32_t)BB};
-    if (int rc = encode_tmap_bf16(&tmap_a, d_in, 5, dims, str, box)) return rc;
+    const uint32_t box[5] = {(uint32_t)KB, (uint32_t)BW, 1, (uint32_t)BH, (uint32_t)BB};
+    if (int rc = encode(&tmap_a, d_in, 5, dims, str, box)) return rc;
     p.phase_view = 1;
     p.pv_ld = d->in_ld;
   } else {
     const uint64_t dims[4] = {(uint64_t)in_c, (uint64_t)Wi, (uint64_t)Hi, (uint64_t)n_img};
     const uint64_t str[4] = {1, (uint64_t)d->in_ld, (uint64_t)Wi * d->in_ld, (uint64_t)Hi * Wi * d->in_ld};
-    const uint32_t box[4] = {(uint32_t)kKBlock, (uint32_t)BW, (uint32_t)BH, (uint32_t)BB};
-    if (int rc = encode_tmap_bf16(&tmap_a, d_in, 4, dims, str, box)) return rc;
+    const uint32_t box[4] = {(uint32_t)KB, (uint32_t)BW, (uint32_t)BH, (uint32_t)BB};
+    if (int rc = encode(&tmap_a, d_in, 4, dims, str, box)) return rc;
   }
   {
     const int w_ntaps = d->w_ntaps > 0 ? d->w_ntaps : d->ntaps;
@@ -767,8 +866,8 @@ extern "C" int iswm_conv_igemm_ex(const iswm_conv_desc* d, const void* d_in, con
     const uint64_t ktot = (uint64_t)w_ntaps * p.cin_pad;
     const uint64_t dims[2] = {ktot, (uint64_t)d->Cout};
     const uint64_t str[2] = {1, ktot};
-    const uint32_t box[2] = {(uint32_t)kKBlock, (uint32_t)BN};
-    if (int rc = encode_tmap_bf16(&tmap_b, d_wgt, 2, dims, str, box)) return rc;
+    const uint32_t box[2] = {(uint32_t)KB, (uint32_t)BN};
+    if (int rc = encode(&tmap_b, d_wgt, 2, dims, str, box)) return rc;
   }
   CUtensorMap tmap_out = tmap_a;                         // placeholder when unused
   if (p.use_tma_out) {
@@ -780,12 +879,13 @@ extern "C" int iswm_conv_igemm_ex(const iswm_conv_desc* d, const void* d_in, con
     if (int rc = encode_tmap_bf16(&tmap_out, d_out, 4, dims, str, box)) return rc;
   }
   const int smem_bytes = p.stages * stage_bytes + fixed;
-  static bool attr_set = false;
-  if (!attr_set) {
-    const cudaError_t e = cudaFuncSetAttribute(conv_igemm_kernel, cudaFuncAttributeMaxDynamicSharedMemorySize, 232448);
+  auto kernel = f8 ? conv_igemm_f8_kernel : conv_igemm_kernel;
+  static bool attr_set[2] = {false, false};
+  if (!attr_set[f8]) {
+    const cudaError_t e = cudaFuncSetAttribute(kernel, cudaFuncAttributeMaxDynamicSharedMemorySize, 232448);
     ISWM_REQUIRE(e == cudaSuccess, "conv_igemm: cudaFuncSetAttribute: %s", cudaGetErrorString(e));
     static_assert(kSmemMax == 232448, "opt-in shared memory limit of sm_100");
-    attr_set = true;
+    attr_set[f8] = true;
   }
   const int grid = std::min(p.total_tiles, num_sms());
   {
@@ -800,8 +900,21 @@ extern "C" int iswm_conv_igemm_ex(const iswm_conv_desc* d, const void* d_in, con
   // second producer warp: pays off when a k-block's MMA time (128 x BN x 64) is short against the ~300-cycle issue path of
   // one producer thread, i.e. for narrow N tiles
   p.nprod = (BN <= 128 && p.stages >= 4) ? 2 : 1;
-  launch_k(conv_igemm_kernel, dim3(grid), dim3(kConvThreads), smem_bytes, static_cast<cudaStream_t>(stream), tmap_a, tmap_b, tmap_out, p);
-  return check_launch("conv_igemm");
+  launch_k(kernel, dim3(grid), dim3(kConvThreads), smem_bytes, static_cast<cudaStream_t>(stream), tmap_a, tmap_b, tmap_out, p);
+  return check_launch(f8 ? "conv_igemm_f8" : "conv_igemm");
+}
+
+extern "C" int iswm_conv_igemm_ex(const iswm_conv_desc* d, const void* d_in, const void* d_wgt,
+                                  void* d_out, const float* d_scale, const float* d_shift,
+                                  const void* d_res, double* d_stats, const uint8_t* d_res_mask, void* stream) {
+  if (debug_skip(ISWM_SKIP_CONV_IGEMM)) return 0;
+  return conv_igemm_launch(d, d_in, d_wgt, d_out, d_scale, d_shift, d_res, d_stats, d_res_mask, false, 1.f, ISWM_BF16, stream);
+}
+
+extern "C" int iswm_conv_igemm_f8(const iswm_conv_desc* d, const void* d_in, const void* d_wgt, void* d_out,
+                                  const float* d_scale, const float* d_shift, const void* d_res, float res_scale,
+                                  int out_type, void* stream) {
+  return conv_igemm_launch(d, d_in, d_wgt, d_out, d_scale, d_shift, d_res, nullptr, nullptr, true, res_scale, out_type, stream);
 }
 
 extern "C" int iswm_aspp_bwd(const void* d_dycat, int dy_ld, const void* d_wcat, int B, int H, int W, int Cb, int Cfeat,

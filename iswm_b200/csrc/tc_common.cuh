@@ -154,6 +154,17 @@ __device__ __forceinline__ void umma_bf16(uint32_t tmem_d, uint64_t desc_a, uint
       "l"(desc_a), "l"(desc_b), "r"(idesc), "r"(accumulate)
       : "memory");
 }
+// D[tmem] (+)= A[smem] * B[smem], e4m3 x e4m3 -> fp32 (kind::f8f6f4: K = 32 per instruction, the same 32 bytes of a
+// 128-byte swizzle row as one bf16 step), issued by ONE thread
+__device__ __forceinline__ void umma_f8(uint32_t tmem_d, uint64_t desc_a, uint64_t desc_b,
+                                        uint32_t idesc, uint32_t accumulate) {
+  asm volatile(
+      "{\n\t.reg .pred p;\n\t"
+      "setp.ne.b32 p, %4, 0;\n\t"
+      "tcgen05.mma.cta_group::1.kind::f8f6f4 [%0], %1, %2, %3, p;\n\t}\n" ::"r"(tmem_d),
+      "l"(desc_a), "l"(desc_b), "r"(idesc), "r"(accumulate)
+      : "memory");
+}
 // arrive on an mbarrier once all previously issued MMAs of this thread retire
 __device__ __forceinline__ void umma_commit(uint32_t bar) {
   asm volatile("tcgen05.commit.cta_group::1.mbarrier::arrive::one.shared::cluster.b64 [%0];" ::"r"(bar)
@@ -191,6 +202,14 @@ __host__ __device__ constexpr uint32_t make_idesc_bf16(int M, int N, int a_mn_ma
          | ((uint32_t)(N >> 3) << 17)
          | ((uint32_t)(M >> 4) << 24);
 }
+// instruction descriptor, kind::f8f6f4, A/B E4M3 (format code 0), D fp32, both K-major
+__host__ __device__ constexpr uint32_t make_idesc_e4m3(int M, int N) {
+  return (1u << 4)                         // c_format = F32
+         | (0u << 7)                       // a_format = E4M3
+         | (0u << 10)                      // b_format = E4M3
+         | ((uint32_t)(N >> 3) << 17)
+         | ((uint32_t)(M >> 4) << 24);
+}
 // shared-memory matrix descriptor, 128-byte swizzle, sm_100 version bit set
 __device__ __forceinline__ uint64_t make_smem_desc_sw128(uint32_t saddr, uint32_t lbo_bytes,
                                                          uint32_t sbo_bytes) {
@@ -210,6 +229,9 @@ __device__ __forceinline__ uint64_t make_smem_desc_sw128(uint32_t saddr, uint32_
 // dims/strides in elements (stride[0] is implicit = 1); returns 0 on success.
 int encode_tmap_bf16(CUtensorMap* out, const void* base, int rank, const uint64_t* dims,
                      const uint64_t* strides_elems, const uint32_t* box);
+// Same for one-byte elements (e4m3 activations and weights): UINT8 map, strides in bytes.
+int encode_tmap_u8(CUtensorMap* out, const void* base, int rank, const uint64_t* dims,
+                   const uint64_t* strides_elems, const uint32_t* box);
 int* abort_flag_ptr();                       // device int, 0 = healthy
 int read_abort_flag(int* out, bool reset);   // synchronising; tests / debug only
 

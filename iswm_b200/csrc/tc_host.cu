@@ -18,8 +18,8 @@ static PFN_cuTensorMapEncodeTiled_v12000 get_encode_fn() {
   return fn;
 }
 
-int encode_tmap_bf16(CUtensorMap* out, const void* base, int rank, const uint64_t* dims,
-                     const uint64_t* strides_elems, const uint32_t* box) {
+static int encode_tmap(CUtensorMapDataType dtype, int esize, CUtensorMap* out, const void* base, int rank,
+                       const uint64_t* dims, const uint64_t* strides_elems, const uint32_t* box) {
   auto fn = get_encode_fn();
   if (!fn) {
     set_error("cuTensorMapEncodeTiled entry point unavailable (no CUDA driver?)");
@@ -32,9 +32,9 @@ int encode_tmap_bf16(CUtensorMap* out, const void* base, int rank, const uint64_
     gdim[i] = dims[i];
     bx[i] = box[i];
     es[i] = 1;
-    if (i > 0) gstr[i - 1] = strides_elems[i] * 2;  // bytes
+    if (i > 0) gstr[i - 1] = strides_elems[i] * esize;  // bytes
   }
-  CUresult r = fn(out, CU_TENSOR_MAP_DATA_TYPE_BFLOAT16, (cuuint32_t)rank, const_cast<void*>(base),
+  CUresult r = fn(out, dtype, (cuuint32_t)rank, const_cast<void*>(base),
                   gdim, gstr, bx, es, CU_TENSOR_MAP_INTERLEAVE_NONE, CU_TENSOR_MAP_SWIZZLE_128B,
                   CU_TENSOR_MAP_L2_PROMOTION_L2_256B, CU_TENSOR_MAP_FLOAT_OOB_FILL_NONE);
   if (r != CUDA_SUCCESS) {
@@ -48,6 +48,16 @@ int encode_tmap_bf16(CUtensorMap* out, const void* base, int rank, const uint64_
     return 3;
   }
   return 0;
+}
+
+int encode_tmap_bf16(CUtensorMap* out, const void* base, int rank, const uint64_t* dims,
+                     const uint64_t* strides_elems, const uint32_t* box) {
+  return encode_tmap(CU_TENSOR_MAP_DATA_TYPE_BFLOAT16, 2, out, base, rank, dims, strides_elems, box);
+}
+
+int encode_tmap_u8(CUtensorMap* out, const void* base, int rank, const uint64_t* dims,
+                   const uint64_t* strides_elems, const uint32_t* box) {
+  return encode_tmap(CU_TENSOR_MAP_DATA_TYPE_UINT8, 1, out, base, rank, dims, strides_elems, box);
 }
 
 int* abort_flag_ptr() {
