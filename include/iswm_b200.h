@@ -230,6 +230,22 @@ int iswm_peer_allreduce_f32(const void* const* buf_ptrs, int rank, int world, in
 int iswm_peer_small_publish(const void* const* slot_ptrs, int rank, int world, const void* d_src, int n, int slot_off, int is_f64, void* stream);
 int iswm_peer_small_sum(const void* const* slot_ptrs, int world, void* d_dst, int n, int slot_off, int is_f64, void* stream);
 
+/* Synchronised BatchNorm statistics exchange (one launch, one block). The fp64 vectors live in a symmetric arena that every
+ * rank carves at the same offsets: job j reads n values x `replicas` copies (iswm_conv_desc.stats_replicas layout: n = 2*C
+ * forward, replicas 1 backward) at arena_ptrs[q] + src_off on every rank q. The kernel writes `count` (this rank's rows) into
+ * the word after job 0's copies, passes a barrier on flag_ptrs / d_epoch (as iswm_peer_barrier), then stores
+ * dst[i] = sum over ranks 0..world-1 in that order of (sum of the copies in order) - identical bits on every rank - and
+ * dst[n] = the sum of the ranks' counts. flag_ptrs NULL (world = 1 only): no barrier - folds the copies and writes the count
+ * (what a torch.distributed transport then all-reduces). At most 4 jobs per call, all with the same row count. */
+typedef struct {
+  int64_t src_off;              /* fp64 elements from the arena base */
+  double* dst;                  /* local: double[n + 1] */
+  int32_t n;
+  int32_t replicas;
+} iswm_syncbn_job;
+int iswm_syncbn_exchange(const iswm_syncbn_job* jobs, int n_jobs, const void* const* arena_ptrs, const void* const* flag_ptrs,
+                         int rank, int world, double count, uint32_t* d_epoch, void* stream);
+
 /* Weight gradient: dW[n, t, c] += sum_{b,ho,wo} dy[b,ho,wo,n] * in[img(t,b), ho+dh[t], wo+dw[t], c]
  * desc as for the forward conv (Cout = channels of dy). d_dw: float [Cout][ntaps][Cin],
  * ACCUMULATED into with fp32 reductions (zero it first). dy row pitch = out_ld. */
@@ -326,6 +342,15 @@ int iswm_bn_train_apply(const void* d_x, int x_ld, const double* d_stats, int st
                         float* d_save_mean, float* d_save_invstd, const void* d_res, int res_ld, int relu,
                         float drop_p, uint64_t drop_seed, const int64_t* d_drop_step, void* d_out, int out_ld,
                         uint8_t* d_relu_bits, void* stream);
+/* Synchronised BatchNorm (iswm_syncbn_exchange): d_gstats = double[2*C + 1], the sums over every rank's rows (one copy) and the
+ * global row count; mean, variance and the running variance's unbiased factor use that count, M is this rank's rows. With
+ * the local sums and count = M it computes exactly what iswm_bn_train_apply does. */
+int iswm_bn_train_apply_global(const void* d_x, int x_ld, const double* d_gstats, int64_t M, int C,
+                               const float* d_gamma, const float* d_beta, float eps, float momentum,
+                               float* d_running_mean, float* d_running_var, int64_t* d_num_batches_tracked,
+                               float* d_save_mean, float* d_save_invstd, const void* d_res, int res_ld, int relu,
+                               float drop_p, uint64_t drop_seed, const int64_t* d_drop_step, void* d_out, int out_ld,
+                               uint8_t* d_relu_bits, void* stream);
 
 /* eval-mode BN folding: scale = gamma / sqrt(running_var + eps), shift = beta - mean*scale */
 int iswm_bn_fold(const float* d_gamma, const float* d_beta, const float* d_mean, const float* d_var,
@@ -350,6 +375,15 @@ int iswm_bn_bwd_apply(const void* d_dout, int dout_ld, const void* d_x, int x_ld
                       const float* d_save_invstd, const double* d_sums, int relu, float drop_p, uint64_t drop_seed, const int64_t* d_drop_step,
                       void* d_dx, int dx_ld, void* d_dz, int dz_ld,
                       float* d_dgamma, float* d_dbeta, void* stream);
+/* Synchronised BatchNorm: d_gsums = double[2*C + 1], the exchanged sums of iswm_bn_bwd_reduce over every rank and the global
+ * row count (the normaliser); dgamma / dbeta accumulate THIS rank's sums d_local_sums, so that a SUM all-reduce of the
+ * parameter gradients yields the global values. */
+int iswm_bn_bwd_apply_global(const void* d_dout, int dout_ld, const void* d_x, int x_ld,
+                             const void* d_out_act, int act_ld, int64_t M, int C,
+                             const float* d_gamma, const float* d_beta, const float* d_save_mean,
+                             const float* d_save_invstd, const double* d_gsums, const double* d_local_sums, int relu, float drop_p,
+                             uint64_t drop_seed, const int64_t* d_drop_step, void* d_dx, int dx_ld, void* d_dz, int dz_ld,
+                             float* d_dgamma, float* d_dbeta, void* stream);
 
 /* ---- the closing BatchNorm of a bottleneck block WITH a downsample branch, both branches per pass (csrc/bn_dual.cu) ----
  *   out = relu( bn3(raw) + bn_ds(raw_ds) )        network/backbone/resnet.py:110-118 with `downsample` (:176-186)
@@ -386,6 +420,17 @@ int iswm_bn_dual_bwd_apply(const void* d_dout, int dout_ld, const uint8_t* d_rel
                            const void* d_x_ds, int x_ds_ld, const iswm_bn_side* ds_bn, const double* d_sums_ds,
                            int64_t M, int C, void* d_dx, int dx_ld, void* d_dx_ds, int dx_ds_ld,
                            float* d_dgamma, float* d_dbeta, float* d_dgamma_ds, float* d_dbeta_ds, void* stream);
+/* Synchronised BatchNorm forms: the sides' stats (forward) and d_gsums / d_gsums_ds (backward) are double[2*C + 1] exchanged
+ * sums with the global row count (iswm_syncbn_exchange; one copy); the backward adds the local sums into dgamma / dbeta. */
+int iswm_bn_dual_train_apply_global(const void* d_x, int x_ld, const iswm_bn_side* main_bn,
+                                    const void* d_x_ds, int x_ds_ld, const iswm_bn_side* ds_bn,
+                                    int64_t M, int C, float eps, float momentum,
+                                    void* d_out, int out_ld, uint8_t* d_relu_bits, void* stream);
+int iswm_bn_dual_bwd_apply_global(const void* d_dout, int dout_ld, const uint8_t* d_relu_bits,
+                                  const void* d_x, int x_ld, const iswm_bn_side* main_bn, const double* d_gsums, const double* d_local_sums,
+                                  const void* d_x_ds, int x_ds_ld, const iswm_bn_side* ds_bn, const double* d_gsums_ds,
+                                  const double* d_local_sums_ds, int64_t M, int C, void* d_dx, int dx_ld, void* d_dx_ds, int dx_ds_ld,
+                                  float* d_dgamma, float* d_dbeta, float* d_dgamma_ds, float* d_dbeta_ds, void* stream);
 
 /* ---- stem tail: BatchNorm + ReLU + 3x3/s2/p1 max pooling in ONE pass (csrc/stem_pool.cu; network/backbone/resnet.py:145-147) ----
  * d_raw bf16 [B,H,W,64] = the stem convolution's pre-BN output (with its statistics in bn->stats); writes the pooled
@@ -394,6 +439,9 @@ int iswm_bn_dual_bwd_apply(const void* d_dout, int dout_ld, const uint8_t* d_rel
  * updated, save_mean / save_invstd written. */
 int iswm_stem_pool_fwd(const void* d_raw, const iswm_bn_side* bn, int B, int H, int W, int C, int Ho, int Wo,
                        float eps, float momentum, void* d_out, uint8_t* d_idx, void* stream);
+/* Synchronised BatchNorm form: bn->stats = double[2*64 + 1] exchanged sums with the global pixel count (one copy). */
+int iswm_stem_pool_fwd_global(const void* d_raw, const iswm_bn_side* bn, int B, int H, int W, int C, int Ho, int Wo,
+                              float eps, float momentum, void* d_out, uint8_t* d_idx, void* stream);
 
 /* Stem 7x7 / stride 2 / pad 3 (network/backbone/resnet.py:144), ROW-TAP form - what the engine runs. The fp32 NCHW image is
  * unrolled along x only: d_out bf16 [2][B][Hh][Wo][kpitch], element [p][b][hh][wo][s*Cin + c] = img[b][c][2*hh + p][2*wo + s - 3]

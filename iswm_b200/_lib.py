@@ -66,6 +66,12 @@ class UnpackJob(C.Structure):
                 ("chunks", C.c_int32), ("blk_begin", C.c_int32), ("pad_", C.c_int32)]
 
 
+class SyncBnJob(C.Structure):
+    """Mirror of iswm_syncbn_job."""
+
+    _fields_ = [("src_off", C.c_int64), ("dst", C.c_void_p), ("n", C.c_int32), ("replicas", C.c_int32)]
+
+
 def fill_unpack_jobs(jobs):
     """jobs: list of (src_ptr, dst_ptr, Cout, Cin, RS) -> (ctypes array, total_blocks)."""
     arr = (UnpackJob * len(jobs))()
@@ -115,6 +121,7 @@ SIGNATURES = {
     "iswm_peer_allreduce_f32": (_i, [C.POINTER(_p), _i, _i, _i64, _i64, _i, _p]),
     "iswm_peer_small_publish": (_i, [C.POINTER(_p), _i, _i, _p, _i, _i, _i, _p]),
     "iswm_peer_small_sum": (_i, [C.POINTER(_p), _i, _p, _i, _i, _i, _p]),
+    "iswm_syncbn_exchange": (_i, [C.POINTER(SyncBnJob), _i, C.POINTER(_p), C.POINTER(_p), _i, _i, C.c_double, _p, _p]),
     "iswm_conv_wgrad": (_i, [C.POINTER(ConvDesc), _p, _p, _p, _p]),
     "iswm_conv_wgrad_grouped": (_i, [C.POINTER(ConvDesc), C.POINTER(_p), C.POINTER(_p), C.POINTER(_p), _i, _p]),
     "iswm_conv_wgrad_ex": (_i, [C.POINTER(ConvDesc), _p, _p, _p, _i, _p]),
@@ -125,14 +132,20 @@ SIGNATURES = {
     "iswm_unpack_wgrad": (_i, [_p, _i, _i, _i, _i, _i, _f, _p, _p]),
     "iswm_unpack_wgrad_batched": (_i, [_p, _i, _i, _p]),
     "iswm_bn_train_apply": (_i, [_p, _i, _p, _i, _i64, _i, _p, _p, _f, _f, _p, _p, _p, _p, _p, _p, _i, _i, _f, _u64, _p, _p, _i, _p, _p]),
+    "iswm_bn_train_apply_global": (_i, [_p, _i, _p, _i64, _i, _p, _p, _f, _f, _p, _p, _p, _p, _p, _p, _i, _i, _f, _u64, _p, _p, _i, _p, _p]),
     "iswm_bn_fold": (_i, [_p, _p, _p, _p, _f, _i, _p, _p, _p]),
     "iswm_bn_bwd_reduce": (_i, [_p, _i, _p, _i, _p, _i, _i64, _i, _p, _p, _p, _p, _i, _f, _u64, _p, _p, _p]),
     "iswm_bn_bwd_apply": (_i, [_p, _i, _p, _i, _p, _i, _i64, _i, _p, _p, _p, _p, _p, _i, _f, _u64, _p, _p, _i, _p, _i, _p, _p, _p]),
+    "iswm_bn_bwd_apply_global": (_i, [_p, _i, _p, _i, _p, _i, _i64, _i, _p, _p, _p, _p, _p, _p, _i, _f, _u64, _p, _p, _i, _p, _i, _p, _p, _p]),
     "iswm_bn_dual_train_apply": (_i, [_p, _i, C.POINTER(BnSide), _p, _i, C.POINTER(BnSide), _i64, _i, _f, _f, _p, _i, _p, _p]),
     "iswm_bn_dual_bwd_reduce": (_i, [_p, _i, _p, _p, _i, C.POINTER(BnSide), _p, _i, C.POINTER(BnSide), _i64, _i, _p, _p, _p]),
     "iswm_bn_dual_bwd_apply": (_i, [_p, _i, _p, _p, _i, C.POINTER(BnSide), _p, _p, _i, C.POINTER(BnSide), _p, _i64, _i, _p, _i, _p, _i,
                                     _p, _p, _p, _p, _p]),
+    "iswm_bn_dual_train_apply_global": (_i, [_p, _i, C.POINTER(BnSide), _p, _i, C.POINTER(BnSide), _i64, _i, _f, _f, _p, _i, _p, _p]),
+    "iswm_bn_dual_bwd_apply_global": (_i, [_p, _i, _p, _p, _i, C.POINTER(BnSide), _p, _p, _p, _i, C.POINTER(BnSide), _p, _p, _i64, _i, _p, _i,
+                                           _p, _i, _p, _p, _p, _p, _p]),
     "iswm_stem_pool_fwd": (_i, [_p, C.POINTER(BnSide), _i, _i, _i, _i, _i, _i, _f, _f, _p, _p, _p]),
+    "iswm_stem_pool_fwd_global": (_i, [_p, C.POINTER(BnSide), _i, _i, _i, _i, _i, _i, _f, _f, _p, _p, _p]),
     "iswm_stem_rows": (_i, [_p, _i, _i, _i, _i, _i, _i, _i, _p, _p]),
     "iswm_unpack_wgrad_stem": (_i, [_p, _i, _i, _i, _i, _f, _p, _p]),
     "iswm_stem_im2col": (_i, [_p, _i, _i, _i, _i, _i, _i, _i, _p, _p]),

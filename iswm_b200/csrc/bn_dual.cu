@@ -31,6 +31,9 @@ struct BnSide {                      // one BatchNorm's per-channel vectors
 };
 
 // ------------------------------------------------------------------------------------------------------------- forward
+// GCNT (synchronised BatchNorm): each side's `stats` holds the sums over every rank's rows (one copy) followed by the global
+// row count at [2C]; M only bounds this rank's row walk
+template <bool GCNT>
 __global__ void __launch_bounds__(kT, 2)
 bn_dual_train_apply_kernel(const __nv_bfloat16* __restrict__ xa, int xa_ld, const __nv_bfloat16* __restrict__ xb, int xb_ld,
                            BnSide A, BnSide Bs, int64_t M, int C, float eps, float momentum,
@@ -54,7 +57,8 @@ bn_dual_train_apply_kernel(const __nv_bfloat16* __restrict__ xa, int xa_ld, cons
       rb[u] = load_raw(pb + u * sb);
     }
   }
-  const double invM = 1.0 / (double)M;
+  const double cnt = GCNT ? A.stats[2 * C] : 0.0;
+  const double invM = GCNT ? 1.0 / cnt : 1.0 / (double)M;
   float sc[8], sc2[8], sh[8];         // out = relu(x*sc + y*sc2 + sh), sh = both shifts
   auto side = [&](const BnSide& S, float* scv, float* shv) {
 #pragma unroll
@@ -75,7 +79,9 @@ bn_dual_train_apply_kernel(const __nv_bfloat16* __restrict__ xa, int xa_ld, cons
         S.save_mean[c] = mean;
         S.save_invstd[c] = invstd;
         if (S.running_mean) {
-          const float unbiased = (M > 1) ? var * ((float)M / (float)(M - 1)) : var;
+          float unbiased;
+          if (GCNT) unbiased = (cnt > 1.0) ? var * ((float)cnt / (float)(cnt - 1.0)) : var;
+          else unbiased = (M > 1) ? var * ((float)M / (float)(M - 1)) : var;
           S.running_mean[c] = (1.f - momentum) * S.running_mean[c] + momentum * mean;
           S.running_var[c] = (1.f - momentum) * S.running_var[c] + momentum * unbiased;
         }
@@ -219,12 +225,15 @@ struct BnBwdSide {
   float* dbeta;
 };
 
+// GCNT (synchronised BatchNorm): the sides' `sums` are the sums over every rank's rows with the global row count at [2C];
+// dgamma / dbeta accumulate this rank's own sums (lsums_a / lsums_b)
+template <bool GCNT>
 __global__ void __launch_bounds__(kT, 2)
 bn_dual_bwd_apply_kernel(const __nv_bfloat16* __restrict__ dout, int dout_ld, const uint8_t* __restrict__ bits,
                          const __nv_bfloat16* __restrict__ xa, int xa_ld, const __nv_bfloat16* __restrict__ xb, int xb_ld,
                          int64_t M, int C, BnBwdSide A, BnBwdSide Bs,
                          __nv_bfloat16* __restrict__ dxa, int dxa_ld, __nv_bfloat16* __restrict__ dxb, int dxb_ld,
-                         int nx, int ny, int rows_per_block) {
+                         int nx, int ny, int rows_per_block, const double* __restrict__ lsums_a, const double* __restrict__ lsums_b) {
   pdl_wait();
   pdl_launch();
   const int tx = threadIdx.x % nx, ty = threadIdx.x / nx;
@@ -248,10 +257,10 @@ bn_dual_bwd_apply_kernel(const __nv_bfloat16* __restrict__ dout, int dout_ld, co
       mb[u] = pm[u * sm_];
     }
   }
-  const float invM = 1.0f / (float)M;
+  const float invM = GCNT ? 1.0f / (float)A.sums[2 * C] : 1.0f / (float)M;
   // dx = k*dz + p*x + q  with  k = gamma*invstd, p = -k*invstd*mean(dz*xhat), q = -k*mean(dz) - p*mu   (per branch)
   float ka[8], pa_[8], qa[8], kb[8], pb_[8], qb[8];
-  auto side = [&](const BnBwdSide& S, float* kk, float* pp, float* qq) {
+  auto side = [&](const BnBwdSide& S, const double* ls, float* kk, float* pp, float* qq) {
 #pragma unroll
     for (int j = 0; j < 8; j++) {
       const int c = c0 + j;
@@ -262,13 +271,13 @@ bn_dual_bwd_apply_kernel(const __nv_bfloat16* __restrict__ dout, int dout_ld, co
       pp[j] = -k * is * (s1 * invM);
       qq[j] = -k * (s0 * invM) - pp[j] * mu;
       if (blockIdx.x == 0 && ty == 0) {
-        if (S.dbeta) S.dbeta[c] += s0;
-        if (S.dgamma) S.dgamma[c] += s1;
+        if (S.dbeta) S.dbeta[c] += GCNT ? (float)ls[c] : s0;
+        if (S.dgamma) S.dgamma[c] += GCNT ? (float)ls[C + c] : s1;
       }
     }
   };
-  side(A, ka, pa_, qa);
-  side(Bs, kb, pb_, qb);
+  side(A, lsums_a, ka, pa_, qa);
+  side(Bs, lsums_b, kb, pb_, qb);
   __nv_bfloat16* oa = dxa + w.first * dxa_ld + c0;
   __nv_bfloat16* ob = dxb + w.first * dxb_ld + c0;
   const int64_t soa = (int64_t)ny * dxa_ld, sob = (int64_t)ny * dxb_ld;
@@ -319,23 +328,41 @@ static int check_dual(const char* what, int64_t M, int C, int ld0, int ld1, int 
   return 0;
 }
 
-extern "C" int iswm_bn_dual_train_apply(const void* d_x, int x_ld, const iswm_bn_side* main_bn,
-                                        const void* d_x_ds, int x_ds_ld, const iswm_bn_side* ds_bn,
-                                        int64_t M, int C, float eps, float momentum,
-                                        void* d_out, int out_ld, uint8_t* d_relu_bits, void* stream) {
+static int bn_dual_train_apply_impl(bool global, const void* d_x, int x_ld, const iswm_bn_side* main_bn,
+                                   const void* d_x_ds, int x_ds_ld, const iswm_bn_side* ds_bn,
+                                   int64_t M, int C, float eps, float momentum,
+                                   void* d_out, int out_ld, uint8_t* d_relu_bits, void* stream) {
   if (debug_skip(ISWM_SKIP_BN)) return 0;
   ISWM_REQUIRE(d_x && d_x_ds && main_bn && ds_bn && d_out, "bn_dual_train_apply: null argument");
   if (int rc = check_dual("bn_dual_train_apply", M, C, x_ld, x_ds_ld, out_ld)) return rc;
-  for (const iswm_bn_side* s : {main_bn, ds_bn})
+  for (const iswm_bn_side* s : {main_bn, ds_bn}) {
     ISWM_REQUIRE(s->stats && s->gamma && s->beta && s->save_mean && s->save_invstd, "bn_dual_train_apply: a BatchNorm side lacks stats / gamma / beta / save slots");
+    ISWM_REQUIRE(!global || s->stats_replicas <= 1, "bn_dual_train_apply_global: the global sums are one copy (stats_replicas=%d)", s->stats_replicas);
+  }
   int nx, ny, rpb, blocks;
   bn_row_grid(C, M, 4, nx, ny, rpb, blocks, 2);          // 2 resident blocks per SM (launch bounds): one wave
   auto mk = [](const iswm_bn_side* s) {
     return BnSide{s->stats, s->gamma, s->beta, s->running_mean, s->running_var, reinterpret_cast<long long*>(s->num_batches_tracked), s->save_mean, s->save_invstd, s->stats_replicas > 1 ? s->stats_replicas : 1};
   };
-  launch_k(bn_dual_train_apply_kernel, dim3(blocks), dim3(kT), 0, ST(stream), BF(d_x), x_ld, BF(d_x_ds), x_ds_ld, mk(main_bn), mk(ds_bn),
-           M, C, eps, momentum, BFW(d_out), out_ld, d_relu_bits, nx, ny, rpb);
+  if (global)
+    launch_k(bn_dual_train_apply_kernel<true>, dim3(blocks), dim3(kT), 0, ST(stream), BF(d_x), x_ld, BF(d_x_ds), x_ds_ld, mk(main_bn), mk(ds_bn),
+             M, C, eps, momentum, BFW(d_out), out_ld, d_relu_bits, nx, ny, rpb);
+  else
+    launch_k(bn_dual_train_apply_kernel<false>, dim3(blocks), dim3(kT), 0, ST(stream), BF(d_x), x_ld, BF(d_x_ds), x_ds_ld, mk(main_bn), mk(ds_bn),
+             M, C, eps, momentum, BFW(d_out), out_ld, d_relu_bits, nx, ny, rpb);
   return check_launch("bn_dual_train_apply");
+}
+extern "C" int iswm_bn_dual_train_apply(const void* d_x, int x_ld, const iswm_bn_side* main_bn,
+                                        const void* d_x_ds, int x_ds_ld, const iswm_bn_side* ds_bn,
+                                        int64_t M, int C, float eps, float momentum,
+                                        void* d_out, int out_ld, uint8_t* d_relu_bits, void* stream) {
+  return bn_dual_train_apply_impl(false, d_x, x_ld, main_bn, d_x_ds, x_ds_ld, ds_bn, M, C, eps, momentum, d_out, out_ld, d_relu_bits, stream);
+}
+extern "C" int iswm_bn_dual_train_apply_global(const void* d_x, int x_ld, const iswm_bn_side* main_bn,
+                                               const void* d_x_ds, int x_ds_ld, const iswm_bn_side* ds_bn,
+                                               int64_t M, int C, float eps, float momentum,
+                                               void* d_out, int out_ld, uint8_t* d_relu_bits, void* stream) {
+  return bn_dual_train_apply_impl(true, d_x, x_ld, main_bn, d_x_ds, x_ds_ld, ds_bn, M, C, eps, momentum, d_out, out_ld, d_relu_bits, stream);
 }
 
 extern "C" int iswm_bn_dual_bwd_reduce(const void* d_dout, int dout_ld, const uint8_t* d_relu_bits,
@@ -364,11 +391,11 @@ extern "C" int iswm_bn_dual_bwd_reduce(const void* d_dout, int dout_ld, const ui
   return check_launch("bn_dual_bwd_reduce");
 }
 
-extern "C" int iswm_bn_dual_bwd_apply(const void* d_dout, int dout_ld, const uint8_t* d_relu_bits,
-                                      const void* d_x, int x_ld, const iswm_bn_side* main_bn, const double* d_sums,
-                                      const void* d_x_ds, int x_ds_ld, const iswm_bn_side* ds_bn, const double* d_sums_ds,
-                                      int64_t M, int C, void* d_dx, int dx_ld, void* d_dx_ds, int dx_ds_ld,
-                                      float* d_dgamma, float* d_dbeta, float* d_dgamma_ds, float* d_dbeta_ds, void* stream) {
+static int bn_dual_bwd_apply_impl(const double* d_lsums, const double* d_lsums_ds, const void* d_dout, int dout_ld, const uint8_t* d_relu_bits,
+                                  const void* d_x, int x_ld, const iswm_bn_side* main_bn, const double* d_sums,
+                                  const void* d_x_ds, int x_ds_ld, const iswm_bn_side* ds_bn, const double* d_sums_ds,
+                                  int64_t M, int C, void* d_dx, int dx_ld, void* d_dx_ds, int dx_ds_ld,
+                                  float* d_dgamma, float* d_dbeta, float* d_dgamma_ds, float* d_dbeta_ds, void* stream) {
   if (debug_skip(ISWM_SKIP_BN)) return 0;
   ISWM_REQUIRE(d_dout && d_relu_bits && d_x && d_x_ds && main_bn && ds_bn && d_sums && d_sums_ds && d_dx && d_dx_ds, "bn_dual_bwd_apply: null argument");
   if (int rc = check_dual("bn_dual_bwd_apply", M, C, dout_ld, x_ld, x_ds_ld)) return rc;
@@ -379,7 +406,30 @@ extern "C" int iswm_bn_dual_bwd_apply(const void* d_dout, int dout_ld, const uin
   bn_row_grid(C, M, 4, nx, ny, rpb, blocks, 2);
   const BnBwdSide A{main_bn->gamma, main_bn->save_mean, main_bn->save_invstd, d_sums, d_dgamma, d_dbeta};
   const BnBwdSide Bs{ds_bn->gamma, ds_bn->save_mean, ds_bn->save_invstd, d_sums_ds, d_dgamma_ds, d_dbeta_ds};
-  launch_k(bn_dual_bwd_apply_kernel, dim3(blocks), dim3(kT), 0, ST(stream), BF(d_dout), dout_ld, d_relu_bits, BF(d_x), x_ld, BF(d_x_ds), x_ds_ld,
-           M, C, A, Bs, BFW(d_dx), dx_ld, BFW(d_dx_ds), dx_ds_ld, nx, ny, rpb);
+  if (d_lsums)
+    launch_k(bn_dual_bwd_apply_kernel<true>, dim3(blocks), dim3(kT), 0, ST(stream), BF(d_dout), dout_ld, d_relu_bits, BF(d_x), x_ld, BF(d_x_ds), x_ds_ld,
+             M, C, A, Bs, BFW(d_dx), dx_ld, BFW(d_dx_ds), dx_ds_ld, nx, ny, rpb, d_lsums, d_lsums_ds);
+  else
+    launch_k(bn_dual_bwd_apply_kernel<false>, dim3(blocks), dim3(kT), 0, ST(stream), BF(d_dout), dout_ld, d_relu_bits, BF(d_x), x_ld, BF(d_x_ds), x_ds_ld,
+             M, C, A, Bs, BFW(d_dx), dx_ld, BFW(d_dx_ds), dx_ds_ld, nx, ny, rpb, (const double*)nullptr, (const double*)nullptr);
   return check_launch("bn_dual_bwd_apply");
+}
+
+extern "C" int iswm_bn_dual_bwd_apply(const void* d_dout, int dout_ld, const uint8_t* d_relu_bits,
+                                      const void* d_x, int x_ld, const iswm_bn_side* main_bn, const double* d_sums,
+                                      const void* d_x_ds, int x_ds_ld, const iswm_bn_side* ds_bn, const double* d_sums_ds,
+                                      int64_t M, int C, void* d_dx, int dx_ld, void* d_dx_ds, int dx_ds_ld,
+                                      float* d_dgamma, float* d_dbeta, float* d_dgamma_ds, float* d_dbeta_ds, void* stream) {
+  return bn_dual_bwd_apply_impl(nullptr, nullptr, d_dout, dout_ld, d_relu_bits, d_x, x_ld, main_bn, d_sums, d_x_ds, x_ds_ld, ds_bn, d_sums_ds,
+                                M, C, d_dx, dx_ld, d_dx_ds, dx_ds_ld, d_dgamma, d_dbeta, d_dgamma_ds, d_dbeta_ds, stream);
+}
+
+extern "C" int iswm_bn_dual_bwd_apply_global(const void* d_dout, int dout_ld, const uint8_t* d_relu_bits,
+                                             const void* d_x, int x_ld, const iswm_bn_side* main_bn, const double* d_gsums, const double* d_local_sums,
+                                             const void* d_x_ds, int x_ds_ld, const iswm_bn_side* ds_bn, const double* d_gsums_ds,
+                                             const double* d_local_sums_ds, int64_t M, int C, void* d_dx, int dx_ld, void* d_dx_ds, int dx_ds_ld,
+                                             float* d_dgamma, float* d_dbeta, float* d_dgamma_ds, float* d_dbeta_ds, void* stream) {
+  ISWM_REQUIRE(d_local_sums && d_local_sums_ds, "bn_dual_bwd_apply_global: null local sums");
+  return bn_dual_bwd_apply_impl(d_local_sums, d_local_sums_ds, d_dout, dout_ld, d_relu_bits, d_x, x_ld, main_bn, d_gsums, d_x_ds, x_ds_ld, ds_bn,
+                                d_gsums_ds, M, C, d_dx, dx_ld, d_dx_ds, dx_ds_ld, d_dgamma, d_dbeta, d_dgamma_ds, d_dbeta_ds, stream);
 }

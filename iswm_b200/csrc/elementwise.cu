@@ -258,7 +258,9 @@ struct DropSeed {
 };
 
 // BatchNorm training forward: stats -> normalise (+residual, ReLU, dropout)
-template <bool RES, bool RELU, bool DROP>
+// GCNT (synchronised BatchNorm): `stats` holds the sums over every rank's rows (one copy) followed by the global row count at
+// [2C]; the count normalises and sets the running-variance factor, M only bounds this rank's row walk
+template <bool RES, bool RELU, bool DROP, bool GCNT = false>
 __global__ void __launch_bounds__(kT, 3)
 bn_train_apply_kernel(const __nv_bfloat16* __restrict__ x, int x_ld, const double* __restrict__ stats, int stats_rep,
                       int64_t M, int C, const float* __restrict__ gamma, const float* __restrict__ beta,
@@ -301,7 +303,8 @@ bn_train_apply_kernel(const __nv_bfloat16* __restrict__ x, int x_ld, const doubl
       if (RES) rr[u] = load_raw(pr + u * sr);
     }
   }
-  const double invM = 1.0 / (double)M;
+  const double cnt = GCNT ? stats[2 * C] : 0.0;
+  const double invM = GCNT ? 1.0 / cnt : 1.0 / (double)M;
   float sc[8], sh[8];
 #pragma unroll
   for (int j = 0; j < 8; j++) {
@@ -327,7 +330,9 @@ bn_train_apply_kernel(const __nv_bfloat16* __restrict__ x, int x_ld, const doubl
       if (save_mean) save_mean[c] = mean;
       if (save_invstd) save_invstd[c] = invstd;
       if (running_mean) {
-        const float unbiased = (M > 1) ? var * ((float)M / (float)(M - 1)) : var;
+        float unbiased;
+        if (GCNT) unbiased = (cnt > 1.0) ? var * ((float)cnt / (float)(cnt - 1.0)) : var;
+        else unbiased = (M > 1) ? var * ((float)M / (float)(M - 1)) : var;
         running_mean[c] = (1.f - momentum) * running_mean[c] + momentum * mean;
         running_var[c] = (1.f - momentum) * running_var[c] + momentum * unbiased;
       }
@@ -537,7 +542,9 @@ bn_bwd_reduce_kernel(const __nv_bfloat16* __restrict__ dout, int dout_ld,
 }
 
 // BatchNorm backward pass 2
-template <int MASK, bool DROP, bool DZ>
+// GCNT (synchronised BatchNorm): `sums` are the sums over every rank's rows with the global row count at [2C], and
+// dgamma / dbeta accumulate this rank's own sums `lsums` (the gradient all-reduce adds the other ranks')
+template <int MASK, bool DROP, bool DZ, bool GCNT = false>
 __global__ void __launch_bounds__(kT, 3)
 bn_bwd_apply_kernel(const __nv_bfloat16* __restrict__ dout, int dout_ld,
                     const __nv_bfloat16* __restrict__ x, int x_ld,
@@ -546,7 +553,7 @@ bn_bwd_apply_kernel(const __nv_bfloat16* __restrict__ dout, int dout_ld,
                     const float* __restrict__ invstd, const double* __restrict__ sums,
                     float drop_p, DropSeed drop_seed_in, __nv_bfloat16* __restrict__ dx, int dx_ld,
                     __nv_bfloat16* __restrict__ dz, int dz_ld, float* dgamma, float* dbeta, int nx,
-                    int ny, int rows_per_block) {
+                    int ny, int rows_per_block, const double* __restrict__ lsums) {
   pdl_wait();
   pdl_launch();
   const uint64_t drop_seed = DROP ? drop_seed_in.resolve() : 0ull;
@@ -571,7 +578,7 @@ bn_bwd_apply_kernel(const __nv_bfloat16* __restrict__ dout, int dout_ld,
       if (MASK == 1) orr[u] = load_raw(pa + u * sa_); else if (MASK == 3) { orr[u] = gr[u]; orr[u].x = pm[u * sm_]; } else orr[u] = gr[u];
     }
   }
-  const float invM = 1.0f / (float)M;
+  const float invM = GCNT ? 1.0f / (float)sums[2 * C] : 1.0f / (float)M;
   // dx = k*dz + p*x + q  with  k = gamma*invstd, p = -k*invstd*mean(dz*xhat), q = -k*mean(dz) - p*mu
   float kk[8], pp[8], qq[8], sh[8];
 #pragma unroll
@@ -586,8 +593,8 @@ bn_bwd_apply_kernel(const __nv_bfloat16* __restrict__ dout, int dout_ld,
     pp[j] = -k * is * mb;
     qq[j] = -k * ma - pp[j] * mu;
     if (blockIdx.x == 0 && ty == 0) {
-      if (dbeta) dbeta[c] += sa;
-      if (dgamma) dgamma[c] += sb;
+      if (dbeta) dbeta[c] += GCNT ? (float)lsums[c] : sa;
+      if (dgamma) dgamma[c] += GCNT ? (float)lsums[C + c] : sb;
     }
   }
   const float keep_scale = DROP ? 1.f / (1.f - drop_p) : 1.f;
@@ -1539,27 +1546,29 @@ extern "C" int iswm_unpack_wgrad(const float* d_dw, int Cout, int Cin, int RS, i
   return check_launch("unpack_wgrad");
 }
 
-extern "C" int iswm_bn_train_apply(const void* d_x, int x_ld, const double* d_stats, int stats_replicas, int64_t M, int C,
-                                   const float* d_gamma, const float* d_beta, float eps, float momentum,
-                                   float* d_running_mean, float* d_running_var, int64_t* d_nbt,
-                                   float* d_save_mean, float* d_save_invstd, const void* d_res, int res_ld,
-                                   int relu, float drop_p, uint64_t drop_seed, const int64_t* d_drop_step, void* d_out, int out_ld,
-                                   uint8_t* d_relu_bits, void* stream) {
+static int bn_train_apply_impl(bool global, const void* d_x, int x_ld, const double* d_stats, int stats_replicas, int64_t M, int C,
+                               const float* d_gamma, const float* d_beta, float eps, float momentum,
+                               float* d_running_mean, float* d_running_var, int64_t* d_nbt,
+                               float* d_save_mean, float* d_save_invstd, const void* d_res, int res_ld,
+                               int relu, float drop_p, uint64_t drop_seed, const int64_t* d_drop_step, void* d_out, int out_ld,
+                               uint8_t* d_relu_bits, void* stream) {
   if (debug_skip(ISWM_SKIP_BN)) return 0;
   REQ_C8(C, "bn_train_apply"); REQ_LD8(x_ld, "bn_train_apply"); REQ_LD8(out_ld, "bn_train_apply");
   ISWM_REQUIRE(d_x && d_stats && d_gamma && d_beta && d_out && M > 0, "bn_train_apply: null/empty");
   ISWM_REQUIRE(!d_res || (res_ld % 8) == 0, "bn_train_apply: res_ld");
   ISWM_REQUIRE(C <= 2048, "bn_train_apply: C=%d > 2048 not supported", C);
+  ISWM_REQUIRE(!global || stats_replicas <= 1, "bn_train_apply_global: the global sums are one copy (stats_replicas=%d)", stats_replicas);
   int nx, ny, rpb, blocks;
   // blocks per SM the row range is cut for: 3 = exactly the resident blocks (80 registers x 256 threads), ONE wave.
   // Measured on B200 against 6 (two waves): 33.6 MB tensor 17.1 -> 12.3 us, 67 MB 30.0 -> 24.9 us, cfg2 1074 -> 1088
   // img/s: a second wave is mostly a tail (each thread's life is one or two batches of loads).
   bn_row_grid(C, M, 4, nx, ny, rpb, blocks, 3);
   const bool has_res = d_res != nullptr, has_drop = drop_p > 0.f;
-#define ISWM_BN_APPLY(R, L, D)                                                                                     \
-  launch_k(bn_train_apply_kernel<R, L, D>, dim3(blocks), dim3(kT), 0, ST(stream), BF(d_x), x_ld, d_stats, std::max(1, stats_replicas), M, C,    \
+#define ISWM_BN_APPLY_G(R, L, D, G)                                                                                \
+  launch_k(bn_train_apply_kernel<R, L, D, G>, dim3(blocks), dim3(kT), 0, ST(stream), BF(d_x), x_ld, d_stats, std::max(1, stats_replicas), M, C, \
            d_gamma, d_beta, eps, momentum, d_running_mean, d_running_var, reinterpret_cast<long long*>(d_nbt),      \
            d_save_mean, d_save_invstd, BF(d_res), res_ld, drop_p, DropSeed{drop_seed, reinterpret_cast<const long long*>(d_drop_step)}, BFW(d_out), out_ld, nx, ny, rpb, relu ? d_relu_bits : nullptr)
+#define ISWM_BN_APPLY(R, L, D) do { if (global) ISWM_BN_APPLY_G(R, L, D, true); else ISWM_BN_APPLY_G(R, L, D, false); } while (0)
   if (has_drop) {
     if (has_res) { if (relu) ISWM_BN_APPLY(true, true, true); else ISWM_BN_APPLY(true, false, true); }
     else         { if (relu) ISWM_BN_APPLY(false, true, true); else ISWM_BN_APPLY(false, false, true); }
@@ -1568,7 +1577,26 @@ extern "C" int iswm_bn_train_apply(const void* d_x, int x_ld, const double* d_st
     else         { if (relu) ISWM_BN_APPLY(false, true, false); else ISWM_BN_APPLY(false, false, false); }
   }
 #undef ISWM_BN_APPLY
+#undef ISWM_BN_APPLY_G
   return check_launch("bn_train_apply");
+}
+extern "C" int iswm_bn_train_apply(const void* d_x, int x_ld, const double* d_stats, int stats_replicas, int64_t M, int C,
+                                   const float* d_gamma, const float* d_beta, float eps, float momentum,
+                                   float* d_running_mean, float* d_running_var, int64_t* d_nbt,
+                                   float* d_save_mean, float* d_save_invstd, const void* d_res, int res_ld,
+                                   int relu, float drop_p, uint64_t drop_seed, const int64_t* d_drop_step, void* d_out, int out_ld,
+                                   uint8_t* d_relu_bits, void* stream) {
+  return bn_train_apply_impl(false, d_x, x_ld, d_stats, stats_replicas, M, C, d_gamma, d_beta, eps, momentum, d_running_mean, d_running_var,
+                             d_nbt, d_save_mean, d_save_invstd, d_res, res_ld, relu, drop_p, drop_seed, d_drop_step, d_out, out_ld, d_relu_bits, stream);
+}
+extern "C" int iswm_bn_train_apply_global(const void* d_x, int x_ld, const double* d_gstats, int64_t M, int C,
+                                          const float* d_gamma, const float* d_beta, float eps, float momentum,
+                                          float* d_running_mean, float* d_running_var, int64_t* d_nbt,
+                                          float* d_save_mean, float* d_save_invstd, const void* d_res, int res_ld,
+                                          int relu, float drop_p, uint64_t drop_seed, const int64_t* d_drop_step, void* d_out, int out_ld,
+                                          uint8_t* d_relu_bits, void* stream) {
+  return bn_train_apply_impl(true, d_x, x_ld, d_gstats, 1, M, C, d_gamma, d_beta, eps, momentum, d_running_mean, d_running_var,
+                             d_nbt, d_save_mean, d_save_invstd, d_res, res_ld, relu, drop_p, drop_seed, d_drop_step, d_out, out_ld, d_relu_bits, stream);
 }
 extern "C" int iswm_bn_fold(const float* d_gamma, const float* d_beta, const float* d_mean,
                             const float* d_var, float eps, int C, float* d_scale, float* d_shift,
@@ -1614,12 +1642,12 @@ extern "C" int iswm_bn_bwd_reduce(const void* d_dout, int dout_ld, const void* d
 #undef ISWM_BN_RED
   return check_launch("bn_bwd_reduce");
 }
-extern "C" int iswm_bn_bwd_apply(const void* d_dout, int dout_ld, const void* d_x, int x_ld,
-                                 const void* d_out_act, int act_ld, int64_t M, int C,
-                                 const float* d_gamma, const float* d_beta, const float* d_save_mean,
-                                 const float* d_save_invstd, const double* d_sums, int relu, float drop_p, uint64_t drop_seed, const int64_t* d_drop_step,
-                                 void* d_dx, int dx_ld, void* d_dz, int dz_ld, float* d_dgamma,
-                                 float* d_dbeta, void* stream) {
+static int bn_bwd_apply_impl(const double* d_lsums, const void* d_dout, int dout_ld, const void* d_x, int x_ld,
+                             const void* d_out_act, int act_ld, int64_t M, int C,
+                             const float* d_gamma, const float* d_beta, const float* d_save_mean,
+                             const float* d_save_invstd, const double* d_sums, int relu, float drop_p, uint64_t drop_seed, const int64_t* d_drop_step,
+                             void* d_dx, int dx_ld, void* d_dz, int dz_ld, float* d_dgamma,
+                             float* d_dbeta, void* stream) {
   if (debug_skip(ISWM_SKIP_BN)) return 0;
   REQ_C8(C, "bn_bwd_apply"); REQ_LD8(dout_ld, "bn_bwd_apply"); REQ_LD8(x_ld, "bn_bwd_apply"); REQ_LD8(dx_ld, "bn_bwd_apply");
   ISWM_REQUIRE(d_dout && d_x && d_gamma && d_save_mean && d_save_invstd && d_sums && d_dx && M > 0, "bn_bwd_apply: null/empty");
@@ -1633,17 +1661,38 @@ extern "C" int iswm_bn_bwd_apply(const void* d_dout, int dout_ld, const void* d_
   bn_row_grid(C, M, 4, nx, ny, rpb, blocks, 3);   // one wave, see iswm_bn_train_apply
   const int mask = !relu ? 0 : (relu == 2 ? 3 : (d_out_act ? 1 : 2));
   const bool has_drop = drop_p > 0.f, has_dz = d_dz != nullptr;
-#define ISWM_BN_BAP(MK, D, Z)                                                                                          \
-  launch_k(bn_bwd_apply_kernel<MK, D, Z>, dim3(blocks), dim3(kT), 0, ST(stream), BF(d_dout), dout_ld, BF(d_x), x_ld,    \
+#define ISWM_BN_BAP_G(MK, D, Z, G)                                                                                     \
+  launch_k(bn_bwd_apply_kernel<MK, D, Z, G>, dim3(blocks), dim3(kT), 0, ST(stream), BF(d_dout), dout_ld, BF(d_x), x_ld, \
            BF(d_out_act), act_ld, M, C, d_gamma, d_beta, d_save_mean, d_save_invstd, d_sums, drop_p, DropSeed{drop_seed, reinterpret_cast<const long long*>(d_drop_step)},        \
-           BFW(d_dx), dx_ld, BFW(d_dz), dz_ld, d_dgamma, d_dbeta, nx, ny, rpb)
+           BFW(d_dx), dx_ld, BFW(d_dz), dz_ld, d_dgamma, d_dbeta, nx, ny, rpb, d_lsums)
+#define ISWM_BN_BAP(MK, D, Z) do { if (d_lsums) ISWM_BN_BAP_G(MK, D, Z, true); else ISWM_BN_BAP_G(MK, D, Z, false); } while (0)
 #define ISWM_BN_BAP_M(D, Z) \
   do { if (mask == 0) ISWM_BN_BAP(0, D, Z); else if (mask == 1) ISWM_BN_BAP(1, D, Z); else if (mask == 2) ISWM_BN_BAP(2, D, Z); else ISWM_BN_BAP(3, D, Z); } while (0)
   if (has_drop) { if (has_dz) ISWM_BN_BAP_M(true, true); else ISWM_BN_BAP_M(true, false); }
   else          { if (has_dz) ISWM_BN_BAP_M(false, true); else ISWM_BN_BAP_M(false, false); }
 #undef ISWM_BN_BAP_M
 #undef ISWM_BN_BAP
+#undef ISWM_BN_BAP_G
   return check_launch("bn_bwd_apply");
+}
+extern "C" int iswm_bn_bwd_apply(const void* d_dout, int dout_ld, const void* d_x, int x_ld,
+                                 const void* d_out_act, int act_ld, int64_t M, int C,
+                                 const float* d_gamma, const float* d_beta, const float* d_save_mean,
+                                 const float* d_save_invstd, const double* d_sums, int relu, float drop_p, uint64_t drop_seed, const int64_t* d_drop_step,
+                                 void* d_dx, int dx_ld, void* d_dz, int dz_ld, float* d_dgamma,
+                                 float* d_dbeta, void* stream) {
+  return bn_bwd_apply_impl(nullptr, d_dout, dout_ld, d_x, x_ld, d_out_act, act_ld, M, C, d_gamma, d_beta, d_save_mean, d_save_invstd, d_sums,
+                           relu, drop_p, drop_seed, d_drop_step, d_dx, dx_ld, d_dz, dz_ld, d_dgamma, d_dbeta, stream);
+}
+extern "C" int iswm_bn_bwd_apply_global(const void* d_dout, int dout_ld, const void* d_x, int x_ld,
+                                        const void* d_out_act, int act_ld, int64_t M, int C,
+                                        const float* d_gamma, const float* d_beta, const float* d_save_mean,
+                                        const float* d_save_invstd, const double* d_gsums, const double* d_local_sums, int relu, float drop_p,
+                                        uint64_t drop_seed, const int64_t* d_drop_step, void* d_dx, int dx_ld, void* d_dz, int dz_ld,
+                                        float* d_dgamma, float* d_dbeta, void* stream) {
+  ISWM_REQUIRE(d_local_sums, "bn_bwd_apply_global: null local sums");
+  return bn_bwd_apply_impl(d_local_sums, d_dout, dout_ld, d_x, x_ld, d_out_act, act_ld, M, C, d_gamma, d_beta, d_save_mean, d_save_invstd, d_gsums,
+                           relu, drop_p, drop_seed, d_drop_step, d_dx, dx_ld, d_dz, dz_ld, d_dgamma, d_dbeta, stream);
 }
 
 extern "C" int iswm_stem_im2col(const float* d_img, int B, int Cin, int H, int W, int Ho, int Wo,

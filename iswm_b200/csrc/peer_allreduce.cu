@@ -33,14 +33,9 @@ __device__ __forceinline__ uint32_t ld_acquire_sys(const uint32_t* addr) {
 
 // flags: every rank owns uint32 flags[kMaxPeers] in symmetric memory (slot q = "rank q has reached barrier number v").
 // epoch: this rank's private device counter of barriers executed (all ranks run the same sequence, so the counters agree).
-__global__ void peer_barrier_kernel(PeerPtrs flags, int rank, int world, uint32_t* epoch, int* abort_flag) {
-  pdl_wait();
-  pdl_launch();
+// Thread q < world of the calling block signals rank q and waits for rank q's signal; the caller synchronises the block after.
+__device__ __forceinline__ void barrier_arrive_wait(const PeerPtrs& flags, int rank, int world, uint32_t e, int* abort_flag, int& bad) {
   const int q = threadIdx.x;
-  __shared__ int bad;
-  if (q == 0) bad = 0;
-  __syncthreads();
-  const uint32_t e = *epoch + 1;
   if (q < world) {
     __threadfence_system();                                   // everything this GPU wrote before the barrier is visible system-wide
     st_release_sys(reinterpret_cast<uint32_t*>(flags.p[q]) + rank, e);
@@ -58,6 +53,17 @@ __global__ void peer_barrier_kernel(PeerPtrs flags, int rank, int world, uint32_
       }
     }
   }
+}
+
+__global__ void peer_barrier_kernel(PeerPtrs flags, int rank, int world, uint32_t* epoch, int* abort_flag) {
+  pdl_wait();
+  pdl_launch();
+  const int q = threadIdx.x;
+  __shared__ int bad;
+  if (q == 0) bad = 0;
+  __syncthreads();
+  const uint32_t e = *epoch + 1;
+  barrier_arrive_wait(flags, rank, world, e, abort_flag, bad);
   __syncthreads();
   if (q == 0) *epoch = e;
   (void)bad;
@@ -110,6 +116,77 @@ __global__ void peer_small_sum_kernel(PeerPtrs slots, int world, T* dst, int n, 
   }
 }
 
+// Synchronised BatchNorm statistics. Every rank's engine carves the SAME offsets of a symmetric fp64 arena for the same
+// BatchNorm (sizes depend on channel counts only), so a peer's vector is read in place at arena.p[peer] + src_off - no publish
+// copy. One launch per exchange, one block:
+//   1. this rank's row count goes into the word after the first job's vector (its replica copies), so counts of unequal
+//      shards are exchanged rather than assumed;
+//   2. barrier (signal every rank, bounded wait; skipped when flags.p[0] is null: a one-rank fold);
+//   3. dst[i] = sum over ranks 0..world-1, in that order, of (sum over the vector's replica copies, in order) - the same bits
+//      on every rank - and dst[n] = the global count.
+// A separate kernel rather than peer reads inside every block of the BatchNorm kernels: one block reads world x n values over
+// NVLink, where every apply block doing so would read ~3 x 148 x world x n (about 100 MB per BatchNorm at C = 2048).
+constexpr int kSyncBnMaxJobs = 4;
+constexpr int kSyncBnThreads = 512;
+struct SyncBnJobs {
+  long long src_off[kSyncBnMaxJobs];      // fp64 elements from the arena base
+  double* dst[kSyncBnMaxJobs];            // local: n sums + 1 count
+  int n[kSyncBnMaxJobs];
+  int rep[kSyncBnMaxJobs];
+  int njobs;
+};
+
+__global__ void __launch_bounds__(kSyncBnThreads)
+syncbn_exchange_kernel(PeerPtrs arena, PeerPtrs flags, int rank, int world, uint32_t* epoch, int* abort_flag, SyncBnJobs jobs,
+                       double count) {
+  pdl_wait();
+  pdl_launch();
+  __shared__ int bad;
+  const int t = threadIdx.x;
+  const long long cnt_off = jobs.src_off[0] + (long long)jobs.n[0] * jobs.rep[0];
+  if (t == 0) {
+    bad = 0;
+    reinterpret_cast<double*>(arena.p[rank])[cnt_off] = count;
+    __threadfence_system();
+  }
+  __syncthreads();
+  const bool peers = flags.p[0] != nullptr;
+  uint32_t e = 0;
+  if (peers) {
+    e = *epoch + 1;
+    barrier_arrive_wait(flags, rank, world, e, abort_flag, bad);
+    __syncthreads();
+  }
+  for (int j = 0; j < jobs.njobs; j++) {
+    const int n = jobs.n[j], rep = jobs.rep[j];
+    const long long off = jobs.src_off[j];
+    for (int i = t; i < n; i += kSyncBnThreads) {
+      double v[kMaxPeers];
+#pragma unroll
+      for (int p = 0; p < kMaxPeers; p++) {
+        if (p < world) {
+          const double* src = reinterpret_cast<const double*>(arena.p[p]) + off + i;
+          double a = __ldcv(src);                             // volatile: peers' data, never cached stale
+          for (int r = 1; r < rep; r++) a += __ldcv(src + (long long)r * n);
+          v[p] = a;
+        }
+      }
+      double acc = v[0];
+#pragma unroll
+      for (int p = 1; p < kMaxPeers; p++)
+        if (p < world) acc += v[p];
+      jobs.dst[j][i] = acc;
+    }
+  }
+  if (t == 0) {
+    double acc = __ldcv(reinterpret_cast<const double*>(arena.p[0]) + cnt_off);
+    for (int p = 1; p < world; p++) acc += __ldcv(reinterpret_cast<const double*>(arena.p[p]) + cnt_off);
+    for (int j = 0; j < jobs.njobs; j++) jobs.dst[j][jobs.n[j]] = acc;
+    if (peers) *epoch = e;
+  }
+  (void)bad;
+}
+
 }  // namespace iswm
 
 using namespace iswm;
@@ -124,16 +201,17 @@ static int fill_ptrs(PeerPtrs& pp, const void* const* ptrs, int world, const cha
   return 0;
 }
 
+static int* barrier_abort_flag() {
+  static thread_local int* cached = nullptr;                 // one per device context in practice (one process per GPU)
+  if (!cached && cudaMalloc(&cached, sizeof(int)) == cudaSuccess) cudaMemset(cached, 0, sizeof(int));
+  return cached;
+}
+
 extern "C" int iswm_peer_barrier(const void* const* flag_ptrs, int rank, int world, uint32_t* d_epoch, void* stream) {
   ISWM_REQUIRE(flag_ptrs && d_epoch && rank >= 0 && rank < world, "peer_barrier: bad arguments");
   PeerPtrs pp;
   if (int rc = fill_ptrs(pp, flag_ptrs, world, "peer_barrier")) return rc;
-  int* abort_flag = nullptr;
-  {
-    static thread_local int* cached = nullptr;               // one per device context in practice (one process per GPU)
-    if (!cached && cudaMalloc(&cached, sizeof(int)) == cudaSuccess) cudaMemset(cached, 0, sizeof(int));
-    abort_flag = cached;
-  }
+  int* abort_flag = barrier_abort_flag();
   ISWM_REQUIRE(abort_flag, "peer_barrier: cannot allocate the abort flag");
   launch_k(peer_barrier_kernel, dim3(1), dim3(32), 0, static_cast<cudaStream_t>(stream), pp, rank, world, d_epoch, abort_flag);
   return check_launch("peer_barrier");
@@ -171,4 +249,29 @@ extern "C" int iswm_peer_small_sum(const void* const* slot_ptrs, int world, void
   if (is_f64) launch_k(peer_small_sum_kernel<double>, dim3(1), dim3(64), 0, static_cast<cudaStream_t>(stream), pp, world, static_cast<double*>(d_dst), n, slot_off);
   else launch_k(peer_small_sum_kernel<long long>, dim3(1), dim3(64), 0, static_cast<cudaStream_t>(stream), pp, world, static_cast<long long*>(d_dst), n, slot_off);
   return check_launch("peer_small_sum");
+}
+
+extern "C" int iswm_syncbn_exchange(const iswm_syncbn_job* jobs, int n_jobs, const void* const* arena_ptrs, const void* const* flag_ptrs,
+                                    int rank, int world, double count, uint32_t* d_epoch, void* stream) {
+  ISWM_REQUIRE(jobs && n_jobs >= 1 && n_jobs <= kSyncBnMaxJobs, "syncbn_exchange: 1..%d jobs", kSyncBnMaxJobs);
+  ISWM_REQUIRE(arena_ptrs && rank >= 0 && rank < world && count >= 1.0, "syncbn_exchange: bad arguments");
+  ISWM_REQUIRE(flag_ptrs || world == 1, "syncbn_exchange: %d ranks need the barrier flags", world);
+  ISWM_REQUIRE(!flag_ptrs || d_epoch, "syncbn_exchange: the barrier needs its epoch counter");
+  PeerPtrs arena, flags;
+  if (int rc = fill_ptrs(arena, arena_ptrs, world, "syncbn_exchange")) return rc;
+  for (int i = 0; i < kMaxPeers; i++) flags.p[i] = nullptr;
+  if (flag_ptrs)
+    if (int rc = fill_ptrs(flags, flag_ptrs, world, "syncbn_exchange")) return rc;
+  SyncBnJobs sj{};
+  for (int j = 0; j < n_jobs; j++) {
+    const iswm_syncbn_job& J = jobs[j];
+    ISWM_REQUIRE(J.dst && J.n > 0 && J.src_off >= 0 && J.replicas >= 1, "syncbn_exchange: job %d: bad slot", j);
+    sj.src_off[j] = J.src_off; sj.dst[j] = J.dst; sj.n[j] = J.n; sj.rep[j] = J.replicas;
+  }
+  sj.njobs = n_jobs;
+  int* abort_flag = barrier_abort_flag();
+  ISWM_REQUIRE(abort_flag, "syncbn_exchange: cannot allocate the abort flag");
+  launch_k(syncbn_exchange_kernel, dim3(1), dim3(kSyncBnThreads), 0, static_cast<cudaStream_t>(stream), arena, flags, rank, world, d_epoch,
+           abort_flag, sj, count);
+  return check_launch("syncbn_exchange");
 }

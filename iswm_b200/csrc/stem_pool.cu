@@ -32,6 +32,9 @@ __device__ __forceinline__ float bn_relu_bf16(float x, float sc, float sh) {
   return __bfloat162float(__float2bfloat16_rn(fmaxf(fmaf(x, sc, sh), 0.f)));
 }
 
+// GCNT (synchronised BatchNorm): bn.stats holds the sums over every rank's pixels (one copy) followed by the global pixel
+// count at [2C]; M only describes this rank's tensor
+template <bool GCNT>
 __global__ void __launch_bounds__(kT)
 stem_pool_fwd_kernel(const __nv_bfloat16* __restrict__ raw, StemBn bn, int B, int H, int W, int Ho, int Wo, int64_t M,
                      float eps, float momentum, __nv_bfloat16* __restrict__ out, uint8_t* __restrict__ idx) {
@@ -46,7 +49,8 @@ stem_pool_fwd_kernel(const __nv_bfloat16* __restrict__ raw, StemBn bn, int B, in
   __syncthreads();
   const int cg = threadIdx.x & 7;                       // kT and the grid stride are multiples of 8: a thread keeps its channels
   const int c0 = cg << 3;
-  const double invM = 1.0 / (double)M;
+  const double cnt = GCNT ? bn.stats[2 * kC] : 0.0;
+  const double invM = GCNT ? 1.0 / cnt : 1.0 / (double)M;
   float sc[8], sh[8];
 #pragma unroll
   for (int j = 0; j < 8; j++) {
@@ -61,7 +65,9 @@ stem_pool_fwd_kernel(const __nv_bfloat16* __restrict__ raw, StemBn bn, int B, in
       bn.save_mean[c] = mean;
       bn.save_invstd[c] = invstd;
       if (bn.running_mean) {
-        const float unbiased = (M > 1) ? var * ((float)M / (float)(M - 1)) : var;
+        float unbiased;
+        if (GCNT) unbiased = (cnt > 1.0) ? var * ((float)cnt / (float)(cnt - 1.0)) : var;
+        else unbiased = (M > 1) ? var * ((float)M / (float)(M - 1)) : var;
         bn.running_mean[c] = (1.f - momentum) * bn.running_mean[c] + momentum * mean;
         bn.running_var[c] = (1.f - momentum) * bn.running_var[c] + momentum * unbiased;
       }
@@ -126,15 +132,30 @@ static int stem_grid(int64_t work_items) {
   return (int)std::max<int64_t>(1, std::min<int64_t>(g, (int64_t)num_sms() * 8));
 }
 
-extern "C" int iswm_stem_pool_fwd(const void* d_raw, const iswm_bn_side* bn, int B, int H, int W, int C, int Ho, int Wo,
-                                  float eps, float momentum, void* d_out, uint8_t* d_idx, void* stream) {
+static int stem_pool_fwd_impl(bool global, const void* d_raw, const iswm_bn_side* bn, int B, int H, int W, int C, int Ho, int Wo,
+                              float eps, float momentum, void* d_out, uint8_t* d_idx, void* stream) {
   if (debug_skip(ISWM_SKIP_BN)) return 0;
   ISWM_REQUIRE(d_raw && bn && d_out && d_idx && bn->stats && bn->gamma && bn->beta && bn->save_mean && bn->save_invstd, "stem_pool_fwd: null argument");
   ISWM_REQUIRE(C == kC, "stem_pool_fwd: C=%d (the stem has %d channels)", C, kC);
   ISWM_REQUIRE(Ho == (H - 1) / 2 + 1 && Wo == (W - 1) / 2 + 1 && B >= 1, "stem_pool_fwd: 3x3 / stride 2 / pad 1 geometry expected");
+  ISWM_REQUIRE(!global || bn->stats_replicas <= 1, "stem_pool_fwd_global: the global sums are one copy (stats_replicas=%d)", bn->stats_replicas);
   const StemBn sb{bn->stats, bn->stats_replicas > 1 ? bn->stats_replicas : 1, bn->gamma, bn->beta, bn->running_mean, bn->running_var,
                   reinterpret_cast<long long*>(bn->num_batches_tracked), bn->save_mean, bn->save_invstd};
-  launch_k(stem_pool_fwd_kernel, dim3(stem_grid((int64_t)B * Ho * Wo * 8)), dim3(kT), 0, ST(stream), BF(d_raw), sb, B, H, W, Ho, Wo,
-           (int64_t)B * H * W, eps, momentum, BFW(d_out), d_idx);
+  if (global)
+    launch_k(stem_pool_fwd_kernel<true>, dim3(stem_grid((int64_t)B * Ho * Wo * 8)), dim3(kT), 0, ST(stream), BF(d_raw), sb, B, H, W, Ho, Wo,
+             (int64_t)B * H * W, eps, momentum, BFW(d_out), d_idx);
+  else
+    launch_k(stem_pool_fwd_kernel<false>, dim3(stem_grid((int64_t)B * Ho * Wo * 8)), dim3(kT), 0, ST(stream), BF(d_raw), sb, B, H, W, Ho, Wo,
+             (int64_t)B * H * W, eps, momentum, BFW(d_out), d_idx);
   return check_launch("stem_pool_fwd");
+}
+
+extern "C" int iswm_stem_pool_fwd(const void* d_raw, const iswm_bn_side* bn, int B, int H, int W, int C, int Ho, int Wo,
+                                  float eps, float momentum, void* d_out, uint8_t* d_idx, void* stream) {
+  return stem_pool_fwd_impl(false, d_raw, bn, B, H, W, C, Ho, Wo, eps, momentum, d_out, d_idx, stream);
+}
+
+extern "C" int iswm_stem_pool_fwd_global(const void* d_raw, const iswm_bn_side* bn, int B, int H, int W, int C, int Ho, int Wo,
+                                         float eps, float momentum, void* d_out, uint8_t* d_idx, void* stream) {
+  return stem_pool_fwd_impl(true, d_raw, bn, B, H, W, C, Ho, Wo, eps, momentum, d_out, d_idx, stream);
 }

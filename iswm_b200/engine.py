@@ -159,6 +159,12 @@ class Engine:
         self.profile = None           # list of (kernel, algorithmic_flops, start_event, end_event) when profiling
         self.debug_taps = None        # dict name -> NCHW fp32 copy of each unit's output (tools/layer_diff.py)
         self.debug_units = None       # list of per-unit records of the engine's own tensors (tests/test_unit_replay_gpu.py)
+        # synchronised BatchNorm (set by iswm_b200.parallel.DataParallel(sync_bn=True)): bn_sync(srcs, dsts, n, rows, stream) turns
+        # this rank's fp64 statistics slots `srcs` [(slot, replicas)] of n = 2C values into the sums over every rank plus the
+        # global row count, dsts[i][:n + 1]; called between each train-mode BatchNorm's producer and its consumer, on the stream
+        # the unit runs on. None: every rank normalises with its own shard's statistics (nn.DataParallel)
+        self.bn_sync: Optional[Callable] = None
+        self.ext_scratch64 = None     # set with bn_sync on the peer transport: a symmetric allocation to carve the fp64 slots from
 
     # ------------------------------------------------------------------ graph description
     def _build_specs(self):
@@ -533,8 +539,11 @@ class Engine:
         Cout = s.cout
         raw = torch.empty((B, Ho, Wo, Cout), dtype=torch.bfloat16, device=self.device)
         rep = self._stats_rep(Cout)
-        stats = self._stats_slot(2 * Cout * rep)
+        sync = self.bn_sync is not None
+        stats = self._stats_slot(2 * Cout * rep + (1 if sync else 0))     # synchronised: + this rank's row count
         self._conv(s, xin, raw, Cout, Ho, Wo, taps, n_img, _lib.EPI_STATS, stats=stats)
+        if sync:
+            stats, rep = self._bn_exchange([(stats, rep)], 2 * Cout, M)[0], 1
         if out is None:
             out = Act.new(B, Ho, Wo, Cout, self.device)
         save = self._save_slot(2 * Cout)
@@ -547,12 +556,14 @@ class Engine:
         # instead of the block output
         bits = torch.empty((M, Cout // 8), dtype=torch.uint8, device=self.device) if (relu and residual is not None) else None
         ev = self._prof_begin()
-        check(L.iswm_bn_train_apply(raw.data_ptr(), Cout, stats.data_ptr(), rep, M, Cout, bn.weight.data_ptr(), bn.bias.data_ptr(),
-                                    BN_EPS, BN_MOMENTUM, bn.running_mean.data_ptr(), bn.running_var.data_ptr(),
-                                    bn.num_batches_tracked.data_ptr(), save.data_ptr(), save[Cout:].data_ptr(),
-                                    None if residual is None else residual.ptr, 0 if residual is None else residual.ld,
-                                    1 if relu else 0, drop_p, seed, step_ptr, out.ptr, out.ld,
-                                    None if bits is None else bits.data_ptr(), _st()), "bn_train_apply " + s.name)
+        apply_args = (bn.weight.data_ptr(), bn.bias.data_ptr(), BN_EPS, BN_MOMENTUM, bn.running_mean.data_ptr(), bn.running_var.data_ptr(),
+                      bn.num_batches_tracked.data_ptr(), save.data_ptr(), save[Cout:].data_ptr(),
+                      None if residual is None else residual.ptr, 0 if residual is None else residual.ld,
+                      1 if relu else 0, drop_p, seed, step_ptr, out.ptr, out.ld, None if bits is None else bits.data_ptr(), _st())
+        if sync:
+            check(L.iswm_bn_train_apply_global(raw.data_ptr(), Cout, stats.data_ptr(), M, Cout, *apply_args), "bn_train_apply_global " + s.name)
+        else:
+            check(L.iswm_bn_train_apply(raw.data_ptr(), Cout, stats.data_ptr(), rep, M, Cout, *apply_args), "bn_train_apply " + s.name)
         # HBM-bound kernels are recorded with their algorithmic BYTES in the flops slot (kernel name prefixed "hbm:")
         self._prof_end(ev, "hbm:bn_train_apply", 2.0 * M * Cout * (3 if residual is not None else 2) + (M * Cout / 8 if bits is not None else 0), "bn_apply " + s.name)
         self._tap(s.name, out)
@@ -609,11 +620,15 @@ class Engine:
                                        relu_mode, drop_p, seed, step_ptr, sums.data_ptr(), _st()), "bn_bwd_reduce " + s.name)
             self._prof_end(ev, "hbm:bn_bwd_reduce", 2.0 * M * Cout * (2 + nmask), "bn_bwd_reduce " + s.name)
             ev = self._prof_begin()
-            check(L.iswm_bn_bwd_apply(dout.ptr, dout.ld, raw.data_ptr(), Cout, act_ptr, out.ld, M, Cout,
-                                      bn.weight.data_ptr(), bn.bias.data_ptr(), save.data_ptr(), save[Cout:].data_ptr(), sums.data_ptr(),
-                                      relu_mode, drop_p, seed, step_ptr, dy.data_ptr(), dy_ld, dz_ptr, dz_ld,
-                                      self.grad_views[id(bn.weight)].data_ptr(), self.grad_views[id(bn.bias)].data_ptr(), _st()),
-                  "bn_bwd_apply " + s.name)
+            head = (dout.ptr, dout.ld, raw.data_ptr(), Cout, act_ptr, out.ld, M, Cout,
+                    bn.weight.data_ptr(), bn.bias.data_ptr(), save.data_ptr(), save[Cout:].data_ptr())
+            tail = (relu_mode, drop_p, seed, step_ptr, dy.data_ptr(), dy_ld, dz_ptr, dz_ld,
+                    self.grad_views[id(bn.weight)].data_ptr(), self.grad_views[id(bn.bias)].data_ptr(), _st())
+            if sync:
+                gsums = self._bn_exchange([(sums, 1)], 2 * Cout, M)[0]
+                check(L.iswm_bn_bwd_apply_global(*head, gsums.data_ptr(), sums.data_ptr(), *tail), "bn_bwd_apply_global " + s.name)
+            else:
+                check(L.iswm_bn_bwd_apply(*head, sums.data_ptr(), *tail), "bn_bwd_apply " + s.name)
             self._prof_end(ev, "hbm:bn_bwd_apply", 2.0 * M * Cout * (3 + nmask + (1 if dz_ptr is not None else 0)), "bn_bwd_apply " + s.name)
             if dz_tmp is not None:
                 check(L.iswm_add_bf16(residual.grad.ptr, dz_tmp.data_ptr(), dz_tmp.numel(), residual.grad.ptr, _st()), "add_bf16")
@@ -633,15 +648,22 @@ class Engine:
         self._pack(s, True)
         xin, taps, n_img, Ho, Wo = self._prep_input(s, x)
         raw = torch.empty((x.B, Ho, Wo, s.cout), dtype=torch.bfloat16, device=self.device)
-        stats = self._stats_slot(2 * s.cout * self._stats_rep(s.cout))
+        stats = self._stats_slot(2 * s.cout * self._stats_rep(s.cout) + (1 if self.bn_sync is not None else 0))
         self._conv(s, xin, raw, s.cout, Ho, Wo, taps, n_img, _lib.EPI_STATS, stats=stats)
         return raw, stats, xin, taps, n_img, Ho, Wo
 
-    def _bn_side(self, bn, stats, save, Cc, train_fwd: bool):
+    def _bn_side(self, bn, stats, save, Cc, train_fwd: bool, rep=None):
         return _lib.BnSide(stats.data_ptr() if stats is not None else None, bn.weight.data_ptr(), bn.bias.data_ptr(),
                            bn.running_mean.data_ptr() if train_fwd else None, bn.running_var.data_ptr() if train_fwd else None,
                            bn.num_batches_tracked.data_ptr() if train_fwd else None, save.data_ptr(), save[Cc:].data_ptr(),
-                           1 if stats is None else stats.numel() // (2 * Cc))
+                           rep if rep is not None else (1 if stats is None else stats.numel() // (2 * Cc)))
+
+    def _bn_exchange(self, srcs, n: int, rows: int):
+        """Synchronised BatchNorm: fp64 slots holding the sums over every rank of the vectors `srcs` [(slot, replicas)] of n
+        values, followed by the global row count (this rank contributes `rows`), from the same slots of every rank's arena."""
+        dsts = [self._stats_slot(n + 1) for _ in srcs]
+        self.bn_sync(srcs, dsts, n, rows, _st())
+        return dsts
 
     def _unit_train_dual(self, s: ConvSpec, x: Act, sds: ConvSpec, dsc) -> Act:
         """Closing unit of a bottleneck block with a downsample branch (resnet.py:110-118): out = relu(bn3(conv3(x)) +
@@ -656,10 +678,17 @@ class Engine:
         out = Act.new(B, Ho, Wo, Cout, self.device)
         save, save_ds = self._save_slot(2 * Cout), self._save_slot(2 * Cout)
         bits = torch.empty((M, Cout // 8), dtype=torch.uint8, device=self.device)
-        a_side, d_side = self._bn_side(s.bn, stats, save, Cout, True), self._bn_side(sds.bn, stats_ds, save_ds, Cout, True)
+        sync = self.bn_sync is not None
+        if sync:
+            # both BatchNorms' statistics are ready here: ONE exchange carries the two vectors
+            rep = self._stats_rep(Cout)
+            stats, stats_ds = self._bn_exchange([(stats, rep), (stats_ds, rep)], 2 * Cout, M)
+        a_side = self._bn_side(s.bn, stats, save, Cout, True, 1 if sync else None)
+        d_side = self._bn_side(sds.bn, stats_ds, save_ds, Cout, True, 1 if sync else None)
         ev = self._prof_begin()
-        check(L.iswm_bn_dual_train_apply(raw.data_ptr(), Cout, C.byref(a_side), raw_ds.data_ptr(), Cout, C.byref(d_side), M, Cout,
-                                         BN_EPS, BN_MOMENTUM, out.ptr, out.ld, bits.data_ptr(), _st()), "bn_dual_train_apply " + s.name)
+        fwd = L.iswm_bn_dual_train_apply_global if sync else L.iswm_bn_dual_train_apply
+        check(fwd(raw.data_ptr(), Cout, C.byref(a_side), raw_ds.data_ptr(), Cout, C.byref(d_side), M, Cout,
+                  BN_EPS, BN_MOMENTUM, out.ptr, out.ld, bits.data_ptr(), _st()), "bn_dual_train_apply " + s.name)
         self._prof_end(ev, "hbm:bn_train_apply", 2.0 * M * Cout * 3 + M * Cout / 8, "bn_apply " + s.name + "+ds")
 
         def backward():
@@ -675,11 +704,16 @@ class Engine:
             self._prof_end(ev, "hbm:bn_bwd_reduce", 2.0 * M * Cout * 3 + M * Cout / 8, "bn_bwd_reduce " + s.name + "+ds")
             gv = self.grad_views
             ev = self._prof_begin()
-            check(L.iswm_bn_dual_bwd_apply(dout.ptr, Cout, bits.data_ptr(), raw.data_ptr(), Cout, C.byref(a_b), sums.data_ptr(),
-                                           raw_ds.data_ptr(), Cout, C.byref(d_b), sums_ds.data_ptr(), M, Cout,
-                                           dy.data_ptr(), Cout, dy_ds.data_ptr(), Cout,
-                                           gv[id(s.bn.weight)].data_ptr(), gv[id(s.bn.bias)].data_ptr(),
-                                           gv[id(sds.bn.weight)].data_ptr(), gv[id(sds.bn.bias)].data_ptr(), _st()), "bn_dual_bwd_apply " + s.name)
+            tail = (M, Cout, dy.data_ptr(), Cout, dy_ds.data_ptr(), Cout, gv[id(s.bn.weight)].data_ptr(), gv[id(s.bn.bias)].data_ptr(),
+                    gv[id(sds.bn.weight)].data_ptr(), gv[id(sds.bn.bias)].data_ptr(), _st())
+            if sync:
+                g, g_ds = self._bn_exchange([(sums, 1), (sums_ds, 1)], 2 * Cout, M)
+                check(L.iswm_bn_dual_bwd_apply_global(dout.ptr, Cout, bits.data_ptr(), raw.data_ptr(), Cout, C.byref(a_b), g.data_ptr(), sums.data_ptr(),
+                                                      raw_ds.data_ptr(), Cout, C.byref(d_b), g_ds.data_ptr(), sums_ds.data_ptr(), *tail),
+                      "bn_dual_bwd_apply_global " + s.name)
+            else:
+                check(L.iswm_bn_dual_bwd_apply(dout.ptr, Cout, bits.data_ptr(), raw.data_ptr(), Cout, C.byref(a_b), sums.data_ptr(),
+                                               raw_ds.data_ptr(), Cout, C.byref(d_b), sums_ds.data_ptr(), *tail), "bn_dual_bwd_apply " + s.name)
             self._prof_end(ev, "hbm:bn_bwd_apply", 2.0 * M * Cout * 5 + M * Cout / 8, "bn_bwd_apply " + s.name + "+ds")
             out.grad = None
             self._conv_backward(s, x, xin, taps, n_img, Ho, Wo, dy, True)
@@ -933,12 +967,24 @@ class Engine:
 
     # per-step scratch carved from two zeroed buffers: fp64 accumulators (conv-epilogue statistics, BN-backward sums)
     # and fp32 saved mean / invstd
-    def _begin_scratch(self):
+    def scratch_need(self, sync: bool) -> int:
+        """fp64 elements of the per-step scratch arena; depends on the model's channel counts only (not on the batch)."""
         need = 0
         for s in self.specs:
             if s.bn is not None:
                 need += 2 * s.cout * (self._stats_rep(s.cout) + 1) + 192    # fwd stats (x copies) + bwd sums and barrier counter (fp64); covers mean/invstd (fp32) too
-        need += 4096
+                if sync:
+                    need += 4 * s.cout + 192                                  # + row counts, global forward and backward sums (+ counts)
+        return need + 4096
+
+    def _begin_scratch(self):
+        need = self.scratch_need(self.bn_sync is not None)
+        ext = self.ext_scratch64
+        if ext is not None and (getattr(self, "_scratch64", None) is None or self._scratch64.data_ptr() != ext.data_ptr()):
+            if ext.numel() < need or ext.device != self.device or ext.dtype != torch.float64:
+                raise RuntimeError("external statistics arena does not fit the model")
+            self._scratch64 = ext
+            self._scratch32 = torch.empty(need, dtype=torch.float32, device=self.device)
         if getattr(self, "_scratch64", None) is None or self._scratch64.numel() < need or self._scratch64.device != self.device:
             self._scratch64 = torch.empty(need, dtype=torch.float64, device=self.device)
             self._scratch32 = torch.empty(need, dtype=torch.float32, device=self.device)
@@ -1176,8 +1222,11 @@ class Engine:
             return out
         raw = torch.empty((M, 64), dtype=torch.bfloat16, device=dev)
         rep = self._stats_rep(64)
-        stats = self._stats_slot(128 * rep)
+        sync = self.bn_sync is not None
+        stats = self._stats_slot(128 * rep + (1 if sync else 0))
         self._conv(s, colA, raw, 64, Ho_, Wo_, taps, n_img, _lib.EPI_STATS, stats=stats, cin=colA.C, **geo)
+        if sync:
+            stats, rep = self._bn_exchange([(stats, rep)], 128, M)[0], 1
         save = self._save_slot(128)
         bn = s.bn
         fused_tail = self.stem_pool and self.debug_units is None and self.debug_taps is None
@@ -1185,9 +1234,10 @@ class Engine:
             H2, W2 = (H1 + 1) // 2, (W1 + 1) // 2
             pooled = Act.new(B, H2, W2, 64, dev)
             idx = torch.empty((B, H2, W2, 64), dtype=torch.uint8, device=dev)
-            side = self._bn_side(bn, stats, save, 64, True)
+            side = self._bn_side(bn, stats, save, 64, True, rep)
             ev = self._prof_begin()
-            check(L.iswm_stem_pool_fwd(raw.data_ptr(), C.byref(side), B, H1, W1, 64, H2, W2, BN_EPS, BN_MOMENTUM, pooled.ptr, idx.data_ptr(), _st()), "stem_pool_fwd")
+            fwd = L.iswm_stem_pool_fwd_global if sync else L.iswm_stem_pool_fwd
+            check(fwd(raw.data_ptr(), C.byref(side), B, H1, W1, 64, H2, W2, BN_EPS, BN_MOMENTUM, pooled.ptr, idx.data_ptr(), _st()), "stem_pool_fwd")
             self._prof_end(ev, "hbm:stem_pool_fwd", 2.0 * M * 64 + 3.0 * B * H2 * W2 * 64, "stem_pool_fwd")
 
             def backward_fused():
@@ -1199,17 +1249,18 @@ class Engine:
                 check(L.iswm_maxpool_bwd(g.ptr, idx.data_ptr(), B, H1, W1, 64, H2, W2, dact.data_ptr(), _st()), "maxpool_bwd")
                 check(L.iswm_bn_bwd_reduce(dact.data_ptr(), 64, raw.data_ptr(), 64, None, 64, M, 64, save.data_ptr(), save[64:].data_ptr(),
                                            bn.weight.data_ptr(), bn.bias.data_ptr(), 1, 0.0, 0, None, sums.data_ptr(), _st()), "bn_bwd_reduce stem")
-                check(L.iswm_bn_bwd_apply(dact.data_ptr(), 64, raw.data_ptr(), 64, None, 64, M, 64, bn.weight.data_ptr(), bn.bias.data_ptr(), save.data_ptr(),
-                                          save[64:].data_ptr(), sums.data_ptr(), 1, 0.0, 0, None, dy.data_ptr(), 64, None, 0,
-                                          self.grad_views[id(bn.weight)].data_ptr(), self.grad_views[id(bn.bias)].data_ptr(), _st()), "bn_bwd_apply stem")
+                self._stem_bwd_apply(bn, dact.data_ptr(), 64, raw, save, sums, dy, M)
                 pooled.grad = None
                 self._stem_wgrad(s, bn, colA, dy, B, H1, W1, M, taps, row_taps, n_img)
 
             self.tape.append(backward_fused)
             return (pooled,)
-        check(L.iswm_bn_train_apply(raw.data_ptr(), 64, stats.data_ptr(), rep, M, 64, bn.weight.data_ptr(), bn.bias.data_ptr(), BN_EPS,
-                                    BN_MOMENTUM, bn.running_mean.data_ptr(), bn.running_var.data_ptr(), bn.num_batches_tracked.data_ptr(),
-                                    save.data_ptr(), save[64:].data_ptr(), None, 0, 1, 0.0, 0, None, out.ptr, 64, None, _st()), "bn_train_apply stem")
+        apply_args = (bn.weight.data_ptr(), bn.bias.data_ptr(), BN_EPS, BN_MOMENTUM, bn.running_mean.data_ptr(), bn.running_var.data_ptr(),
+                      bn.num_batches_tracked.data_ptr(), save.data_ptr(), save[64:].data_ptr(), None, 0, 1, 0.0, 0, None, out.ptr, 64, None, _st())
+        if sync:
+            check(L.iswm_bn_train_apply_global(raw.data_ptr(), 64, stats.data_ptr(), M, 64, *apply_args), "bn_train_apply_global stem")
+        else:
+            check(L.iswm_bn_train_apply(raw.data_ptr(), 64, stats.data_ptr(), rep, M, 64, *apply_args), "bn_train_apply stem")
         self._tap(s.name, out)
 
         def backward():
@@ -1218,9 +1269,7 @@ class Engine:
             dy = torch.empty((M, 64), dtype=torch.bfloat16, device=dev)
             check(L.iswm_bn_bwd_reduce(dout.ptr, dout.ld, raw.data_ptr(), 64, None, 64, M, 64, save.data_ptr(), save[64:].data_ptr(),
                                        bn.weight.data_ptr(), bn.bias.data_ptr(), 1, 0.0, 0, None, sums.data_ptr(), _st()), "bn_bwd_reduce stem")
-            check(L.iswm_bn_bwd_apply(dout.ptr, dout.ld, raw.data_ptr(), 64, None, 64, M, 64, bn.weight.data_ptr(), bn.bias.data_ptr(), save.data_ptr(),
-                                      save[64:].data_ptr(), sums.data_ptr(), 1, 0.0, 0, None, dy.data_ptr(), 64, None, 0,
-                                      self.grad_views[id(bn.weight)].data_ptr(), self.grad_views[id(bn.bias)].data_ptr(), _st()), "bn_bwd_apply stem")
+            self._stem_bwd_apply(bn, dout.ptr, dout.ld, raw, save, sums, dy, M)
             out.grad = None
             gview = self.grad_views[id(s.conv.weight)]
             self._stem_wgrad(s, bn, colA, dy, B, H1, W1, M, taps, row_taps, n_img)
@@ -1234,6 +1283,17 @@ class Engine:
 
         self.tape.append(backward)
         return out
+
+    def _stem_bwd_apply(self, bn, dout_ptr, dout_ld, raw, save, sums, dy, M):
+        """The stem BatchNorm's backward pass 2 (after iswm_bn_bwd_reduce into `sums`), synchronised or not."""
+        L = _lib.lib()
+        head = (dout_ptr, dout_ld, raw.data_ptr(), 64, None, 64, M, 64, bn.weight.data_ptr(), bn.bias.data_ptr(), save.data_ptr(), save[64:].data_ptr())
+        tail = (1, 0.0, 0, None, dy.data_ptr(), 64, None, 0, self.grad_views[id(bn.weight)].data_ptr(), self.grad_views[id(bn.bias)].data_ptr(), _st())
+        if self.bn_sync is not None:
+            gsums = self._bn_exchange([(sums, 1)], 128, M)[0]
+            check(L.iswm_bn_bwd_apply_global(*head, gsums.data_ptr(), sums.data_ptr(), *tail), "bn_bwd_apply_global stem")
+        else:
+            check(L.iswm_bn_bwd_apply(*head, sums.data_ptr(), *tail), "bn_bwd_apply stem")
 
     def _stem_wgrad(self, s, bn, colA: Act, dy: torch.Tensor, B, H1, W1, M, taps, row_taps, n_img):
         """Weight gradient of the stem convolution from dy (gradient of its pre-BN output) on the weight-gradient stream."""

@@ -1,7 +1,8 @@
 """Data parallelism for the hot path: one process per GPU, NCCL over NVLink 5 / NVSwitch.
 
 The reference is single-process nn.DataParallel (train.py:970): parameters replicated, the batch
-scattered along dim 0, PER-REPLICA BatchNorm statistics, logits gathered to GPU 0 where the criterion
+scattered along dim 0, PER-REPLICA BatchNorm statistics (the default here too; `sync_bn=True` for statistics over the global
+batch, below), logits gathered to GPU 0 where the criterion
 normalises over the WHOLE batch (train.py:1045-1046), gradients reduce-added to GPU 0. The same
 semantics here, without the GPU-0 bottleneck:
   * each rank runs forward/backward on its shard with its own BN statistics;
@@ -17,6 +18,18 @@ step - histogram, gradient buckets, loss - is a plain kernel over NVLink peer me
 on a communication stream ordered by events, with sums that are bit-identical on every rank. No host synchronisation and no
 library call, so the data-parallel step is captured in ONE CUDA graph (GraphedTrainStep(dp=...)). "nccl": torch.distributed
 collectives (async_op on the bucket all-reduces); also what the gloo CPU tests drive.
+
+Synchronised BatchNorm (`sync_bn=True`, torch.nn.SyncBatchNorm semantics; convert_sync_batchnorm does not apply to this model,
+whose BatchNorms are parameter holders the engine runs itself): every train-mode BatchNorm normalises with the mean and biased
+variance over ALL ranks' rows, the running variance uses the unbiased factor of the global row count, and the input gradient
+uses the globally reduced sum(dz), sum(dz.xhat) and count. The gamma / beta gradients each rank writes are its OWN
+contributions, which the gradient all-reduce (SUM) completes. Each BatchNorm's per-channel fp64 sums (convolution epilogue
+forward, iswm_bn_bwd_reduce backward) and its row count are exchanged between producer and consumer (Engine.bn_sync):
+  * peer: the engine's fp64 scratch arena is a symmetric allocation carved at the same offsets on every rank, and one
+    iswm_syncbn_exchange launch per exchange reads the peers' slots in place after a barrier, summing in rank order (same bits
+    on every rank); capturable, so GraphedTrainStep(dp=...) still replays ONE graph per step;
+  * nccl: the same kernel folds this rank's copies and count into a slot that dist.all_reduce (SUM) completes, eagerly.
+Counts are exchanged, not assumed: shards of different sizes are normalised over the true global batch.
 """
 from __future__ import annotations
 
@@ -100,7 +113,8 @@ class GradBucketer:
 class DataParallel:
     """Wraps an iswm_b200 DeepLabV3 model + criterion for multi-rank training (see module docstring)."""
 
-    def __init__(self, model, criterion, bucket_bytes: int = 25 << 20, group=None, metrics=None, comm: str = "auto"):
+    def __init__(self, model, criterion, bucket_bytes: int = 25 << 20, group=None, metrics=None, comm: str = "auto",
+                 sync_bn: bool = False):
         if not dist.is_initialized():
             raise RuntimeError("torch.distributed must be initialised (backend 'nccl', one process per GPU)")
         self.model, self.criterion, self.group = model, criterion, group
@@ -132,6 +146,9 @@ class DataParallel:
         with torch.no_grad():
             for t in list(model.parameters()) + list(model.buffers()):
                 dist.broadcast(t.data, 0, group=group)
+        self.sync_bn = bool(sync_bn)
+        if self.sync_bn:
+            self._setup_sync_bn(p0.device)
         criterion.hist_hook = self._allreduce_hist_peer if self.comm_mode == "peer" else self._allreduce_hist
         self.engine.grad_ready_hook = self._grad_ready
         self._index = {id(p): i for i, p in enumerate(model.parameters())}
@@ -160,6 +177,64 @@ class DataParallel:
         # a bucket's kernel only runs in the gaps the (register-file-filling) convolution CTAs leave: a modest grid is enough
         self._ar_blocks = int(os.environ.get("ISWM_DP_AR_BLOCKS", "64"))
         self.comm_mode = "peer"
+
+    # ---- synchronised BatchNorm ------------------------------------------------------------------------------------
+    def _setup_sync_bn(self, device):
+        eng = self.engine
+        if self.comm_mode == "peer":
+            # size depends on the model's channel counts only: every rank allocates (collectively) the same arena, and the
+            # engine carves it in the same order, so a BatchNorm's slot sits at the same offset on every rank
+            arena, ptrs = self.peer.alloc(eng.scratch_need(True), torch.float64)
+            arena.zero_()
+            self._arena = arena
+            self._arena_ptrs = self.peer._ptr_array(ptrs)
+            eng.ext_scratch64 = arena
+            eng.bn_sync = self._bn_exchange_peer
+        else:
+            eng.bn_sync = self._bn_exchange_nccl
+
+    def _bn_jobs(self, srcs, dsts, n: int, base: int, size: int):
+        from . import _lib
+        jobs = (_lib.SyncBnJob * len(srcs))()
+        for j, ((src, rep), dst) in enumerate(zip(srcs, dsts)):
+            off = src.data_ptr() - base
+            if off < 0 or off + 8 * (n * rep + 1) > 8 * size:
+                raise RuntimeError("synchronised BatchNorm: a statistics slot lies outside the engine's arena")
+            jobs[j].src_off, jobs[j].dst, jobs[j].n, jobs[j].replicas = off // 8, dst.data_ptr(), n, rep
+        return jobs
+
+    def _bn_exchange_peer(self, srcs, dsts, n: int, rows: int, stream: int):
+        # Barrier ordering: exchanges on the main stream share channel 0 with the histogram and loss reductions (all issued in
+        # program order on one stream, the same on every rank). The low-level projection and the pooled ASPP branch run on the
+        # engine's side stream during the forward (Engine._fwd_fork), where they interleave with the main stream's exchanges in
+        # an order that differs from rank to rank: they use their own channel 2, whose barriers are in program order on that stream.
+        # Arena reuse: a peer reads this rank's step-i slots only inside step i's exchanges. This rank zeroes its arena for step
+        # i+1 (Engine._begin_scratch) after the loss reduction of step i (train_step: channel-0 barrier after the backward),
+        # which no peer passes before its stream has finished every exchange of step i - the backward's last (the stem's) on
+        # the main stream, the side-stream ones before the forward's join - so no peer can still be reading.
+        ws = self.engine._wstream
+        channel = 2 if (ws is not None and stream == ws.cuda_stream) else 0
+        jobs = self._bn_jobs(srcs, dsts, n, self._arena.data_ptr(), self._arena.numel())
+        self.peer.bn_exchange(self._arena_ptrs, jobs, len(srcs), rows, channel, stream)
+
+    def _bn_exchange_nccl(self, srcs, dsts, n: int, rows: int, stream: int):
+        from . import _lib
+        from ._lib import check
+        import ctypes as C
+        arena = self.engine._scratch64
+        jobs = self._bn_jobs(srcs, dsts, n, arena.data_ptr(), arena.numel())
+        local = (C.c_void_p * 1)(arena.data_ptr())
+        check(_lib.lib().iswm_syncbn_exchange(jobs, len(srcs), local, None, 0, 1, float(rows), None, stream), "syncbn_exchange (fold)")
+        cur = torch.cuda.current_stream()
+        ctx = torch.cuda.stream(torch.cuda.ExternalStream(stream)) if cur.cuda_stream != stream else None
+        if ctx is not None:
+            ctx.__enter__()
+        try:
+            for d in dsts:
+                dist.all_reduce(d, op=dist.ReduceOp.SUM, group=self.group)
+        finally:
+            if ctx is not None:
+                ctx.__exit__(None, None, None)
 
     def _launch_peer(self, s: int, e: int):
         cur = torch.cuda.current_stream()                  # the stream that produced the bucket (weight-gradient stream)

@@ -5,9 +5,11 @@ every GPU, every rank's copy mapped into every other rank's address space); the 
 write the peers' copies directly. Nothing here synchronises with the host and nothing calls into a communication library
 after set-up, so the whole data-parallel step - gradient all-reduce included - is captured in ONE CUDA graph.
 
-Two independent barrier CHANNELS (own flags, own epoch counter): 0 for the main stream's small reductions (class histogram
-before the loss kernel, loss numerators after it), 1 for the gradient buckets on the communication stream. Barriers of one
-channel are issued in the same order on every rank; barriers of different channels may interleave differently per rank.
+Three independent barrier CHANNELS (own flags, own epoch counter): 0 for the main stream's exchanges (class histogram before
+the loss kernel, loss numerators after it, and with synchronised BatchNorm the statistics of every BatchNorm the main stream
+runs), 1 for the gradient buckets on the communication stream, 2 for the synchronised-BatchNorm statistics of the forward
+branches the engine runs on its side stream (low-level projection, pooled ASPP branch). Barriers of one channel are issued in
+the same order on every rank; barriers of different channels may interleave differently per rank.
 """
 from __future__ import annotations
 
@@ -20,7 +22,7 @@ from . import _lib
 from ._lib import check
 
 _FLAGS_BYTES = 64            # per channel: 8 x uint32 (+ padding)
-_N_CHANNELS = 2
+_N_CHANNELS = 3
 _SLOT_REGION = 64            # 8-byte slots per region
 _N_REGIONS = 4
 _CTL_BYTES = _N_CHANNELS * _FLAGS_BYTES + _N_REGIONS * _SLOT_REGION * 8
@@ -71,6 +73,12 @@ class PeerComm:
         self.barrier(channel, stream)
         check(L.iswm_peer_allreduce_f32(ptr_array, self.rank, self.world, offset, n, max_blocks, stream), "peer_allreduce_f32")
         self.barrier(channel, stream)
+
+    def bn_exchange(self, arena_ptrs, jobs, n_jobs: int, rows: int, channel: int, stream: int):
+        """Synchronised BatchNorm statistics (iswm_syncbn_exchange): `jobs` (ctypes iswm_syncbn_job array) name slots of the
+        symmetric arena whose peer mappings are `arena_ptrs`; this rank contributes `rows` rows to the global count."""
+        check(_lib.lib().iswm_syncbn_exchange(jobs, n_jobs, arena_ptrs, self._flag_ptrs[channel], self.rank, self.world, float(rows),
+                                              self.epochs[channel:].data_ptr(), stream), "syncbn_exchange")
 
     def small_allreduce_(self, t: torch.Tensor, region: int, stream: int, channel: int = 0) -> torch.Tensor:
         """In-place SUM over ranks of a small int64 / float64 device vector (<= 64 values); `region` names the call site."""
