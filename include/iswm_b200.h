@@ -114,6 +114,35 @@ int iswm_predict_epilogue(const float* d_lo, int B, int Hi, int Wi, int C, int H
                           float threshold, const void* d_true, int true_dtype, uint8_t* d_pred_out,
                           uint8_t* d_conf_out, int64_t* d_cm, void* stream);
 
+/* ---- test-time augmentation (multi-scale + horizontal flip) for the predict step --------------------- */
+/* Bilinear resize (align_corners=False, no antialias) of fp32 NCHW [B,C,Hi,Wi] to [B,C,Ho,Wo], then an optional
+ * horizontal mirror: F.interpolate(x, size=(Ho,Wo), mode="bilinear") followed by .flip(-1), with the four taps mixed in
+ * torch's association. With (Ho,Wo) == (Hi,Wi) it is an exact copy (mirrored when flip). d_out may be a batch slice of a
+ * larger buffer. */
+int iswm_resize_flip_f32(const float* d_x, int B, int C, int Hi, int Wi, int Ho, int Wo, int flip, float* d_out,
+                         void* stream);
+
+/* One view of iswm_predict_tta_epilogue: the low-resolution logits of the network run on the view's input. */
+typedef struct {
+  const float* lo; /* device, float32 NHWC [B,Hi,Wi,2] (forward_lowres output, or a batch slice of it) */
+  int Hi, Wi;      /* low-resolution size */
+  int Hv, Wv;      /* the view's full-resolution size (the size of the input the network ran on) */
+  int flip;        /* 1: the view's input was mirrored horizontally */
+} IswmTtaView;
+#define ISWM_TTA_MAX_VIEWS 8
+
+/* Multi-view predict epilogue: for every output pixel and view v, logits bilinear (Hi,Wi) -> (Hv,Wv) -> (Ho,Wo)
+ * (the second resize skipped when (Hv,Wv) == (Ho,Wo)), un-mirrored when flip, then the 2-class softmax; the
+ * probabilities are summed in view order and divided by n_views. mode 1: pred = p1 > threshold; mode 0: pred = p1 > p0
+ * (a tie goes to the sign of the summed logit margin, which makes one view equal the logit argmax).
+ * d_conf_out = uint8(p1*255) in mode 1, zeros in mode 0. d_true / d_cm / d_pred_out / d_conf_out as in
+ * iswm_predict_epilogue. h_views is a HOST array of n_views (1..ISWM_TTA_MAX_VIEWS) records passed to the kernel by
+ * value (graph-capturable). C == 2 only; any Wo >= 1. A single unflipped view with (Hv,Wv) == (Ho,Wo) is
+ * bit-identical to iswm_predict_epilogue. */
+int iswm_predict_tta_epilogue(const IswmTtaView* h_views, int n_views, int B, int C, int Ho, int Wo, int mode,
+                              float threshold, const void* d_true, int true_dtype, uint8_t* d_pred_out,
+                              uint8_t* d_conf_out, int64_t* d_cm, void* stream);
+
 /* Focal loss forward + backward in one pass (utils/loss.py:14-35 FocalLoss, exported through create_loss :37-39):
  *   ce_i = w[y_i] * nll_i (0 where y_i == ignore_index or outside [0,C)); pt = exp(-ce_i)
  *   loss = sum_i alpha * (1 - pt)^gamma * ce_i, divided by the number of ALL pixels when size_average

@@ -15,6 +15,7 @@ _HERE = os.path.dirname(os.path.abspath(__file__))
 LIB_PATH = os.environ.get("ISWM_B200_LIB") or os.path.join(_HERE, "libiswm_b200.so")
 
 MAX_TAPS = 32
+TTA_MAX_VIEWS = 8
 U8, I32, I64 = 0, 1, 2
 F32, BF16, E4M3 = 0, 1, 2
 EPI_AFFINE, EPI_RELU, EPI_RESIDUAL, EPI_STATS, EPI_OUT_F32, EPI_RES_MASK = 1, 2, 4, 8, 16, 32
@@ -66,6 +67,12 @@ class UnpackJob(C.Structure):
                 ("chunks", C.c_int32), ("blk_begin", C.c_int32), ("pad_", C.c_int32)]
 
 
+class TtaView(C.Structure):
+    """Mirror of IswmTtaView."""
+
+    _fields_ = [("lo", C.c_void_p), ("Hi", C.c_int32), ("Wi", C.c_int32), ("Hv", C.c_int32), ("Wv", C.c_int32), ("flip", C.c_int32)]
+
+
 class SyncBnJob(C.Structure):
     """Mirror of iswm_syncbn_job."""
 
@@ -112,6 +119,8 @@ SIGNATURES = {
     "iswm_confusion": (_i, [_p, _i, _p, _i, _i64, _i, _p, _p]),
     "iswm_argmax_confusion": (_i, [_p, _i, _p, _i, _i64, _i, _i64, _i, _f, _p, _p, _p, _p]),
     "iswm_predict_epilogue": (_i, [_p, _i, _i, _i, _i, _i, _i, _i, _f, _p, _i, _p, _p, _p, _p]),
+    "iswm_resize_flip_f32": (_i, [_p, _i, _i, _i, _i, _i, _i, _i, _p, _p]),
+    "iswm_predict_tta_epilogue": (_i, [C.POINTER(TtaView), _i, _i, _i, _i, _i, _i, _f, _p, _i, _p, _p, _p, _p]),
     "iswm_focal_fwd_bwd": (_i, [_p, _i, _p, _i, _p, _i64, _i, _i64, _i, _f, _f, _i, _p, _p, _p, _p]),
     "iswm_conv_igemm": (_i, [C.POINTER(ConvDesc), _p, _p, _p, _p, _p, _p, _p, _p]),
     "iswm_conv_igemm_ex": (_i, [C.POINTER(ConvDesc), _p, _p, _p, _p, _p, _p, _p, _p, _p]),

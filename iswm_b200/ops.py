@@ -130,6 +130,63 @@ def predict_epilogue(lo: torch.Tensor, H: int, W: int, true: Optional[torch.Tens
     return (out if true is not None else None), pred, conf
 
 
+def resize_flip_f32(x: torch.Tensor, size: Tuple[int, int], flip: bool = False, out: Optional[torch.Tensor] = None) -> torch.Tensor:
+    """fp32 NCHW [B,C,H,W] -> [B,C,*size]: F.interpolate(bilinear, align_corners=False) then .flip(-1) when `flip`; an exact
+    (mirrored) copy when `size` is the input's. `out` may be a contiguous batch slice of a larger buffer."""
+    if x.dtype != torch.float32 or x.dim() != 4:
+        raise TypeError("resize_flip_f32 wants fp32 NCHW [B,C,H,W]")
+    x = x.contiguous()
+    B, Cc, Hi, Wi = x.shape
+    Ho, Wo = size
+    if out is None:
+        out = torch.empty((B, Cc, Ho, Wo), dtype=torch.float32, device=x.device)
+    if tuple(out.shape) != (B, Cc, Ho, Wo) or out.dtype != torch.float32 or not out.is_contiguous():
+        raise ValueError(f"out must be a contiguous fp32 [{B},{Cc},{Ho},{Wo}] tensor")
+    check(_lib.lib().iswm_resize_flip_f32(_ptr(x), B, Cc, Hi, Wi, Ho, Wo, 1 if flip else 0, _ptr(out), _stream()), "resize_flip_f32")
+    return out
+
+
+def predict_tta_epilogue(views: Sequence[Tuple[torch.Tensor, Tuple[int, int], bool]], H: int, W: int,
+                         true: Optional[torch.Tensor] = None, mode: int = 1, threshold: float = 0.5,
+                         out: Optional[torch.Tensor] = None, pred: Optional[torch.Tensor] = None,
+                         conf: Optional[torch.Tensor] = None):
+    """Multi-view form of predict_epilogue (test-time augmentation): `views` lists (lo, (Hv, Wv), flip) with lo the fp32
+    NHWC [B,h,w,2] low-resolution logits of the network run on a view of full-resolution size (Hv, Wv), mirrored when
+    `flip`. Writes the uint8 maps of the view-averaged softmax at [B,H,W] (into `pred` / `conf` when given, e.g. batch
+    slices of larger maps) and accumulates the confusion counts into `out`. Returns (cm or None, pred, conf)."""
+    if not views:
+        raise ValueError("predict_tta_epilogue needs at least one view")
+    arr = (_lib.TtaView * len(views))()
+    keep = []
+    B = Cc = None
+    for i, (lo, (Hv, Wv), flip) in enumerate(views):
+        if lo.dtype != torch.float32 or lo.dim() != 4:
+            raise TypeError("predict_tta_epilogue wants fp32 NHWC [B,h,w,C] low-resolution logits")
+        lo = lo.contiguous()
+        keep.append(lo)
+        if B is None:
+            B, Cc = lo.shape[0], lo.shape[3]
+        elif (lo.shape[0], lo.shape[3]) != (B, Cc):
+            raise ValueError("every view needs the same batch and class count")
+        arr[i].lo, arr[i].Hi, arr[i].Wi, arr[i].Hv, arr[i].Wv, arr[i].flip = _ptr(lo), lo.shape[1], lo.shape[2], Hv, Wv, int(bool(flip))
+    dev = keep[0].device
+    for name, t in (("pred", pred), ("conf", conf)):
+        if t is not None and (tuple(t.shape) != (B, H, W) or t.dtype != torch.uint8 or not t.is_contiguous()):
+            raise ValueError(f"{name} must be a contiguous uint8 [{B},{H},{W}] tensor")
+    pred = torch.empty((B, H, W), dtype=torch.uint8, device=dev) if pred is None else pred
+    conf = torch.empty((B, H, W), dtype=torch.uint8, device=dev) if conf is None else conf
+    if true is not None:
+        true = true.contiguous()
+        if true.numel() != B * H * W:
+            raise ValueError(f"labels {tuple(true.shape)} do not match the {B}x{H}x{W} output")
+        if out is None:
+            out = torch.zeros(Cc * Cc + 1, dtype=torch.int64, device=dev)
+    check(_lib.lib().iswm_predict_tta_epilogue(arr, len(views), B, Cc, H, W, mode, threshold, _ptr(true),
+                                               _label_code(true) if true is not None else _lib.I64, _ptr(pred), _ptr(conf),
+                                               _ptr(out) if true is not None else None, _stream()), "predict_tta_epilogue")
+    return (out if true is not None else None), pred, conf
+
+
 def focal_fwd_bwd(logits: torch.Tensor, labels: torch.Tensor, weight: Optional[torch.Tensor], alpha: float = 1.0,
                   gamma: float = 0.0, size_average: bool = True, ignore_index: int = 255,
                   want_grad: bool = True) -> Tuple[torch.Tensor, Optional[torch.Tensor]]:
