@@ -143,6 +143,26 @@ int iswm_predict_tta_epilogue(const IswmTtaView* h_views, int n_views, int B, in
                               float threshold, const void* d_true, int true_dtype, uint8_t* d_pred_out,
                               uint8_t* d_conf_out, int64_t* d_cm, void* stream);
 
+/* ---- sliding-window inference for the predict step ------------------------------------------------------------ */
+/* Window placement along an axis of length L, for a window side `win` and stride s (1 <= s <= win): the side is
+ * w = min(win, L), there are n = ceil((L - w) / s) + 1 windows at offsets o_i = min(i*s, L - w) (the last one snapped
+ * to the border). The windows of a batch are listed image-major, then row-major over (iy, ix): B*ny*nx in all. */
+
+/* Copies windows [first, first+n) of that list out of fp32 NCHW [B,C,H,W] into d_out fp32 [n,C,wh',ww'] (wh' = min(wh,H),
+ * ww' = min(ww,W)), exactly. The offsets are computed in the kernel from (H, W, wh, ww, sh, sw). */
+int iswm_window_gather_f32(const float* d_x, int B, int C, int H, int W, int wh, int ww, int sh, int sw, int first, int n,
+                           float* d_out, void* stream);
+
+/* Overlap-averaging predict epilogue: d_lo is fp32 NHWC [B*ny*nx, hi, wi, 2], the low-resolution logits of every window
+ * in list order (forward_lowres of the gathered windows). For every pixel, the windows covering it are visited in
+ * ascending (iy, ix) order; each contributes the 2-class softmax of its logits bilinear (hi,wi) -> (wh',ww') at the
+ * window-local pixel (the arithmetic of iswm_predict_epilogue); the sum is divided by the covering count, then
+ * pred = p1 > threshold and conf = uint8(p1*255). d_true / d_cm / d_pred_out / d_conf_out as in iswm_predict_epilogue.
+ * C == 2 only; any W >= 1. */
+int iswm_predict_window_epilogue(const float* d_lo, int B, int H, int W, int wh, int ww, int sh, int sw, int hi, int wi,
+                                 int C, float threshold, const void* d_true, int true_dtype, uint8_t* d_pred_out,
+                                 uint8_t* d_conf_out, int64_t* d_cm, void* stream);
+
 /* Focal loss forward + backward in one pass (utils/loss.py:14-35 FocalLoss, exported through create_loss :37-39):
  *   ce_i = w[y_i] * nll_i (0 where y_i == ignore_index or outside [0,C)); pt = exp(-ce_i)
  *   loss = sum_i alpha * (1 - pt)^gamma * ce_i, divided by the number of ALL pixels when size_average

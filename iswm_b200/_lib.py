@@ -121,6 +121,8 @@ SIGNATURES = {
     "iswm_predict_epilogue": (_i, [_p, _i, _i, _i, _i, _i, _i, _i, _f, _p, _i, _p, _p, _p, _p]),
     "iswm_resize_flip_f32": (_i, [_p, _i, _i, _i, _i, _i, _i, _i, _p, _p]),
     "iswm_predict_tta_epilogue": (_i, [C.POINTER(TtaView), _i, _i, _i, _i, _i, _i, _f, _p, _i, _p, _p, _p, _p]),
+    "iswm_window_gather_f32": (_i, [_p, _i, _i, _i, _i, _i, _i, _i, _i, _i, _i, _p, _p]),
+    "iswm_predict_window_epilogue": (_i, [_p, _i, _i, _i, _i, _i, _i, _i, _i, _i, _i, _f, _p, _i, _p, _p, _p, _p]),
     "iswm_focal_fwd_bwd": (_i, [_p, _i, _p, _i, _p, _i64, _i, _i64, _i, _f, _f, _i, _p, _p, _p, _p]),
     "iswm_conv_igemm": (_i, [C.POINTER(ConvDesc), _p, _p, _p, _p, _p, _p, _p, _p]),
     "iswm_conv_igemm_ex": (_i, [C.POINTER(ConvDesc), _p, _p, _p, _p, _p, _p, _p, _p, _p]),

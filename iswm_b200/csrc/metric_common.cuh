@@ -1,5 +1,5 @@
-// metric_common.cuh - packed vector loads / stores and the block counter flush shared by the HBM-bound metric kernels
-// (loss_metric.cu, tta.cu).
+// metric_common.cuh - packed vector loads / stores, the block counter flush and the low-resolution logit tap shared by
+// the HBM-bound metric and predict-epilogue kernels (loss_metric.cu, tta.cu, window.cu).
 #pragma once
 #include "common.cuh"
 
@@ -75,6 +75,18 @@ __device__ __forceinline__ void flush_counters(unsigned (&cnt)[NREG], int n_vali
     for (int w = 0; w < kWarps; w++) t += s_part[w][threadIdx.x];
     if (t) atomicAdd(g_out + threadIdx.x, t);
   }
+}
+
+// the two logits of one output column, bilinear from the low-resolution row pair (r0, r1) with row weight ly: the
+// arithmetic of logits_up_fwd / predict_epilogue2 (bil_src, then bil_mix over the four taps in the same order)
+__device__ __forceinline__ float2 lo_tap(const float2* r0, const float2* r1, float ly, int col, float sw, int Wi) {
+  int x0, x1;
+  float lx;
+  bil_src(col, sw, Wi, x0, x1, lx);
+  const float w00 = (1.f - ly) * (1.f - lx), w01 = (1.f - ly) * lx, w10 = ly * (1.f - lx), w11 = ly * lx;
+  const float2 v00 = __ldg(r0 + x0), v01 = __ldg(r0 + x1), v10 = __ldg(r1 + x0), v11 = __ldg(r1 + x1);
+  return make_float2(bil_mix(w00, v00.x, w01, v01.x, w10, v10.x, w11, v11.x),
+                     bil_mix(w00, v00.y, w01, v01.y, w10, v10.y, w11, v11.y));
 }
 
 }  // namespace iswm

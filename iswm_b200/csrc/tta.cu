@@ -50,18 +50,6 @@ struct TtaViews {
   IswmTtaView v[ISWM_TTA_MAX_VIEWS];
 };
 
-// the two logits of one view-grid column, bilinear from the low-resolution row pair (r0, r1) with row weight ly: the
-// arithmetic of logits_up_fwd / predict_epilogue2 (bil_src, then bil_mix over the four taps in the same order)
-__device__ __forceinline__ float2 lo_tap(const float2* r0, const float2* r1, float ly, int col, float sw, int Wi) {
-  int x0, x1;
-  float lx;
-  bil_src(col, sw, Wi, x0, x1, lx);
-  const float w00 = (1.f - ly) * (1.f - lx), w01 = (1.f - ly) * lx, w10 = ly * (1.f - lx), w11 = ly * lx;
-  const float2 v00 = __ldg(r0 + x0), v01 = __ldg(r0 + x1), v10 = __ldg(r1 + x0), v11 = __ldg(r1 + x1);
-  return make_float2(bil_mix(w00, v00.x, w01, v01.x, w10, v10.x, w11, v11.x),
-                     bil_mix(w00, v00.y, w01, v01.y, w10, v10.y, w11, v11.y));
-}
-
 // One grid row per output image row; a thread produces 4 consecutive pixels, looping over the views for each of them
 // (the views' low-resolution logits are small and stay in L1 / L2, so the taps cost latency, not HBM traffic).
 template <typename TT, bool HAS_CM, bool VEC4>

@@ -7,7 +7,7 @@ streams only. There is no fallback path: a CPU tensor or a missing library is an
 from __future__ import annotations
 
 import ctypes as C
-from typing import Optional, Sequence, Tuple
+from typing import List, Optional, Sequence, Tuple
 
 import torch
 
@@ -184,6 +184,73 @@ def predict_tta_epilogue(views: Sequence[Tuple[torch.Tensor, Tuple[int, int], bo
     check(_lib.lib().iswm_predict_tta_epilogue(arr, len(views), B, Cc, H, W, mode, threshold, _ptr(true),
                                                _label_code(true) if true is not None else _lib.I64, _ptr(pred), _ptr(conf),
                                                _ptr(out) if true is not None else None, _stream()), "predict_tta_epilogue")
+    return (out if true is not None else None), pred, conf
+
+
+def window_offsets(L: int, window: int, stride: int) -> Tuple[int, List[int]]:
+    """Window placement along an axis of length L (the rule of csrc/window.cu's WinAxis): the side w = min(window, L)
+    and the offsets min(i * stride, L - w) of the ceil((L - w) / stride) + 1 windows, the last one snapped to the border.
+    A stride above the window would leave pixels uncovered."""
+    if window < 1 or not 1 <= stride <= window:
+        raise ValueError(f"window {window}, stride {stride}: need 1 <= stride <= window")
+    w = min(window, L)
+    return w, [min(i * stride, L - w) for i in range((L - w + stride - 1) // stride + 1)]
+
+
+def window_gather_f32(x: torch.Tensor, window: Tuple[int, int], stride: Tuple[int, int], first: int = 0,
+                      n: Optional[int] = None, out: Optional[torch.Tensor] = None) -> torch.Tensor:
+    """fp32 NCHW [B,C,H,W] -> windows [first, first+n) of the batch's window list (image-major, then row-major over the
+    window grid) as [n,C,wh,ww], copied exactly; (wh, ww) is `window` clamped to the scene. `out` may be a contiguous
+    batch slice of a larger buffer."""
+    if x.dtype != torch.float32 or x.dim() != 4:
+        raise TypeError("window_gather_f32 wants fp32 NCHW [B,C,H,W]")
+    x = x.contiguous()
+    B, Cc, H, W = x.shape
+    (wh, ys), (ww, xs) = window_offsets(H, window[0], stride[0]), window_offsets(W, window[1], stride[1])
+    total = B * len(ys) * len(xs)
+    n = total - first if n is None else n
+    if first < 0 or n < 0 or first + n > total:
+        raise ValueError(f"windows [{first}, {first + n}) outside the {total} windows of the batch")
+    if out is None:
+        out = torch.empty((n, Cc, wh, ww), dtype=torch.float32, device=x.device)
+    if tuple(out.shape) != (n, Cc, wh, ww) or out.dtype != torch.float32 or not out.is_contiguous():
+        raise ValueError(f"out must be a contiguous fp32 [{n},{Cc},{wh},{ww}] tensor")
+    check(_lib.lib().iswm_window_gather_f32(_ptr(x), B, Cc, H, W, window[0], window[1], stride[0], stride[1], first, n,
+                                            _ptr(out), _stream()), "window_gather_f32")
+    return out
+
+
+def predict_window_epilogue(lo: torch.Tensor, H: int, W: int, window: Tuple[int, int], stride: Tuple[int, int],
+                            true: Optional[torch.Tensor] = None, threshold: float = 0.5, out: Optional[torch.Tensor] = None,
+                            pred: Optional[torch.Tensor] = None, conf: Optional[torch.Tensor] = None):
+    """Sliding-window form of predict_epilogue: `lo` is fp32 NHWC [B*ny*nx,h,w,2], the low-resolution logits of every
+    window of B scenes of [H,W] in window_gather_f32's order. Writes the uint8 maps of the softmax averaged over the
+    windows covering each pixel at [B,H,W] (threshold mode; into `pred` / `conf` when given) and accumulates the
+    confusion counts into `out`. Returns (cm or None, pred, conf)."""
+    if lo.dtype != torch.float32 or lo.dim() != 4:
+        raise TypeError("predict_window_epilogue wants fp32 NHWC [N,h,w,C] low-resolution logits")
+    lo = lo.contiguous()
+    N, hi, wi, Cc = lo.shape
+    per_img = len(window_offsets(H, window[0], stride[0])[1]) * len(window_offsets(W, window[1], stride[1])[1])
+    if N % per_img:
+        raise ValueError(f"{N} windows of logits are not a whole number of {H}x{W} scenes of {per_img} windows")
+    B = N // per_img
+    dev = lo.device
+    for name, t in (("pred", pred), ("conf", conf)):
+        if t is not None and (tuple(t.shape) != (B, H, W) or t.dtype != torch.uint8 or not t.is_contiguous()):
+            raise ValueError(f"{name} must be a contiguous uint8 [{B},{H},{W}] tensor")
+    pred = torch.empty((B, H, W), dtype=torch.uint8, device=dev) if pred is None else pred
+    conf = torch.empty((B, H, W), dtype=torch.uint8, device=dev) if conf is None else conf
+    if true is not None:
+        true = true.contiguous()
+        if true.numel() != B * H * W:
+            raise ValueError(f"labels {tuple(true.shape)} do not match the {B}x{H}x{W} output")
+        if out is None:
+            out = torch.zeros(Cc * Cc + 1, dtype=torch.int64, device=dev)
+    check(_lib.lib().iswm_predict_window_epilogue(_ptr(lo), B, H, W, window[0], window[1], stride[0], stride[1], hi, wi, Cc,
+                                                  threshold, _ptr(true), _label_code(true) if true is not None else _lib.I64,
+                                                  _ptr(pred), _ptr(conf), _ptr(out) if true is not None else None, _stream()),
+          "predict_window_epilogue")
     return (out if true is not None else None), pred, conf
 
 

@@ -16,20 +16,31 @@ views (s, f), s in scales, f in (False, True) when flip:
 The fused path builds each scale's views with `iswm_resize_flip_f32` into one input (unflipped and flipped halves run
 as one forward: eval-mode BatchNorm is per sample), keeps every view's low-resolution logits, and runs ONE
 `iswm_predict_tta_epilogue` over all of them; no view's full-resolution logits are written.
+
+Sliding-window inference (`window`, `stride`: mmseg's mode='slide') runs the network on windows of the scene and
+averages the softmax where windows overlap. Per axis of length L the window side is w = min(window, L) and the
+n = ceil((L - w) / s) + 1 windows sit at o_i = min(i * s, L - w), the last one snapped to the border:
+
+    p = sum over the windows covering a pixel, in ascending (iy, ix) order, of softmax(model(window))[local pixel];
+    p /= the covering count
+
+The fused path cuts chunks of windows with `iswm_window_gather_f32` straight into the batch of one forward (windows of
+different scenes share it: eval-mode BatchNorm is per sample), keeps every window's low-resolution logits, and runs ONE
+`iswm_predict_window_epilogue` over all of them. Every forward stays within MAX_FORWARD_PIXELS, whatever the scene size.
 """
 from __future__ import annotations
 
 import math
-from typing import List, Optional, Sequence, Tuple
+from typing import List, NamedTuple, Optional, Sequence, Tuple
 
 import torch
 import torch.nn.functional as F
 
 from . import _lib, ops
 
-# B x H x W of the largest single forward the test-time augmentation issues: that of the largest predict geometry the
-# engine is benchmarked at (8 x 2048^2). Beyond it the engine's 32-bit element counts are untested (at s = 2 on 2048^2
-# inputs, 8 images of layer1 activations hold exactly 2^31 elements), so larger batches run in chunks.
+# B x H x W of the largest single forward test-time augmentation or sliding windows issue: that of the largest predict
+# geometry the engine is benchmarked at (8 x 2048^2). Beyond it the engine's 32-bit element counts are untested (at s = 2
+# on 2048^2 inputs, 8 images of layer1 activations hold exactly 2^31 elements), so larger batches run in chunks.
 MAX_FORWARD_PIXELS = 8 * 2048 * 2048
 
 
@@ -51,13 +62,45 @@ def _tta_views(scales: Sequence[float], flip: bool, H: int, W: int) -> List[Tupl
     return views
 
 
+class Windows(NamedTuple):
+    """Sliding-window geometry of one [H,W] scene: the window side per axis (clamped to the scene), the strides, and
+    the window offsets per axis (`ys` rows, `xs` columns)."""
+    size: Tuple[int, int]
+    stride: Tuple[int, int]
+    ys: List[int]
+    xs: List[int]
+
+
+def _pair(v, name: str) -> Tuple[int, int]:
+    t = (v, v) if not isinstance(v, (tuple, list)) else tuple(v)
+    if len(t) != 2 or not all(isinstance(e, int) for e in t):
+        raise ValueError(f"{name} must be an int or a pair of ints, got {v!r}")
+    return t
+
+
+def _windows(H: int, W: int, window, stride=None) -> Windows:
+    """The window placement of predict_mask(window=, stride=), validated: sides of at least 16 pixels, strides in
+    [1, window]; `stride` defaults to max(1, 2 * window // 3) per axis."""
+    win = _pair(window, "window")
+    if min(win) < 16:
+        raise ValueError(f"window {win[0]}x{win[1]}: windows need at least 16x16 pixels")
+    st = tuple(max(1, (2 * w) // 3) for w in win) if stride is None else _pair(stride, "stride")
+    (wh, ys), (ww, xs) = ops.window_offsets(H, win[0], st[0]), ops.window_offsets(W, win[1], st[1])
+    return Windows((wh, ww), st, ys, xs)
+
+
 @torch.no_grad()
 def predict_mask(model, images: torch.Tensor, threshold: float = 0.5, labels: Optional[torch.Tensor] = None,
                  metrics=None, fused: bool = True, scales: Sequence[float] = (1.0,),
-                 flip: bool = False) -> Tuple[torch.Tensor, torch.Tensor]:
+                 flip: bool = False, window=None, stride=None) -> Tuple[torch.Tensor, torch.Tensor]:
     """images: float32 [B,3,H,W] on CUDA (already normalised, predict.py:259-260). Returns (pred uint8 [B,H,W] in
     {0,1}, confidence uint8 [B,H,W]); `metrics` (a StreamMetrics) receives the confusion counts when labels are given.
-    `scales` / `flip` request test-time augmentation (two-class models; at most 8 views); the defaults run one view."""
+    `scales` / `flip` request test-time augmentation (two-class models; at most 8 views); the defaults run one view.
+    `window` (an int or (wh, ww)) requests sliding-window inference: per axis of length L the window side is
+    w = min(window, L), and windows sit at min(i * s, L - w) for i < ceil((L - w) / s) + 1 with the stride s (an int or
+    (sh, sw), 1 <= s <= window; default max(1, 2 * window // 3)). Each pixel's softmax is averaged over the windows
+    covering it (uniform weights), then thresholded. Two-class models; not combined with `scales` / `flip`; window
+    sides of at least 16. With window=None the scene runs as one forward."""
     if not images.is_cuda:
         raise RuntimeError("iswm_b200.predict runs on CUDA only (no CPU fallback)")
     net = getattr(model, "module", model)
@@ -66,6 +109,17 @@ def predict_mask(model, images: torch.Tensor, threshold: float = 0.5, labels: Op
     n_classes = net.engine().cls.cout
     if n_classes < 2:
         raise ValueError("predict_mask needs at least 2 classes (foreground = class 1)")
+    if window is not None:
+        if flip or [float(s) for s in scales] != [1.0]:
+            raise ValueError("sliding windows are not combined with test-time augmentation (scales / flip)")
+        win = _windows(H, W, window, stride)
+        if n_classes != 2:
+            raise ValueError(f"sliding-window inference needs a two-class model, this one has {n_classes}")
+        if fused:
+            return _predict_window(net, images, win, threshold, labels if cm is not None else None, cm)
+        return _predict_window_unfused(model, images, win, threshold, labels if cm is not None else None, cm)
+    if stride is not None:
+        raise ValueError("stride is the step of sliding windows; it needs window")
     if flip or [float(s) for s in scales] != [1.0]:
         views = _tta_views(scales, flip, H, W)
         if n_classes != 2:
@@ -143,6 +197,54 @@ def _predict_tta_unfused(model, images, views, threshold, labels, cm):
         if was_training:
             model.train()
     p1 = p[:, 1] / len(views)
+    pred = (p1 > threshold).to(torch.uint8)
+    conf = (p1 * 255).to(torch.uint8)
+    if cm is not None:
+        ops.confusion(labels, pred, 2, out=cm)
+    return pred, conf
+
+
+def _predict_window(net, images, win, threshold, labels, cm):
+    """Fused sliding windows: the batch's flat window list in chunks of at most MAX_FORWARD_PIXELS pixels (one window
+    at least), each chunk gathered into one input and run as one forward whose low-resolution logits are copied into
+    one buffer for all windows; then ONE epilogue writes the maps and counts."""
+    x = images.contiguous()
+    B, C = x.shape[:2]
+    (wh, ww), n_win = win.size, B * len(win.ys) * len(win.xs)
+    chunk = max(1, min(n_win, MAX_FORWARD_PIXELS // (wh * ww)))
+    xb = torch.empty((chunk, C, wh, ww), dtype=torch.float32, device=x.device)
+    lows = None
+    for g0 in range(0, n_win, chunk):
+        n = min(chunk, n_win - g0)
+        lo = net.forward_lowres(ops.window_gather_f32(x, win.size, win.stride, g0, n, out=xb[:n]))
+        if lows is None:
+            lows = torch.empty((n_win,) + tuple(lo.shape[1:]), dtype=torch.float32, device=x.device)
+        lows[g0:g0 + n].copy_(lo)
+    _, pred, conf = ops.predict_window_epilogue(lows, x.shape[2], x.shape[3], win.size, win.stride, labels,
+                                                threshold=threshold, out=cm)
+    return pred, conf
+
+
+def _predict_window_unfused(model, images, win, threshold, labels, cm):
+    """The torch composition of sliding windows through the public forward: the reference the fused path is tested
+    against."""
+    B, _, H, W = images.shape
+    (wh, ww) = win.size
+    s = torch.zeros((B, H, W), dtype=torch.float32, device=images.device)
+    cnt = torch.zeros_like(s)
+    was_training = model.training
+    model.eval()
+    try:
+        for b in range(B):
+            for y0 in win.ys:
+                for x0 in win.xs:
+                    sm = torch.softmax(model(images[b:b + 1, :, y0:y0 + wh, x0:x0 + ww]), 1)
+                    s[b:b + 1, y0:y0 + wh, x0:x0 + ww] += sm[:, 1]
+                    cnt[b:b + 1, y0:y0 + wh, x0:x0 + ww] += 1
+    finally:
+        if was_training:
+            model.train()
+    p1 = s / cnt
     pred = (p1 > threshold).to(torch.uint8)
     conf = (p1 * 255).to(torch.uint8)
     if cm is not None:
